@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the MergeRec hot paths on B200, one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input (random-init weights of the named
 architecture; there is no network for checkpoints).  `value` is the whole-job throughput with inputs already
@@ -10,6 +10,8 @@ copies inside the timed region.  `roofline` times the dominant kernel alone with
 `cpu_baseline` times the UNMODIFIED reference packages (baseline/_ref, copied there by baseline/install_ref.py) on the
 box's host cores, with the oracle port (oracle/) beside it; where baseline/_ref is absent only the port runs and the
 line says `kind: "port"`.  `--impl reference` runs only that CPU arm.  See DESIGN.md section "Measurement".
+`--dump-outputs DIR` saves what the last timed step returned (the companion's too) as DIR/<name>.npy, larger outputs
+as a fixed seeded sample, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -43,6 +45,25 @@ def emit(line: dict) -> None:
         sys.stdout.flush()
     else:
         os.write(_JSON_FD, data)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, outputs: dict) -> None:
+    """Write every output as `directory/<name>.npy` (float32 or float64), at most DUMP_LIMIT_BYTES in all: the inputs
+    are seeded, so two builds run with the same arguments can be compared array by array."""
+    arrays = {name: np.asarray(a) for name, a in outputs.items()}
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"output {name} is {a.dtype}, not float32 / float64")
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"outputs hold {total} bytes, more than the {DUMP_LIMIT_BYTES} a dump may take")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"wrote {len(arrays)} outputs ({total} bytes) to {directory}")
 
 
 def measured_peaks():
@@ -192,10 +213,12 @@ def flush_l2(device):
     _L2_FLUSH.fill_(1)
 
 
-def measure(wl, steps: int, warmup: int, rank: int, world: int, local_rank: int, cpu_arm: bool, sample_clocks: bool):
+def measure(wl, steps: int, warmup: int, rank: int, world: int, local_rank: int, cpu_arm: bool, sample_clocks: bool,
+            outputs: dict = None):
     """One workload through the bench contract: W untimed warm-up steps, exactly K timed steps between barrier +
     synchronize pairs (CUDA events, max over ranks), the end-to-end arm (pinned host inputs, host<->device copies in
-    the timed region), the roofline of the dominant kernel and the CPU arm.  Returns the JSON line (rank 0) or None."""
+    the timed region), the roofline of the dominant kernel and the CPU arm.  Returns the JSON line (rank 0) or None.
+    `outputs`, when given, receives the host arrays that the last timed step computed (`wl.outputs()`)."""
     import torch.distributed as dist
 
     def barrier():
@@ -238,6 +261,8 @@ def measure(wl, steps: int, warmup: int, rank: int, world: int, local_rank: int,
         total_ms = reduce_max(ev0.elapsed_time(ev1))
     if hasattr(wl, "finish"):
         wl.finish()   # deferred host-side checks of the timed steps, checksums, stage timings (every rank)
+    if outputs is not None:
+        outputs.update(wl.outputs())     # before the end-to-end arm overwrites the step's buffers
 
     # end to end through the public API: pinned host inputs -> H2D -> kernels -> D2H result, every step
     wl.setup_e2e()
@@ -298,8 +323,9 @@ def run_ours(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=device)
     cpu_arm = world == 1 and not args.no_cpu_baseline
+    outputs = {} if (args.dump_outputs and rank == 0) else None
     wl = WORKLOADS[args.workload](rank=rank, world=world, device=device)
-    line = measure(wl, args.steps, args.warmup, rank, world, local_rank, cpu_arm, sample_clocks=True)
+    line = measure(wl, args.steps, args.warmup, rank, world, local_rank, cpu_arm, sample_clocks=True, outputs=outputs)
     # the other hot path, carried beside the headline: the merger at the size BASELINE.json quotes it on (single GPU)
     # or its sharded form (several GPUs) -- a complete nested line with its own roofline / e2e / cpu_baseline
     comp_cls = None if args.no_companion else wl.companion()
@@ -308,17 +334,22 @@ def run_ours(args):
         del wl
         torch.cuda.empty_cache()
         comp = comp_cls(rank=rank, world=world, device=device)
+        comp_outputs = None if outputs is None else {}
         try:
             sub = measure(comp, min(args.steps, 20), max(3, min(args.warmup, 5)), rank, world, local_rank, cpu_arm,
-                          sample_clocks=False)
+                          sample_clocks=False, outputs=comp_outputs)
         except Exception as e:  # noqa: BLE001 -- the headline line must still be printed
             if world > 1:
                 raise
             sub = {"error": repr(e)}
         if rank == 0:
             line[comp.companion_key] = sub
+        if comp_outputs:
+            outputs.update({f"{comp.companion_key}.{name}": a for name, a in comp_outputs.items()})
     if rank == 0:
         emit(line)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -360,7 +391,13 @@ def main():
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-companion", action="store_true", help="skip the nested merger line of the evaluator workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (the companion's as <key>.<name>)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         log("note: fewer than 3 warm-up steps requested; the timing rules ask for >= 3")
     if args.impl == "reference":

@@ -43,6 +43,11 @@ class Workload:
             if name not in ("rank", "world", "device"):
                 delattr(self, name)
 
+    def outputs(self) -> Dict[str, np.ndarray]:
+        """What the last timed step handed to its caller, as float32 / float64 host arrays by name (`bench.py
+        --dump-outputs`)."""
+        raise NotImplementedError(f"workload {self.name} does not name its outputs")
+
 
 def reference_package():
     """The unmodified reference hot-path packages installed under baseline/_ref (baseline/install_ref.py), or None."""
@@ -94,6 +99,19 @@ def _pinned(t: torch.Tensor) -> torch.Tensor:
     return out
 
 
+OUTPUT_SAMPLE = 1 << 21     # elements kept of a larger output (8 MB of float32), so that a dump stays small
+
+
+def _output(t: torch.Tensor) -> np.ndarray:
+    """`t` as a float32 host array.  Above OUTPUT_SAMPLE elements: the flattened tensor at OUTPUT_SAMPLE positions drawn
+    with a fixed seed (ascending), the same positions in every run of the same workload."""
+    t = t.detach()
+    if t.numel() > OUTPUT_SAMPLE:
+        pos = np.sort(np.random.Generator(np.random.PCG64(0)).choice(t.numel(), OUTPUT_SAMPLE, replace=False))
+        t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+    return t.float().cpu().numpy()
+
+
 class LambdaMergeK8(Workload):
     """Per-layer lambda merge of 8 BLaIR-base task vectors (the merge half of BASELINE config 2; A4).
     Algorithmic bytes per step: (K+2) * d * 4 (read base + K task-vector rows, write merged)."""
@@ -136,6 +154,9 @@ class LambdaMergeK8(Workload):
         from mergerec_b200 import _lib
         from mergerec_b200.merger.algorithms._common import merge_axpy
         merge_axpy(self.base, self.rows, self.w, _lib.MR_ORDER_SUM_FIRST, False, self.seg_end, self.seg_group, out=self.out)
+
+    def outputs(self):
+        return {"merged": _output(self.out)}
 
     def units_per_step_all_ranks(self):
         return self.bytes_per_step / GB     # one job; with several ranks every rank repeats it (no "x N" credit)
@@ -540,6 +561,9 @@ class EvalCatalog(Workload):
     def step(self):
         self.last = self.ev.evaluate_embeddings(self.queries, self.table, self.labels, mode=self.mode)
 
+    def outputs(self):
+        return {name: np.float64(v) for name, v in self.last.items()}
+
     def units_per_step_all_ranks(self):
         return float(self.Q) * float(self.N)
 
@@ -865,6 +889,11 @@ class CollabStepCfg3(Workload):
         self.opt.step()
         self.loss = loss.detach()
 
+    def outputs(self):
+        out = {"loss": _output(self.loss)}
+        out.update({f"lambda.{k}": _output(v) for k, v in self.module.per_weights.items()})
+        return out
+
     def units_per_step_all_ranks(self):
         return float(self.world)
 
@@ -1118,6 +1147,9 @@ class DistillStep(Workload):
         else:
             self._eager_step()
 
+    def outputs(self):
+        return {"loss": _output(self.loss), "rep_grad": _output(self.rep.grad)}
+
     def units_per_step_all_ranks(self):
         return float(self.B * self.world)
 
@@ -1331,6 +1363,9 @@ class MergeCfg4(TiesCfg2):
 
     def step(self):
         self._eager_step()
+
+    def outputs(self):
+        return {"task_arithmetic": _output(self.out_arith), "merged": _output(self.out)}
 
     def step_fused(self):
         from mergerec_b200.merger.algorithms import ties as T
