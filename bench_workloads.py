@@ -1067,6 +1067,112 @@ class TiesSharded(TiesCfg2):
         return {"slice": [self.lo, self.hi], "merged_bits_checksum": self._checksum}
 
 
+class PcbSharded(TiesSharded):
+    """SURVEY.md section 8(e), merger row, for PCB merging (pcb.py:37-73): K = 8 BLaIR-base models, the flat vector
+    SHARDED d/G over the ranks, the same seeded inputs as `ties_sharded`.  One step = `get_pcb_vectors_sharded` (two
+    sharded magnitude selects for the 1 % / 99 % clamps, the phased quantile search `mr_pcb_vectors_dist` with all-reduced
+    histograms, the build of the local slice; one host synchronisation for the status words) followed by the base-first
+    merge of the slice.  Strong scaling: the whole job's algorithmic bytes divided by the slowest rank's time.  The merged
+    slices are bit-identical to the single-GPU `merge_pcb` (tests/test_sharded_pcb_gpu.py); `merged_bits_checksum` is
+    the same for every G."""
+
+    name = "pcb_sharded"
+    scaling = "strong"
+    launches_per_step = 40  # 2 x 6-phase select, 7-phase search (incl. build), merge (+ NCCL's)
+
+    def __init__(self, rank, world, device):
+        super().__init__(rank, world, device)
+        K, d = self.K, self.d
+        # two clamp selects and the quantile search read base + K models once each, the build reads them and writes K
+        # rows, the merge reads base + K rows and writes the result
+        self.bytes_build = 3 * (K + 1) * d * 4 + (2 * K + 1) * d * 4
+        self.bytes_merge = (K + 2) * d * 4
+        self.bytes_per_step = self.bytes_build + self.bytes_merge
+
+    def config(self):
+        return {"workload": "PCB merge (density 0.2) of K=8 BLaIR-base models, flat vector sharded d/G per GPU; global "
+                            "clamps and balancing-weight quantile via all-reduced radix histograms; local build + "
+                            "base-first merge",
+                "K": self.K, "d": self.d, "density": 0.2, "weights": 0.3,
+                "l2": "per-rank inputs (4.5 GB / G) exceed L2 for G <= 8",
+                "algorithmic_bytes": "3 x (K+1) d 4 (two clamp selects, quantile search) + (2K+1) d 4 (build) + (K+2) d 4 "
+                                     "(merge)",
+                "parallelism": "flat dimension sharded d/G per GPU (strong scaling); per step 2 x (4 all-reduces + 1 "
+                               "all-gather) for the clamp selects, 6 all-reduces of the (2, K, 2048) histograms + 1 of "
+                               "the row maxima for the quantile search, 1 all-reduce of the status words; the same code "
+                               "path without collectives on 1 GPU"}
+
+    def setup(self):
+        super().setup()
+        del self.That, self.Trows
+        self.wl = [0.3] * self.K
+
+    def _vectors(self):
+        from mergerec_b200.merger.sharded import get_pcb_vectors_sharded
+        self.vectors = get_pcb_vectors_sharded(self.base, self.models, 0.2, self.d, self.group)
+
+    def _merge_only(self):
+        from mergerec_b200 import _lib
+        from mergerec_b200.merger.algorithms._common import merge_axpy, weights_tensor
+        if self.hi > self.lo:
+            merge_axpy(self.base, list(self.vectors.unbind(0)), weights_tensor(self.wl, self.device), _lib.MR_ORDER_BASE_FIRST,
+                       False, out=self.out)
+
+    def step(self):
+        self._vectors()
+        self._merge_only()
+
+    def roofline(self, peaks):
+        from bench import event_time_ms
+        n, K = self.hi - self.lo, self.K
+        ms_vec = event_time_ms(self._vectors, 3) if self.world == 1 else None     # collectives: every rank or none
+        ms_merge = event_time_ms(self._merge_only, 10)
+        b_merge = (K + 2) * n * 4
+        ach = b_merge / GB / (ms_merge * 1e-3)
+        return {"bound": "hbm", "kernel": "mr::merge_kernel (base-first PCB merge) on this rank's slice",
+                "achieved": ach, "peak": peaks["hbm_gbs"], "peak_source": peaks["source"], "unit": "GB/s",
+                "frac": ach / peaks["hbm_gbs"], "traffic": None, "ms_per_launch": ms_merge,
+                "algorithmic_bytes_per_launch": b_merge,
+                "other_kernels": {
+                    "get_pcb_vectors_sharded (clamp selects + quantile search + build; timed without collectives, 1 GPU "
+                    "only)": {"ms": ms_vec}}}
+
+    # -- CPU arms: the unmodified reference `merge_pcb` (get_pcb_vectors + base-first sum) from baseline/_ref, and the
+    #    numpy port of oracle/oracle.py beside it, both on a RoBERTa-shaped slice (12 layers, hidden 64, d = 3.85 M): at
+    #    full size the reference sorts (K, 1.2e8) tensors three times per step.
+    def _slice_inputs(self):
+        shapes = synth.roberta_shapes(hidden=64, ffn=256)
+        d = synth.total_numel(shapes)
+        g = torch.Generator().manual_seed(7)
+        base = torch.randn(d, generator=g) * 0.02
+        models = [base + 1e-3 * torch.randn(d, generator=g) for _ in range(self.K)]
+        return d, base, models
+
+    def _port_step_fn(self):
+        from oracle import oracle as orc
+        d, base, models = self._slice_inputs()
+        b, ms = base.numpy(), [m.numpy() for m in models]
+
+        def step():
+            orc.merge_pcb(b, ms, [0.3] * self.K, 0.2)
+        nbytes = (4 * (self.K + 1) + self.K + (self.K + 2)) * d * 4
+        return step, nbytes, (f"numpy port of get_pcb_vectors + merge_pcb (oracle/oracle.py) on a RoBERTa-shaped slice: 12 "
+                              f"layers, hidden 64, d={d}, K={self.K}, density 0.2")
+
+    def _reference_step_fn(self):
+        ref = reference_package()
+        if ref is None:
+            return None
+        from rec_retrieval.merger.algorithms.pcb import merge_pcb
+        d, base, models = self._slice_inputs()
+
+        def step():
+            merge_pcb(base, models, [0.3] * self.K, density=0.2)
+        nbytes = (4 * (self.K + 1) + self.K + (self.K + 2)) * d * 4
+        return step, nbytes, (f"UNMODIFIED reference merge_pcb (get_pcb_vectors + base-first sum) on a RoBERTa-shaped slice: "
+                              f"12 layers, hidden 64, d={d}, K={self.K}, density 0.2")
+
+
 class DistillStep(Workload):
     """The distillation half of a collaborative-merging step (SURVEY.md section 8(f) rank 1; reference:
     module/distiller/sequence/module.py:59-76 + loss_fn.py KD loss): catalogue logits of 16 pseudo-user representations
@@ -1499,5 +1605,6 @@ class EvalCfg4(EvalCatalog):
 
 WORKLOADS = {LambdaMergeK8.name: LambdaMergeK8, TiesCfg2.name: TiesCfg2, EvalCatalog.name: EvalCatalog,
              CollabStepCfg3.name: CollabStepCfg3, DistillStep.name: DistillStep, TiesSharded.name: TiesSharded,
+             PcbSharded.name: PcbSharded,
              TaskArithCfg1.name: TaskArithCfg1, MergeCfg4.name: MergeCfg4, EvalCfg1.name: EvalCfg1, EvalCfg4.name: EvalCfg4}
 DEFAULT_WORKLOAD = EvalCatalog.name

@@ -306,6 +306,33 @@ int mr_pcb_vectors(const float* base, const float* const* models, int K, int64_t
                    const float* clamp_hi, int64_t q_index, int flags, int32_t* status, float* out, int64_t ldo,
                    float* task_out, float* thr_out, void* ws, int64_t ws_bytes, mr_stream_t stream);
 
+/* Sharded PCB vectors, stream-ordered (no host synchronisation): mr_pcb_vectors over a flat vector whose columns are split
+ * over ranks, bit for bit the single-GPU result on this rank's columns.  Every quantity that spans columns is an order
+ * statistic of a model row (clamps, quantile, row maximum) and every float sum stays inside a column, so the search is
+ * the single-GPU one with its counters summed over the ranks: the sample is the whole vector's sample (each rank visits
+ * the share in its slice), and the fast / dense choice is taken from d_global.  The caller runs phases
+ * 0 .. n-1 in order on every rank (n and the collectives from mr_pcb_dist_plan) and, after phase p, applies to the
+ * workspace regions that mr_pcb_dist_layout reports (the library never communicates itself):
+ *   collectives[p] & MR_PCB_SUM: all-reduce(sum, as int32 words) of the sum region (histograms + below-window counts);
+ *   collectives[p] & MR_PCB_MAX: all-reduce(max, as int32 words) of the max region (row maxima + list-overflow flags).
+ * The last phase writes status (as mr_pcb_vectors; identical on every rank, since every decision is taken from reduced
+ * counts) and builds this slice's vectors into out (K rows, leading dimension ldo).  Slice [j_off, j_off + d_local):
+ * j_off a multiple of 32 (unless d_local == 0), the slice ends on a multiple of 32 or at d_global (then ATen's interleaved torch.sum(dim=0)
+ * order on the trailing d_global mod 32 columns falls on the last rank exactly as in the single-GPU kernel), d_global <
+ * 2^32; d_local == 0 is allowed (base / models / out may then be NULL: the rank contributes zero counts).  clamp_lo /
+ * clamp_hi / q_index / flags: the values of the WHOLE vector, the same on every rank.  ws: dev scratch of the size
+ * mr_pcb_dist_layout reports.  ref: merger/algorithms/pcb.py:37-58; SURVEY.md section 8(e) merger row. */
+enum { MR_PCB_SUM = 1, MR_PCB_MAX = 2 };
+int mr_pcb_dist_layout(int64_t d_local, int64_t d_global, int K, int64_t* ws_bytes, int64_t* sum_off, int64_t* sum_bytes,
+                       int64_t* max_off, int64_t* max_bytes);
+/* HOST helper (no device work): the number of phases (> 0) for d_global / flags; collectives[p] (p < cap) = the
+ * MR_PCB_SUM / MR_PCB_MAX bits of the all-reduces after phase p (0 after the last). */
+int mr_pcb_dist_plan(int64_t d_global, int flags, int32_t* collectives, int cap);
+int mr_pcb_vectors_dist(const float* base, const float* const* models, int K, int64_t d_local, int64_t j_off,
+                        int64_t d_global, const float* clamp_lo, const float* clamp_hi, int64_t q_index, int flags,
+                        int phase, int32_t* status, float* out, int64_t ldo, void* ws, int64_t ws_bytes,
+                        mr_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Sharded merger (SURVEY.md section 8(e)): the flat vector is split over ranks; the global TIES trim
  * (ref: merger/algorithms/ties.py:14-23, top-k over the WHOLE vector) is found by radix refinement of a window of

@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libmergerec_b200.so")
 MR_ORDER_BASE_FIRST, MR_ORDER_SUM_FIRST, MR_ORDER_LINEAR = 0, 1, 2
 MR_TIES_VECTORS, MR_TIES_TRIMSUM, MR_TIES_FUSED_MERGE, MR_TIES_LNS = 0, 1, 2, 3
 MR_PCB_DENSE, MR_PCB_IEEE = 1, 2
+MR_PCB_SUM, MR_PCB_MAX = 1, 2
 MR_MAX_K = 16
 MR_DISTILL_MAX_B, MR_DISTILL_MAX_GROUPS, MR_DISTILL_MAX_E = 128, 64, 1024
 
@@ -55,7 +56,10 @@ SIGNATURES = {
     "mr_normalize_rows": ([_vp, _i64, _i32, _vp, _vp], C.c_int),
     "mr_pcb_workspace_bytes": ([_i64, _i32], _i64),
     "mr_pcb_vectors": ([_vp, _vp, _i32, _i64, _vp, _vp, _i64, _i32, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp], C.c_int),
-    "mr_ties_mag_hist": ([_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp], C.c_int),
+    "mr_pcb_dist_layout": ([_i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "mr_pcb_dist_plan": ([_i64, _i32, _vp, _i32], C.c_int),
+    "mr_pcb_vectors_dist": ([_vp, _vp, _i32, _i64, _i64, _i64, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _i64, _vp, _i64, _vp], C.c_int),
+    "mr_ties_mag_hist":([_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp], C.c_int),
     "mr_ties_dist_layout": ([_i64, _i32, _vp, _vp, _vp, _vp], C.c_int),
     "mr_ties_select_dist": ([_vp, _vp, _i32, _i64, _i64, _i64, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_merge_dare": ([_vp, _vp, _i32, _i64, _vp, _vp, _i64, C.c_float, _vp, _vp], C.c_int),

@@ -147,7 +147,7 @@ __device__ __forceinline__ int pcb_load_quad(const float* __restrict__ base, con
 // plain stride of 32 would only ever see columns = 0 mod 32 of a 768- or 1024-wide row -- e.g. never, or always, an outlier
 // dimension of a transformer -- and a biased sample costs the fallback to the dense search).  Only whole blocks are sampled.
 __host__ __device__ __forceinline__ int64_t pcb_sample_count(int64_t d, int64_t stride) { return 4 * (d / (4 * stride)); }
-__device__ __forceinline__ int64_t pcb_sample_column(int64_t i, int64_t stride) {
+__host__ __device__ __forceinline__ int64_t pcb_sample_column(int64_t i, int64_t stride) {
     const int64_t c = i >> 2;
     const uint32_t h = ((uint32_t)c * 2654435761u) >> 16;
     return c * (4 * stride) + 4 * (int64_t)(h % (uint32_t)stride) + (i & 3);
@@ -155,12 +155,16 @@ __device__ __forceinline__ int64_t pcb_sample_column(int64_t i, int64_t stride) 
 
 // Radix pass over the columns (stride = 1) or over the sample (stride > 1) -- pass 0: bins = key >> 21 (+ row maxima); pass 1:
 // (key >> 10) & 2047 inside prefix; pass 2: key & 1023 inside prefix.  stride = 1: the dense search (all three passes);
-// stride > 1: the fast path's only pass over the sample (pass 0), which also caches the keys in skeys (K, n_s).
-template <int K>
+// stride > 1: the fast path's only pass over the sample (pass 0), which also caches the keys in skeys (K, n_vis).
+// SLICE (the sharded search's sample pass): the vector is columns j_off .. j_off + d - 1 of a longer one, and the pass
+// visits the elements s0 .. s0 + n_s - 1 of that vector's sample (pcb_slice_sample); otherwise s0 / j_off / n_s are
+// unused and the sweep is the whole-vector one, kept apart because the slice arithmetic costs the gather-bound sample
+// pass ~8 % (20 us at K = 8 BLaIR-base).
+template <int K, bool SLICE>
 __global__ void __launch_bounds__(kPcbThreads)
 pcb_hist_kernel(const float* __restrict__ base, PtrPack<K> m, int64_t d, int64_t stride, const float* __restrict__ lo,
                 const float* __restrict__ hi, int pass, PcbState* __restrict__ st, uint32_t* __restrict__ hist,
-                uint32_t* __restrict__ skeys, int ieee) {
+                uint32_t* __restrict__ skeys, int ieee, int64_t s0, int64_t j_off, int64_t n_s) {
     extern __shared__ uint32_t s_hist[];  // K * kPcbBins
     __shared__ PcbClamp<K> s_c;
     __shared__ uint32_t s_prefix[K];
@@ -173,14 +177,15 @@ pcb_hist_kernel(const float* __restrict__ base, PtrPack<K> m, int64_t d, int64_t
     for (int k = 0; k < K; ++k) mx[k] = 0;
     const int64_t tail0 = d & ~(int64_t)31;
     const int64_t span = (int64_t)gridDim.x * blockDim.x;
-    const int64_t n_vis = stride == 1 ? d : pcb_sample_count(d, stride);
+    const int64_t n_vis = SLICE ? n_s : (stride == 1 ? d : pcb_sample_count(d, stride));
     const int64_t rounds = (n_vis + span - 1) / span;  // every lane runs every round (the match below is warp-wide)
     auto sweep = [&](auto safe_tag) {
     constexpr bool SAFE = decltype(safe_tag)::value;
     for (int64_t it = 0; it < rounds; ++it) {
         const int64_t i = it * span + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
         const bool live = i < n_vis;
-        const int64_t j = !live ? 0 : (stride == 1 ? i : pcb_sample_column(i, stride));
+        const int64_t j = !live ? 0 : (SLICE ? pcb_sample_column(s0 + i, stride) - j_off
+                                             : (stride == 1 ? i : pcb_sample_column(i, stride)));
         float x[K], tau[K], A[K], task[K];
         const float b = live ? ldg_stream1(base + j) : 0.f;
 #pragma unroll
@@ -500,6 +505,23 @@ __global__ void pcb_init_kernel(PcbState* st, int K, int64_t rank0, int64_t rank
     }
 }
 
+// Sharded search: the row maxima and the window-overflow flags of every rank meet in a region that is all-reduced with MAX
+// as int32 words -- [maxkey ^ 0x80000000 (K) | miss (K)]: the xor maps the unsigned key order onto the signed order.
+__global__ void pcb_export_kernel(const PcbState* st, int K, int32_t* maxreg) {
+    const int k = threadIdx.x;
+    if (k < K) {
+        maxreg[k] = (int32_t)(st[k].maxkey ^ 0x80000000u);
+        maxreg[K + k] = st[k].miss;
+    }
+}
+__global__ void pcb_import_kernel(PcbState* st, int K, const int32_t* maxreg) {
+    const int k = threadIdx.x;
+    if (k < K) {
+        st[k].maxkey = (uint32_t)maxreg[k] ^ 0x80000000u;
+        st[k].miss = maxreg[K + k] != 0;
+    }
+}
+
 template <int K, bool VEC>
 __global__ void __launch_bounds__(kPcbThreads, K <= 8 ? 2 : 1)
 pcb_build_kernel(const float* __restrict__ base, PtrPack<K> m, int64_t d, const float* __restrict__ lo,
@@ -568,19 +590,20 @@ pcb_build_kernel(const float* __restrict__ base, PtrPack<K> m, int64_t d, const 
 
 static inline size_t pcb_align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// Workspace layout (sizes depend on d and K only, so the query function and the launch agree).
+// Workspace layout.  n_s: the sample keys cached here; n_s_win: the sample the window is derived from (the whole vector's,
+// which the per-warp lists are sized for).  Sizes depend on those, K and the SM count only, so query and launch agree.
 struct PcbWs {
     size_t state_off, hist_off, below_off, cnt_off, keys_off, skeys_off, total;
     int64_t n_s;          // sample size
     int64_t list_total;   // list capacity per model over all warps (in keys)
     int64_t max_lists;    // upper bound on the number of warp lists
 };
-static PcbWs pcb_layout(int64_t d, int K) {
+static PcbWs pcb_layout_n(int64_t n_s, int64_t n_s_win, int K) {
     PcbWs L;
-    L.n_s = pcb_sample_count(d, kPcbStride);
+    L.n_s = n_s;
     // sampling error of an order statistic of the sample: sigma <= sqrt(n_s) / 2 ranks; the window spans +-R = 6 sigma
     // + 16 sample ranks, i.e. about 2 R * stride elements of the full vector -- provisioned four times over
-    const int64_t r_max = (int64_t)(3.0 * sqrt((double)L.n_s)) + 16;
+    const int64_t r_max = (int64_t)(3.0 * sqrt((double)n_s_win)) + 16;
     L.max_lists = (int64_t)sm_count() * 8 * kPcbWarps;
     L.list_total = 4 * 2 * r_max * kPcbStride + 64 * L.max_lists;
     size_t off = 0;
@@ -592,6 +615,155 @@ static PcbWs pcb_layout(int64_t d, int K) {
     L.skeys_off = off; off += pcb_align256((size_t)K * L.n_s * sizeof(uint32_t));
     L.total = off;
     return L;
+}
+static PcbWs pcb_layout(int64_t d, int K) {
+    const int64_t n_s = pcb_sample_count(d, kPcbStride);
+    return pcb_layout_n(n_s, n_s, K);
+}
+// bytes of the histograms (both slots) and the below-window counters, which sit back to back
+static size_t pcb_counter_bytes(const PcbWs& L) { return L.below_off + (size_t)MR_MAX_K * sizeof(unsigned long long) - L.hist_off; }
+
+// The fast search runs where the sample is large enough to be worth it (small vectors: the dense passes are cheap and
+// exact anyway).  Sharded: decided from the WHOLE vector, so that every rank takes the same path.
+static bool pcb_fast(int64_t d, int flags) { return !(flags & MR_PCB_DENSE) && pcb_sample_count(d, kPcbStride) >= 4096; }
+
+// ranks of the window's ends inside the sample (the sample's quantile +- R, R = 6 sigma of the sampling error); an end
+// clipped to the sample is open
+static void pcb_window_ranks(int64_t q_index, int64_t d, int64_t n_s, int64_t* r_lo, int64_t* r_hi, int* lo_open, int* hi_open) {
+    const long double p = (long double)q_index / (long double)d;
+    const int64_t q_s = (int64_t)(p * (long double)n_s);
+    const int64_t R = (int64_t)(6.0 * sqrt((double)n_s * (double)(p * (1.0L - p)))) + 16;
+    *r_lo = q_s - R; *r_hi = q_s + R;
+    *lo_open = *hi_open = 0;
+    if (*r_lo < 0) { *r_lo = 0; *lo_open = 1; }
+    if (*r_hi > n_s - 1) { *r_hi = n_s - 1; *hi_open = 1; }
+}
+
+// The elements [s0, s0 + n) of the whole vector's sample that lie in the slice [j_off, j_off + d_local): every whole
+// block of 4 * stride columns inside the slice, plus a block straddling a slice boundary when its sampled quad falls
+// inside (quads are 4-aligned, slice boundaries 32-aligned or the vector's end: a quad never straddles one).  Over the
+// ranks of a sharded vector the ranges partition the sample.
+static void pcb_slice_sample(int64_t d_local, int64_t j_off, int64_t d_global, int64_t* s0, int64_t* n) {
+    const int64_t blk = 4 * kPcbStride;
+    int64_t c0 = j_off / blk, c1 = (j_off + d_local + blk - 1) / blk;
+    if (c1 > d_global / blk) c1 = d_global / blk;                  // only whole blocks are sampled
+    auto inside = [&](int64_t c) {
+        const int64_t j = pcb_sample_column(4 * c, kPcbStride);
+        return j >= j_off && j < j_off + d_local;
+    };
+    if (c0 < c1 && !inside(c0)) ++c0;
+    if (c0 < c1 && !inside(c1 - 1)) --c1;
+    if (c1 < c0) c1 = c0;
+    *s0 = 4 * c0;
+    *n = 4 * (c1 - c0);
+}
+
+// ---- launchers shared by the single-GPU and the sharded entry points ------------------------------------------------
+// n_vis: the elements the pass visits (d, or the sample size); slice != 0: the sharded sample pass (pcb_hist_kernel SLICE)
+template <int K>
+static void pcb_launch_hist(const float* base, const PtrPack<K>& pk, int64_t d, int64_t stride, int64_t n_vis, bool slice,
+                            int64_t s0, int64_t j_off, const float* lo, const float* hi, int pass, PcbState* state,
+                            uint32_t* hist, uint32_t* skeys, int ieee, cudaStream_t st) {
+    if (n_vis <= 0) return;
+    const size_t hist_bytes = (size_t)K * kPcbBins * sizeof(uint32_t);
+    int64_t hblocks = (n_vis + kPcbThreads - 1) / kPcbThreads;
+    const int64_t hcap = (int64_t)sm_count() * 3;         // one resident wave at K = 8 (64 KB of histograms per CTA)
+    if (hblocks > hcap) hblocks = hcap;
+    if (slice) {
+        cudaFuncSetAttribute(pcb_hist_kernel<K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes);
+        pcb_hist_kernel<K, true><<<(unsigned)hblocks, kPcbThreads, hist_bytes, st>>>(base, pk, d, stride, lo, hi, pass, state,
+                                                                                    hist, skeys, ieee, s0, j_off, n_vis);
+    } else {
+        cudaFuncSetAttribute(pcb_hist_kernel<K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes);
+        pcb_hist_kernel<K, false><<<(unsigned)hblocks, kPcbThreads, hist_bytes, st>>>(base, pk, d, stride, lo, hi, pass, state,
+                                                                                     hist, skeys, ieee, 0, 0, 0);
+    }
+}
+
+static void pcb_launch_keys_hist(const uint32_t* skeys, int64_t n_s, int K, int pass, const PcbState* state, uint32_t* hist,
+                                 cudaStream_t st) {
+    if (n_s <= 0) return;
+    int64_t kblocks = (n_s + kPcbThreads * 8 - 1) / (kPcbThreads * 8);
+    if (kblocks > sm_count()) kblocks = sm_count();
+    pcb_keys_hist_kernel<<<dim3((unsigned)kblocks, K), kPcbThreads, 0, st>>>(skeys, n_s, K, pass, state, hist);
+}
+
+// the pass over everything: one resident wave, one list per warp; the number of lists (0: nothing to do) -- the list
+// kernels of a search must use the count its window pass used
+template <int K>
+static int64_t pcb_window_lists(int64_t d, bool vec) {
+    if (d <= 0) return 0;
+    int occ = 1;
+    if (vec) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pcb_window_kernel<K, true>, kPcbThreads, 0);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pcb_window_kernel<K, false>, kPcbThreads, 0);
+    if (occ < 1) occ = 1;
+    if (occ > 8) occ = 8;
+    int64_t wblocks = (int64_t)sm_count() * occ;
+    const int64_t nq = (d + 3) >> 2;
+    if (wblocks > (nq + kPcbThreads - 1) / kPcbThreads) wblocks = (nq + kPcbThreads - 1) / kPcbThreads;
+    return wblocks * kPcbWarps;
+}
+static int pcb_list_cap(const PcbWs& L, int64_t n_lists) { return (int)((L.list_total / n_lists) & ~(int64_t)31); }
+
+template <int K>
+static void pcb_launch_window(const float* base, const PtrPack<K>& pk, int64_t d, bool vec, const float* lo, const float* hi,
+                              PcbState* state, unsigned long long* below, uint32_t* list_keys, uint32_t* list_cnt,
+                              int64_t n_lists, const PcbWs& L, int ieee, cudaStream_t st) {
+    if (!n_lists) return;
+    const unsigned wblocks = (unsigned)(n_lists / kPcbWarps);
+    const int list_cap = pcb_list_cap(L, n_lists);
+    if (vec)
+        pcb_window_kernel<K, true><<<wblocks, kPcbThreads, 0, st>>>(base, pk, d, lo, hi, state, below, list_keys, list_cnt,
+                                                                    list_cap, ieee);
+    else
+        pcb_window_kernel<K, false><<<wblocks, kPcbThreads, 0, st>>>(base, pk, d, lo, hi, state, below, list_keys, list_cnt,
+                                                                     list_cap, ieee);
+}
+
+static void pcb_launch_list_hist(int K, const uint32_t* list_keys, const uint32_t* list_cnt, int64_t n_lists, const PcbWs& L,
+                                 const PcbState* state, uint32_t* hist, cudaStream_t st) {
+    if (!n_lists) return;
+    int64_t lblocks = (n_lists + kPcbWarps - 1) / kPcbWarps;
+    if (lblocks > sm_count()) lblocks = sm_count();
+    pcb_list_hist_kernel<<<dim3((unsigned)lblocks, K), kPcbThreads, 0, st>>>(list_keys, list_cnt, n_lists, pcb_list_cap(L, n_lists),
+                                                                            state, hist);
+}
+
+template <int K>
+static void pcb_launch_build(const float* base, const PtrPack<K>& pk, int64_t d, bool vec, const float* lo, const float* hi,
+                             const PcbState* state, float* out, int64_t ldo, float* task_out, float* thr_out, int ieee,
+                             cudaStream_t st) {
+    if (d <= 0) return;
+    int64_t bblocks = (((d + 3) >> 2) + kPcbThreads - 1) / kPcbThreads;
+    if (bblocks > (int64_t)sm_count() * 8) bblocks = (int64_t)sm_count() * 8;
+    if (vec)
+        pcb_build_kernel<K, true><<<(unsigned)bblocks, kPcbThreads, 0, st>>>(base, pk, d, lo, hi, state, out, ldo, task_out,
+                                                                             thr_out, ieee);
+    else
+        pcb_build_kernel<K, false><<<(unsigned)bblocks, kPcbThreads, 0, st>>>(base, pk, d, lo, hi, state, out, ldo, task_out,
+                                                                              thr_out, ieee);
+}
+
+static bool pcb_vec(const float* base, const float* const* models, int K, const float* out, int64_t ldo, const float* task_out) {
+    bool vec = host_aligned16(base) && host_aligned16(out) && (ldo % 4 == 0) && (!task_out || host_aligned16(task_out));
+    for (int k = 0; k < K; ++k) vec = vec && host_aligned16(models[k]);
+    return vec;
+}
+
+// Sharded search: the workspace is the single-GPU one with the sample cache sized for the slice, the lists sized for
+// the whole vector's window, and the MAX region behind it.
+struct PcbDistWs {
+    PcbWs L;
+    size_t max_off, max_bytes, total;
+};
+static PcbDistWs pcb_dist_layout(int64_t d_local, int64_t d_global, int K) {
+    PcbDistWs D;
+    // a slice of d_local columns meets at most d_local / 128 + 2 sampled blocks
+    D.L = pcb_layout_n(4 * (d_local / (4 * kPcbStride) + 2), pcb_sample_count(d_global, kPcbStride), K);
+    D.max_off = D.L.total;
+    D.max_bytes = (size_t)2 * K * sizeof(int32_t);
+    D.total = D.max_off + pcb_align256(D.max_bytes);
+    return D;
 }
 
 }  // namespace mr
@@ -625,89 +797,200 @@ extern "C" int mr_pcb_vectors(const float* base, const float* const* models, int
     uint32_t* list_keys = reinterpret_cast<uint32_t*>(w + L.keys_off);
     uint32_t* skeys = reinterpret_cast<uint32_t*>(w + L.skeys_off);
     const size_t hist_bytes = (size_t)K * kPcbBins * sizeof(uint32_t);           // one histogram per model
-    const size_t hist_all = L.below_off + (size_t)MR_MAX_K * sizeof(unsigned long long) - L.hist_off;   // both slots + below
-    cudaMemsetAsync(hist, 0, hist_all, st);
+    cudaMemsetAsync(hist, 0, pcb_counter_bytes(L), st);                           // both slots + below
     const int64_t n_s = L.n_s;
     const int ieee = (flags & MR_PCB_IEEE) ? 1 : 0;
-    const bool fast = !(flags & MR_PCB_DENSE) && n_s >= 4096;   // small vectors: the dense passes are cheap and exact anyway
-    // fast: ranks of the window's ends inside the sample (the sample's quantile +- R, R = 6 sigma of the sampling error)
+    const bool fast = pcb_fast(d, flags);
     int64_t r_lo = q_index, r_hi = q_index;
     int lo_open = 0, hi_open = 0;
-    if (fast) {
-        const long double p = (long double)q_index / (long double)d;
-        const int64_t q_s = (int64_t)(p * (long double)n_s);
-        const int64_t R = (int64_t)(6.0 * sqrt((double)n_s * (double)(p * (1.0L - p)))) + 16;
-        r_lo = q_s - R; r_hi = q_s + R;
-        if (r_lo < 0) { r_lo = 0; lo_open = 1; }
-        if (r_hi > n_s - 1) { r_hi = n_s - 1; hi_open = 1; }
-    }
+    if (fast) pcb_window_ranks(q_index, d, n_s, &r_lo, &r_hi, &lo_open, &hi_open);
     pcb_init_kernel<<<1, 64, 0, st>>>(state, K, r_lo, r_hi);
-    bool vec = host_aligned16(base) && host_aligned16(out) && (ldo % 4 == 0) && (!task_out || host_aligned16(task_out));
-    for (int k = 0; k < K; ++k) vec = vec && host_aligned16(models[k]);
-    const int sms = sm_count();
+    const bool vec = pcb_vec(base, models, K, out, ldo, task_out);
     MR_DISPATCH_K(K, {
         PtrPack<KK> pk;
         for (int k = 0; k < KK; ++k) pk.p[k] = models[k];
-        cudaFuncSetAttribute(pcb_hist_kernel<KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes);
-        int64_t hblocks = ((fast ? n_s : d) + kPcbThreads - 1) / kPcbThreads;
-        const int64_t hcap = (int64_t)sms * 3;         // one resident wave at K = 8 (64 KB of histograms per CTA)
-        if (hblocks > hcap) hblocks = hcap;
         if (!fast) {
             for (int pass = 0; pass < 3; ++pass) {      // dense radix passes over everything
-                pcb_hist_kernel<KK><<<(unsigned)hblocks, kPcbThreads, hist_bytes, st>>>(base, pk, d, 1, clamp_lo, clamp_hi, pass,
-                                                                                       state, hist, nullptr, ieee);
+                pcb_launch_hist<KK>(base, pk, d, 1, d, false, 0, 0, clamp_lo, clamp_hi, pass, state, hist, nullptr, ieee, st);
                 pcb_pick_kernel<<<dim3(KK, 1), 256, 0, st>>>(pass, KK, 0, state, hist);
                 cudaMemsetAsync(hist, 0, hist_bytes, st);
             }
         } else {
             // the sample: one pass computes and caches its keys, passes 1 and 2 of both order statistics read the cache
-            pcb_hist_kernel<KK><<<(unsigned)hblocks, kPcbThreads, hist_bytes, st>>>(base, pk, d, kPcbStride, clamp_lo, clamp_hi, 0,
-                                                                                   state, hist, skeys, ieee);
+            pcb_launch_hist<KK>(base, pk, d, kPcbStride, n_s, false, 0, 0, clamp_lo, clamp_hi, 0, state, hist, skeys, ieee, st);
             pcb_pick_kernel<<<dim3(KK, kPcbSlots), 256, 0, st>>>(0, KK, 1, state, hist);
             cudaMemsetAsync(hist, 0, kPcbSlots * hist_bytes, st);
-            int64_t kblocks = (n_s + kPcbThreads * 8 - 1) / (kPcbThreads * 8);
-            if (kblocks > sms) kblocks = sms;
             for (int pass = 1; pass < 3; ++pass) {
-                pcb_keys_hist_kernel<<<dim3((unsigned)kblocks, KK), kPcbThreads, 0, st>>>(skeys, n_s, KK, pass, state, hist);
+                pcb_launch_keys_hist(skeys, n_s, KK, pass, state, hist, st);
                 pcb_pick_kernel<<<dim3(KK, kPcbSlots), 256, 0, st>>>(pass, KK, 0, state, hist);
                 cudaMemsetAsync(hist, 0, kPcbSlots * hist_bytes, st);
             }
             pcb_window_init_kernel<<<1, 32, 0, st>>>(state, KK, q_index, lo_open, hi_open);
-            // the pass over everything: one resident wave, one list per warp
-            int occ = 1;
-            if (vec) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pcb_window_kernel<KK, true>, kPcbThreads, 0);
-            else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pcb_window_kernel<KK, false>, kPcbThreads, 0);
-            if (occ < 1) occ = 1;
-            if (occ > 8) occ = 8;
-            int64_t wblocks = (int64_t)sms * occ;
-            const int64_t nq = (d + 3) >> 2;
-            if (wblocks > (nq + kPcbThreads - 1) / kPcbThreads) wblocks = (nq + kPcbThreads - 1) / kPcbThreads;
-            const int64_t n_lists = wblocks * kPcbWarps;
-            const int list_cap = (int)((L.list_total / n_lists) & ~(int64_t)31);
-            if (vec)
-                pcb_window_kernel<KK, true><<<(unsigned)wblocks, kPcbThreads, 0, st>>>(
-                    base, pk, d, clamp_lo, clamp_hi, state, below, list_keys, list_cnt, list_cap, ieee);
-            else
-                pcb_window_kernel<KK, false><<<(unsigned)wblocks, kPcbThreads, 0, st>>>(
-                    base, pk, d, clamp_lo, clamp_hi, state, below, list_keys, list_cnt, list_cap, ieee);
-            int64_t lblocks = (n_lists + kPcbWarps - 1) / kPcbWarps;
-            if (lblocks > sms) lblocks = sms;
+            const int64_t n_lists = pcb_window_lists<KK>(d, vec);
+            pcb_launch_window<KK>(base, pk, d, vec, clamp_lo, clamp_hi, state, below, list_keys, list_cnt, n_lists, L, ieee, st);
             for (int level = 0; level < 3; ++level) {   // 2048 bins x 2^21 keys cover the key space: three levels at most
-                pcb_list_hist_kernel<<<dim3((unsigned)lblocks, KK), kPcbThreads, 0, st>>>(list_keys, list_cnt, n_lists, list_cap,
-                                                                                         state, hist);
+                pcb_launch_list_hist(KK, list_keys, list_cnt, n_lists, L, state, hist, st);
                 pcb_window_pick_kernel<<<KK, 256, 0, st>>>(level == 0, state, hist, below);
             }
         }
         pcb_status_kernel<<<1, 32, 0, st>>>(state, KK, fast ? 1 : 0, ieee, clamp_lo, clamp_hi, status);
-        int64_t bblocks = (((d + 3) >> 2) + kPcbThreads - 1) / kPcbThreads;
-        if (bblocks > (int64_t)sms * 8) bblocks = (int64_t)sms * 8;
-        if (vec)
-            pcb_build_kernel<KK, true><<<(unsigned)bblocks, kPcbThreads, 0, st>>>(base, pk, d, clamp_lo, clamp_hi, state, out, ldo,
-                                                                                 task_out, thr_out, ieee);
-        else
-            pcb_build_kernel<KK, false><<<(unsigned)bblocks, kPcbThreads, 0, st>>>(base, pk, d, clamp_lo, clamp_hi, state, out, ldo,
-                                                                                  task_out, thr_out, ieee);
+        pcb_launch_build<KK>(base, pk, d, vec, clamp_lo, clamp_hi, state, out, ldo, task_out, thr_out, ieee, st);
     });
     MR_CUDA_LAUNCH_CHECK("mr_pcb_vectors");
+    return MR_OK;
+}
+
+// ---- sharded search ----------------------------------------------------------------------------------------------------
+// The same kernels over one rank's slice, split into phases at the points where the single-GPU search reads a count of
+// the whole vector.  After each phase but the last the caller all-reduces, over the ranks, the regions that
+// mr_pcb_dist_plan names (the library itself never communicates):
+//   fast search (7 phases)                                                     dense search (4 phases)
+//   0  init, sample pass (pass 0 over this slice's share of the sample)  SUM    0  init, dense pass 0, row maxima  SUM+MAX
+//   1  pick, pass 1 over the cached sample keys                          SUM    1  pick, dense pass 1              SUM
+//   2  pick, pass 2 over the cached sample keys                          SUM    2  pick, dense pass 2              SUM
+//   3  pick, window, full pass (below / lists / row maxima), level 0     SUM+MAX  3  pick, status, build
+//   4  pick (subtracts the global count below), list level 1             SUM
+//   5  pick, list level 2                                                SUM
+//   6  pick, status, build of this slice
+// SUM: the histograms and below-window counters (uint32 / uint64 counts of at most d_global < 2^32, summed as int32 words:
+// exact, the high words are zero); MAX: the row maxima and the list-overflow flags.  Every pick then reads the counts of
+// the whole vector, so every rank takes the same decisions and reports the same status; the sample is the whole vector's
+// sample (each rank visits its share, pcb_slice_sample), so the windows are the single-GPU windows.
+extern "C" int mr_pcb_dist_layout(int64_t d_local, int64_t d_global, int K, int64_t* ws_bytes, int64_t* sum_off,
+                                  int64_t* sum_bytes, int64_t* max_off, int64_t* max_bytes) {
+    using namespace mr;
+    MR_REQUIRE(K >= 1 && K <= MR_MAX_K, "mr_pcb_dist_layout: K=%d outside [1,%d]", K, MR_MAX_K);
+    MR_REQUIRE(ws_bytes && sum_off && sum_bytes && max_off && max_bytes, "mr_pcb_dist_layout: null pointer");
+    MR_REQUIRE(d_local >= 0 && d_local <= d_global && d_global < ((int64_t)1 << 32),
+               "mr_pcb_dist_layout: need 0 <= d_local <= d_global < 2^32");
+    const PcbDistWs D = pcb_dist_layout(d_local, d_global, K);
+    *ws_bytes = (int64_t)D.total;
+    *sum_off = (int64_t)D.L.hist_off;
+    *sum_bytes = (int64_t)pcb_counter_bytes(D.L);
+    *max_off = (int64_t)D.max_off;
+    *max_bytes = (int64_t)D.max_bytes;
+    return MR_OK;
+}
+
+extern "C" int mr_pcb_dist_plan(int64_t d_global, int flags, int32_t* collectives, int cap) {
+    using namespace mr;
+    MR_REQUIRE(d_global >= 1 && d_global < ((int64_t)1 << 32), "mr_pcb_dist_plan: d_global=%lld outside [1, 2^32)",
+               (long long)d_global);
+    MR_REQUIRE(cap >= 0 && (collectives || cap == 0), "mr_pcb_dist_plan: null pointer");
+    static const int32_t kFast[7] = {MR_PCB_SUM, MR_PCB_SUM, MR_PCB_SUM, MR_PCB_SUM | MR_PCB_MAX, MR_PCB_SUM, MR_PCB_SUM, 0};
+    static const int32_t kDense[4] = {MR_PCB_SUM | MR_PCB_MAX, MR_PCB_SUM, MR_PCB_SUM, 0};
+    const bool fast = pcb_fast(d_global, flags);
+    const int n = fast ? 7 : 4;
+    for (int p = 0; p < n && p < cap; ++p) collectives[p] = fast ? kFast[p] : kDense[p];
+    return n;
+}
+
+extern "C" int mr_pcb_vectors_dist(const float* base, const float* const* models, int K, int64_t d_local, int64_t j_off,
+                                   int64_t d_global, const float* clamp_lo, const float* clamp_hi, int64_t q_index, int flags,
+                                   int phase, int32_t* status, float* out, int64_t ldo, void* ws, int64_t ws_bytes,
+                                   mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE(K >= 1 && K <= MR_MAX_K, "mr_pcb_vectors_dist: K=%d outside [1,%d]", K, MR_MAX_K);
+    MR_REQUIRE(d_global >= 1 && d_global < ((int64_t)1 << 32), "mr_pcb_vectors_dist: d_global=%lld outside [1, 2^32)",
+               (long long)d_global);
+    MR_REQUIRE(d_local >= 0 && j_off >= 0 && j_off + d_local <= d_global,
+               "mr_pcb_vectors_dist: need 0 <= j_off, 0 <= d_local, j_off + d_local <= d_global");
+    MR_REQUIRE(j_off % 32 == 0 || d_local == 0, "mr_pcb_vectors_dist: j_off=%lld is not a multiple of 32", (long long)j_off);
+    MR_REQUIRE(d_local % 32 == 0 || j_off + d_local == d_global,
+               "mr_pcb_vectors_dist: a slice must end on a multiple of 32 columns or at d_global");
+    MR_REQUIRE(q_index >= 0 && q_index < d_global, "mr_pcb_vectors_dist: quantile index %lld outside [0,d_global)",
+               (long long)q_index);
+    const bool fast = pcb_fast(d_global, flags);
+    const int n_phases = fast ? 7 : 4;
+    MR_REQUIRE(phase >= 0 && phase < n_phases, "mr_pcb_vectors_dist: phase %d outside [0,%d)", phase, n_phases);
+    MR_REQUIRE(clamp_lo && clamp_hi && status && ws, "mr_pcb_vectors_dist: null pointer");
+    MR_REQUIRE(d_local == 0 || (base && models && out), "mr_pcb_vectors_dist: null pointer");
+    MR_REQUIRE(d_local == 0 || ldo >= d_local, "mr_pcb_vectors_dist: need ldo >= d_local");
+    for (int k = 0; d_local > 0 && k < K; ++k) MR_REQUIRE(models[k] != nullptr, "mr_pcb_vectors_dist: models[%d] is NULL", k);
+    const PcbDistWs D = pcb_dist_layout(d_local, d_global, K);
+    if (ws_bytes < (int64_t)D.total) {
+        set_error("mr_pcb_vectors_dist: workspace too small (%lld < %lld bytes)", (long long)ws_bytes, (long long)D.total);
+        return MR_ERR_WORKSPACE;
+    }
+    const PcbWs& L = D.L;
+    cudaStream_t st = (cudaStream_t)stream;
+    char* w = reinterpret_cast<char*>(ws);
+    PcbState* state = reinterpret_cast<PcbState*>(w + L.state_off);
+    uint32_t* hist = reinterpret_cast<uint32_t*>(w + L.hist_off);
+    unsigned long long* below = reinterpret_cast<unsigned long long*>(w + L.below_off);
+    uint32_t* list_cnt = reinterpret_cast<uint32_t*>(w + L.cnt_off);
+    uint32_t* list_keys = reinterpret_cast<uint32_t*>(w + L.keys_off);
+    uint32_t* skeys = reinterpret_cast<uint32_t*>(w + L.skeys_off);
+    int32_t* maxreg = reinterpret_cast<int32_t*>(w + D.max_off);
+    const size_t hist_bytes = (size_t)K * kPcbBins * sizeof(uint32_t);
+    const int ieee = (flags & MR_PCB_IEEE) ? 1 : 0;
+    int64_t s0 = 0, n_s = 0;                                 // this slice's share of the whole vector's sample
+    pcb_slice_sample(d_local, j_off, d_global, &s0, &n_s);
+    int64_t r_lo = q_index, r_hi = q_index;
+    int lo_open = 0, hi_open = 0;
+    if (fast) pcb_window_ranks(q_index, d_global, pcb_sample_count(d_global, kPcbStride), &r_lo, &r_hi, &lo_open, &hi_open);
+    const bool vec = d_local > 0 && pcb_vec(base, models, K, out, ldo, nullptr);
+    MR_DISPATCH_K(K, {
+        PtrPack<KK> pk;
+        for (int k = 0; k < KK; ++k) pk.p[k] = d_local > 0 ? models[k] : nullptr;
+        if (!fast) {
+            switch (phase) {
+                case 0:
+                    cudaMemsetAsync(hist, 0, pcb_counter_bytes(L), st);
+                    pcb_init_kernel<<<1, 64, 0, st>>>(state, KK, r_lo, r_hi);
+                    pcb_launch_hist<KK>(base, pk, d_local, 1, d_local, false, 0, 0, clamp_lo, clamp_hi, 0, state, hist, nullptr, ieee, st);
+                    pcb_export_kernel<<<1, 32, 0, st>>>(state, KK, maxreg);
+                    break;
+                case 1:
+                case 2:
+                    if (phase == 1) pcb_import_kernel<<<1, 32, 0, st>>>(state, KK, maxreg);
+                    pcb_pick_kernel<<<dim3(KK, 1), 256, 0, st>>>(phase - 1, KK, 0, state, hist);
+                    cudaMemsetAsync(hist, 0, hist_bytes, st);
+                    pcb_launch_hist<KK>(base, pk, d_local, 1, d_local, false, 0, 0, clamp_lo, clamp_hi, phase, state, hist, nullptr, ieee, st);
+                    break;
+                default:
+                    pcb_pick_kernel<<<dim3(KK, 1), 256, 0, st>>>(2, KK, 0, state, hist);
+                    pcb_status_kernel<<<1, 32, 0, st>>>(state, KK, 0, ieee, clamp_lo, clamp_hi, status);
+                    pcb_launch_build<KK>(base, pk, d_local, vec, clamp_lo, clamp_hi, state, out, ldo, nullptr, nullptr, ieee, st);
+                    break;
+            }
+        } else {
+            switch (phase) {
+                case 0:
+                    cudaMemsetAsync(hist, 0, pcb_counter_bytes(L), st);
+                    pcb_init_kernel<<<1, 64, 0, st>>>(state, KK, r_lo, r_hi);
+                    pcb_launch_hist<KK>(base, pk, d_local, kPcbStride, n_s, true, s0, j_off, clamp_lo, clamp_hi, 0, state, hist, skeys,
+                                        ieee, st);
+                    break;
+                case 1:
+                case 2:
+                    pcb_pick_kernel<<<dim3(KK, kPcbSlots), 256, 0, st>>>(phase - 1, KK, phase == 1 ? 1 : 0, state, hist);
+                    cudaMemsetAsync(hist, 0, kPcbSlots * hist_bytes, st);
+                    pcb_launch_keys_hist(skeys, n_s, KK, phase, state, hist, st);
+                    break;
+                case 3:
+                    pcb_pick_kernel<<<dim3(KK, kPcbSlots), 256, 0, st>>>(2, KK, 0, state, hist);
+                    cudaMemsetAsync(hist, 0, kPcbSlots * hist_bytes, st);
+                    pcb_window_init_kernel<<<1, 32, 0, st>>>(state, KK, q_index, lo_open, hi_open);
+                    pcb_launch_window<KK>(base, pk, d_local, vec, clamp_lo, clamp_hi, state, below, list_keys, list_cnt,
+                                          pcb_window_lists<KK>(d_local, vec), L, ieee, st);
+                    pcb_export_kernel<<<1, 32, 0, st>>>(state, KK, maxreg);
+                    pcb_launch_list_hist(KK, list_keys, list_cnt, pcb_window_lists<KK>(d_local, vec), L, state, hist, st);
+                    break;
+                case 4:
+                case 5:
+                    if (phase == 4) pcb_import_kernel<<<1, 32, 0, st>>>(state, KK, maxreg);
+                    pcb_window_pick_kernel<<<KK, 256, 0, st>>>(phase == 4, state, hist, below);
+                    pcb_launch_list_hist(KK, list_keys, list_cnt, pcb_window_lists<KK>(d_local, vec), L, state, hist, st);
+                    break;
+                default:
+                    pcb_window_pick_kernel<<<KK, 256, 0, st>>>(0, state, hist, below);
+                    pcb_status_kernel<<<1, 32, 0, st>>>(state, KK, 1, ieee, clamp_lo, clamp_hi, status);
+                    pcb_launch_build<KK>(base, pk, d_local, vec, clamp_lo, clamp_hi, state, out, ldo, nullptr, nullptr, ieee, st);
+                    break;
+            }
+        }
+    });
+    MR_CUDA_LAUNCH_CHECK("mr_pcb_vectors_dist");
     return MR_OK;
 }

@@ -24,12 +24,19 @@ from ..types import FlattenedModel
 from ._common import as_rows, merge_axpy, weights_tensor
 from .ties import select_kth_largest
 
-__all__ = ["get_pcb_vectors", "merge_pcb"]
+__all__ = ["get_pcb_vectors", "merge_pcb", "pcb_clamp_ranks"]
 
 
 def _magnitude_of(cut: torch.Tensor) -> torch.Tensor:
     """fp32 magnitude held in the high word of the selection keys."""
     return (cut >> 32).to(torch.int32).view(torch.float32)
+
+
+def pcb_clamp_ranks(d: int):
+    """(i_lo, i_hi): ascending ranks of the 1 % / 99 % magnitude clamps in a row of d (pcb.py:20-21 with min_ratio =
+    max_ratio = 0.01); i_hi wraps like the reference's `sorted_x[-1]` indexing for tiny d."""
+    i_lo, i_hi = int(d * 0.01), int(d * (1 - 0.01) - 1)
+    return i_lo, (i_hi if i_hi >= 0 else d + i_hi)
 
 
 def get_pcb_vectors(base_model: FlattenedModel, models: List[FlattenedModel], density: float = 0.2,
@@ -38,8 +45,7 @@ def get_pcb_vectors(base_model: FlattenedModel, models: List[FlattenedModel], de
     rows = as_rows(models)
     K, d = len(rows), base_model.numel()
     dev = base_model.device
-    i_lo, i_hi = int(d * 0.01), int(d * (1 - 0.01) - 1)          # pcb.py:20-21 with min_ratio = max_ratio = 0.01
-    i_hi = i_hi if i_hi >= 0 else d + i_hi                       # sorted_x[-1] for tiny d, like the reference's indexing
+    i_lo, i_hi = pcb_clamp_ranks(d)
     def clamps(defer: bool):
         """1 % / 99 % magnitude clamps (exact order statistics of |tau_k|) and the deferred select statuses."""
         sts = []

@@ -9,6 +9,10 @@ on the trailing `d mod 32` columns falls entirely on the last rank, exactly wher
   radix passes (`mr_ties_mag_hist`) whose (K, 2048) int64 histograms are summed with ONE all-reduce per pass; when
   equal magnitudes straddle the cut, an all-gather of the per-rank tie counts and an exclusive scan in rank order keep
   the lowest GLOBAL indices (the canonical tie rule) -- the result is bit-identical to the single-GPU merge;
+* PCB (pcb.py) needs three order statistics per model row -- the 1 % / 99 % magnitude clamps (the sharded select above)
+  and the quantile and maximum of the balancing weights (`DistPcb`: the single-GPU search with all-reduced histograms) --
+  and is otherwise column-local, so it is bit-identical to the single-GPU merge too;
+* DARE is column-local given the keep masks: every rank reads its columns of the (K, d) masks;
 * `gather_flat` (one all-gather of the merged slices) rebuilds the full vector where a caller wants it on every rank.
 
 One process per GPU, `torch.distributed` (NCCL over NVLink) for the collectives; with the gloo backend the small
@@ -18,18 +22,21 @@ from __future__ import annotations
 
 from typing import List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from .. import _lib
 from .algorithms import ties as _ties
 from .algorithms._common import as_rows, merge_axpy, weights_tensor
+from .algorithms.pcb import _magnitude_of, pcb_clamp_ranks
 from .layout import alloc_rows
-from .merger import ModelMerger
+from .merger import _NEEDS_BASE, ModelMerger
 from .types import StateDict
 from .utils.model_operations import unflatten_model
 
 __all__ = ["flat_shard_bounds", "sharded_select", "sharded_select_fast", "DistSelect", "get_ties_vectors_sharded", "merge_ties_sharded",
-           "merge_task_vector_sharded", "merge_linear_sharded", "gather_flat", "ShardedModelMerger", "CudaKernels"]
+           "merge_task_vector_sharded", "merge_linear_sharded", "DistPcb", "get_pcb_vectors_sharded", "merge_pcb_sharded",
+           "merge_dare_sharded", "gather_flat", "ShardedModelMerger", "CudaKernels"]
 
 BINS = 2048
 
@@ -68,6 +75,19 @@ def _all_reduce_sum(t: torch.Tensor, group) -> torch.Tensor:
         t.copy_(c)
     else:
         dist.all_reduce(t, group=group)
+    return t
+
+
+def _all_reduce_max(t: torch.Tensor, group) -> torch.Tensor:
+    if group is None:
+        return t
+    import torch.distributed as dist
+    if _host_hop(t, group):
+        c = t.cpu()
+        dist.all_reduce(c, op=dist.ReduceOp.MAX, group=group)
+        t.copy_(c)
+    else:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
     return t
 
 
@@ -213,7 +233,8 @@ def _ceil_log2(x: torch.Tensor) -> torch.Tensor:
 
 
 def sharded_select(base_l: torch.Tensor, rows_l: Sequence[torch.Tensor], k_cnt: int, d_global: int,
-                   w: Optional[torch.Tensor] = None, group=None, kernels=CudaKernels, defer_status: bool = False):
+                   w: Optional[torch.Tensor] = None, group=None, kernels=CudaKernels, defer_status: bool = False,
+                   magnitude: bool = False):
     """Per-model cut keys FOR THIS RANK'S SLICE (int64 (K,), bit pattern of the uint64 `mr_ties_build` expects with
     LOCAL indices) such that, over all ranks, exactly the `k_cnt` largest `|w_k (m_k - base)|` of the whole vector
     survive, equal magnitudes resolved towards the lowest global index.
@@ -231,7 +252,10 @@ def sharded_select(base_l: torch.Tensor, rows_l: Sequence[torch.Tensor], k_cnt: 
        rank k -> that bin becomes the next window, 11 bits finer; repeat until a bin is a single bit pattern (one level
        when the shards have the same statistics, up to three for the full range); the last level also records
        (bin, index) of its in-window elements;
-    3. all-gather of the per-rank counts AT the cut magnitude, exclusive scan in rank order: lowest global index first."""
+    3. all-gather of the per-rank counts AT the cut magnitude, exclusive scan in rank order: lowest global index first.
+
+    `magnitude=True` returns the cut's magnitude bit pattern (int64 (K,), the same on every rank) from the exact search
+    instead, without step 3 (the fallback of the PCB clamps after a deferred select reported a miss)."""
     K, dev = len(rows_l), base_l.device
     world, rank = _world(group)
     if k_cnt <= 0:
@@ -239,7 +263,7 @@ def sharded_select(base_l: torch.Tensor, rows_l: Sequence[torch.Tensor], k_cnt: 
     if k_cnt >= d_global:
         return torch.zeros(K, dtype=torch.int64, device=dev)                # everything survives
     lo_r, hi_r = flat_shard_bounds(d_global, world, rank)
-    if (kernels is CudaKernels and base_l.is_cuda and base_l.numel() == hi_r - lo_r
+    if (not magnitude and kernels is CudaKernels and base_l.is_cuda and base_l.numel() == hi_r - lo_r
             and (group is None or not _host_hop(base_l, group))):
         # product path: the stream-ordered device-side select; its status is the only thing the host looks at.  Every
         # rank reaches the same verdict (the brackets are decided from all-reduced counters), so the fallback below is
@@ -339,6 +363,8 @@ def sharded_select(base_l: torch.Tensor, rows_l: Sequence[torch.Tensor], k_cnt: 
             break
     else:
         raise _lib.MergeRecLibraryError("sharded TIES select did not converge")
+    if magnitude:
+        return mag
     counts = _all_gather(mine, group)                                        # (world, K)
     before = counts[:rank].sum(0) if rank > 0 else torch.zeros_like(mine)
     keep = torch.minimum((left - before).clamp(min=0), mine)                 # how many of MY ties survive
@@ -405,6 +431,215 @@ def merge_linear_sharded(models_l, weights: Sequence[float], kernels=CudaKernels
     return kernels.merge(None, rows, weights_tensor(weights, rows[0].device), _lib.MR_ORDER_LINEAR, False)
 
 
+class DistPcb:
+    """One rank's side of the stream-ordered sharded PCB search (`mr_pcb_vectors_dist`): the single-GPU quantile search of
+    `mr_pcb_vectors` (sample, key window, one pass over everything, list refinement; or the three dense passes) with every
+    histogram and counter summed over the ranks and the row maxima reduced with MAX, then the build of this rank's
+    columns.  No host synchronisation: per phase one library call and up to two all-reduces on views of the workspace.
+
+        pcb = DistPcb(base_l, rows_l, d_global, j_off, flags)
+        for phase, coll in enumerate(pcb.collectives):
+            pcb.run(phase, clamp_lo, clamp_hi, q_index)
+            if coll & MR_PCB_SUM:  all-reduce(sum) of pcb.sum    # int32 words
+            if coll & MR_PCB_MAX:  all-reduce(max) of pcb.max    # int32 words
+        pcb.out, pcb.status                                      # status as for mr_pcb_vectors, the same on every rank
+
+    `get_pcb_vectors_sharded` drives it with torch.distributed; tests drive several instances on one GPU by reducing the
+    views themselves."""
+
+    def __init__(self, base_l: torch.Tensor, rows_l: Sequence[torch.Tensor], d_global: int, j_off: int, flags: int = 0):
+        import ctypes as C
+        lib = _lib.load()
+        self.base, self.rows = base_l, list(rows_l)
+        self.K, self.d_local, self.d_global, self.j_off = len(self.rows), base_l.numel(), int(d_global), int(j_off)
+        dev = base_l.device
+        offs = [C.c_int64() for _ in range(5)]
+        _lib.check(lib.mr_pcb_dist_layout(self.d_local, self.d_global, self.K, *[C.byref(o) for o in offs]), "mr_pcb_dist_layout")
+        self.ws_bytes, s_off, s_bytes, m_off, m_bytes = (int(o.value) for o in offs)
+        self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
+        self.sum = self.ws[s_off:s_off + s_bytes].view(torch.int32)
+        self.max = self.ws[m_off:m_off + m_bytes].view(torch.int32)
+        self.out = alloc_rows(self.K, self.d_local, dev)
+        self.status = torch.zeros(self.K, dtype=torch.int32, device=dev)
+        self._parr = _lib.ptr_array(self.rows) if self.d_local else None
+        self.set_flags(flags)
+
+    def set_flags(self, flags: int) -> None:
+        """MR_PCB_DENSE / MR_PCB_IEEE for the next search (the phases and their collectives follow from them)."""
+        import ctypes as C
+        lib = _lib.load()
+        self.flags = int(flags)
+        n = lib.mr_pcb_dist_plan(self.d_global, self.flags, None, 0)
+        _lib.check(min(n, 0), "mr_pcb_dist_plan")
+        plan = (C.c_int32 * n)()
+        lib.mr_pcb_dist_plan(self.d_global, self.flags, plan, n)
+        self.collectives = [int(c) for c in plan]
+
+    def run(self, phase: int, clamp_lo: torch.Tensor, clamp_hi: torch.Tensor, q_index: int) -> None:
+        rc = _lib.load().mr_pcb_vectors_dist(
+            _lib.dptr(self.base, torch.float32) if self.d_local else None, self._parr, self.K, self.d_local, self.j_off,
+            self.d_global, _lib.dptr(clamp_lo, torch.float32), _lib.dptr(clamp_hi, torch.float32), int(q_index), self.flags,
+            phase, _lib.dptr(self.status), _lib.dptr(self.out) if self.d_local else None, max(self.out.stride(0), self.d_local),
+            _lib.dptr(self.ws), self.ws_bytes, _lib.stream_handle())
+        _lib.check(rc, "mr_pcb_vectors_dist")
+
+
+def _dist_select_global(base_l, rows_l, k_cnt: int, d_global: int, j_off: int, group):
+    """(global cut keys, status) of `DistSelect` with host-hop aware collectives (also over gloo with CUDA tensors)."""
+    world, _ = _world(group)
+    sel = DistSelect(base_l, rows_l, k_cnt, d_global, j_off)
+    gathered = None
+    for phase in range(DistSelect.PHASES):
+        sel.run(phase, gathered, world)
+        if world > 1 and phase < 4:
+            _all_reduce_sum(sel.counters, group)
+        elif world > 1 and phase == 4:
+            gathered = _all_gather(sel.survivors, group).reshape(-1)
+    return sel.cut_global, sel.status
+
+
+def get_pcb_vectors_sharded(base_l: torch.Tensor, models_l, density: float, d_global: int, group=None,
+                            force_dense: bool = False, force_ieee: bool = False) -> torch.Tensor:
+    """This rank's columns of `get_pcb_vectors` (pcb.py:37-58) of the whole vector, bit for bit: (K, d_local).
+
+    The magnitude clamps are global order statistics of |tau_k| (the sharded select; the row minimum, all-reduced, for
+    d_global < 100), the quantile and maximum of the balancing weights come from `DistPcb`, everything else is per
+    column.  Like the single-GPU call, the common case synchronises the host once: both selects run deferred, then the
+    search and the build; the statuses are reduced over the ranks and read together, and a miss reruns the affected
+    step on every rank (exact select; dense passes; IEEE divides)."""
+    rows = as_rows(models_l)
+    K, d = len(rows), base_l.numel()
+    dev = base_l.device
+    world, rank = _world(group)
+    lo_r, hi_r = flat_shard_bounds(d_global, world, rank)
+    if d != hi_r - lo_r:
+        raise ValueError(f"rank {rank} holds {d} columns, flat_shard_bounds gives [{lo_r}, {hi_r})")
+    i_lo, i_hi = pcb_clamp_ranks(d_global)
+
+    def magnitude(k_cnt: int, defer: bool):
+        """fp32 (K,) magnitude of the k_cnt-th largest |tau_k| over the whole vector, and the deferred select status."""
+        if k_cnt >= d_global:       # the single-GPU select answers "keep everything" with cut 0
+            return torch.zeros(K, dtype=torch.float32, device=dev), None
+        if defer:
+            cut, st_ = _dist_select_global(base_l, rows, k_cnt, d_global, lo_r, group)
+            return _magnitude_of(cut).contiguous(), st_
+        mag = sharded_select(base_l, rows, k_cnt, d_global, None, group, magnitude=True)
+        return mag.to(torch.int32).view(torch.float32).contiguous(), None
+
+    def clamps(defer: bool):
+        sts = []
+        if i_lo == 0:
+            # d_global < 100: the row minimum of |tau| (pcb.py:20), -max(-x) over the ranks, +inf for an empty slice
+            mins = [(r - base_l).abs().min() if d else torch.tensor(float("inf"), device=dev) for r in rows]
+            lo_ = _all_reduce_max(-torch.stack(mins).to(torch.float32), group).neg().contiguous()
+        else:
+            lo_, st_ = magnitude(d_global - i_lo, defer)
+            sts.append(st_)
+        hi_, st_ = magnitude(d_global - i_hi, defer)
+        sts.append(st_)
+        return lo_, hi_, [s for s in sts if s is not None]
+
+    q_index = int(d_global * (1 - density))                      # pcb.py:53
+    flags = _lib.MR_PCB_DENSE if force_dense else 0
+    if force_ieee:
+        flags |= _lib.MR_PCB_IEEE
+    pcb = DistPcb(base_l, rows, d_global, lo_r, flags)
+
+    def search(lo_, hi_, flags_: int) -> None:
+        pcb.set_flags(flags_)
+        for phase, coll in enumerate(pcb.collectives):
+            pcb.run(phase, lo_, hi_, q_index)
+            if world > 1 and coll & _lib.MR_PCB_SUM:
+                _all_reduce_sum(pcb.sum, group)
+            if world > 1 and coll & _lib.MR_PCB_MAX:
+                _all_reduce_max(pcb.max, group)
+
+    def verdict(sel_status):
+        """[a select missed, the window missed (status 0), the range needs IEEE divides (status 2)], MAX over the ranks:
+        the one host synchronisation of the common case."""
+        sel_bad = torch.stack([(s != 1).any() for s in sel_status]).any() if sel_status else torch.zeros((), dtype=torch.bool, device=dev)
+        v = torch.stack([sel_bad, (pcb.status == 0).any(), (pcb.status == 2).any()]).to(torch.int32)
+        return [bool(x) for x in _all_reduce_max(v, group).cpu()]
+
+    lo, hi, sel_status = clamps(defer=True)
+    search(lo, hi, flags)
+    sel_bad, miss, rng = verdict(sel_status)
+    if sel_bad:
+        lo, hi, _ = clamps(defer=False)
+        search(lo, hi, flags)
+        _, miss, rng = verdict([])
+    for _ in range(2):          # at most: window missed -> dense, then range -> IEEE (or the other way round)
+        if not (miss or rng):
+            break
+        if miss:
+            if flags & _lib.MR_PCB_DENSE:
+                raise _lib.MergeRecLibraryError("PCB quantile search failed")
+            flags |= _lib.MR_PCB_DENSE
+        if rng:
+            flags |= _lib.MR_PCB_IEEE
+        search(lo, hi, flags)
+        _, miss, rng = verdict([])
+    else:
+        if miss or rng:
+            raise _lib.MergeRecLibraryError(f"PCB vectors failed with status {pcb.status.cpu().tolist()}")
+    return pcb.out
+
+
+def merge_pcb_sharded(base_l: torch.Tensor, models_l, weights: Sequence[float], density: float, d_global: int,
+                      group=None) -> torch.Tensor:
+    """This rank's columns of `merge_pcb` (pcb.py:61-73): the sharded PCB vectors, then base-first accumulation."""
+    assert len(models_l) == len(weights), "Number of models and weights should match."
+    vectors = get_pcb_vectors_sharded(base_l, models_l, density, d_global, group)
+    if not base_l.numel():
+        return torch.empty_like(base_l)
+    return merge_axpy(base_l, list(vectors.unbind(0)), weights_tensor(weights, base_l.device), _lib.MR_ORDER_BASE_FIRST, False)
+
+
+def merge_dare_sharded(base_l: torch.Tensor, models_l, weights: Sequence[float], density: float, d_global: int,
+                       masks: Optional[torch.Tensor] = None, generator: Optional[torch.Generator] = None,
+                       group=None) -> torch.Tensor:
+    """This rank's columns of `merge_dare` (dare.py:9-31), bit for bit.  DARE is column-local given the keep masks:
+
+    * `masks=` (K, d_global), on any device: this rank reads its columns -- in place (leading dimension d_global) when
+      the masks are a bool / uint8 tensor on this device, otherwise only its slice is converted and copied;
+    * no masks: the whole (K, d_global) mask is drawn from `generator` exactly as `merge_dare` draws it and this rank
+      keeps its columns, so equal seeds on every rank give the single-GPU bits.  That costs each rank the transient
+      K * d_global * 4 bytes the single-GPU merge pays."""
+    assert len(models_l) == len(weights), "Number of models and weights should match."
+    p = float(density)
+    if p < 0.0 or p > 1.0:
+        raise ValueError(f"dropout probability has to be between 0 and 1, but got {p}")
+    K, d = len(models_l), base_l.numel()
+    if masks is not None and masks.shape != (K, d_global):
+        raise ValueError(f"masks must have shape {(K, d_global)}, got {tuple(masks.shape)}")
+    rows = as_rows(models_l)
+    dev = base_l.device
+    world, rank = _world(group)
+    lo, hi = flat_shard_bounds(d_global, world, rank)
+    if d != hi - lo:
+        raise ValueError(f"rank {rank} holds {d} columns, flat_shard_bounds gives [{lo}, {hi})")
+    if masks is None:
+        masks = torch.empty((K, d_global), dtype=torch.float32, device=dev).bernoulli_(1.0 - p, generator=generator) != 0
+    if p == 1.0:                 # torch: `input * zeros`
+        keep, scale = torch.zeros((K, d), dtype=torch.uint8, device=dev), 0.0
+    elif p == 0.0:               # torch returns the input unchanged
+        keep, scale = torch.ones((K, d), dtype=torch.uint8, device=dev), 1.0
+    else:
+        scale = float(np.float32(1.0) / np.float32(1.0 - p))      # `noise.div_(1 - p)` on an fp32 tensor
+        if masks.device == dev and masks.dtype in (torch.bool, torch.uint8) and masks.stride(1) == 1:
+            keep = masks.view(torch.uint8)[:, lo:hi]                 # read in place
+        else:
+            keep = masks[:, lo:hi].to(device=dev).to(torch.uint8).contiguous()
+    out = torch.empty_like(base_l)
+    if not d:
+        return out
+    w = weights_tensor(weights, dev)
+    rc = _lib.load().mr_merge_dare(_lib.dptr(base_l, torch.float32), _lib.ptr_array(rows), K, d, _lib.dptr(w),
+                                   _lib.dptr(keep), keep.stride(0), scale, _lib.dptr(out), _lib.stream_handle())
+    _lib.check(rc, "mr_merge_dare")
+    return out
+
+
 def gather_flat(local: torch.Tensor, d_global: int, group=None) -> torch.Tensor:
     """All ranks' slices -> the full flat vector on every rank (one all-gather; slices padded to the largest)."""
     world, rank = _world(group)
@@ -420,8 +655,10 @@ def gather_flat(local: torch.Tensor, d_global: int, group=None) -> torch.Tensor:
 
 class ShardedModelMerger(ModelMerger):
     """`ModelMerger` (merger/merger.py:10-93) whose flat vectors are sharded over the ranks of `group`.  Same
-    constructor and `merge(merge_type, weights, **kwargs)` contract for "linear", "task_vector" and "ties"; the merged
-    state_dict returned on every rank is bit-identical to the single-GPU one."""
+    constructor and `merge(merge_type, weights, **kwargs)` contract for every merge type ("linear", "task_vector",
+    "ties", "pcb", "dare"); the merged state_dict returned on every rank is bit-identical to the single-GPU one.  "dare"
+    without `masks=` draws the whole mask from `generator` on every rank (`merge_dare_sharded`): pass generators with
+    the same seed on every rank to get the single-GPU bits."""
 
     def __init__(self, models: Sequence[StateDict], base_model: Optional[StateDict] = None, align_key_order: bool = True,
                  group=None):
@@ -441,16 +678,22 @@ class ShardedModelMerger(ModelMerger):
             weights = [weights] * len(self.models)
         elif not (isinstance(weights, list) and all(isinstance(w, float) for w in weights)):
             raise ValueError("Weights should be a float or a list of floats.")
-        if merge_type in ("task_vector", "ties") and self.base_model is None:
-            raise ValueError(f"{'Task vector' if merge_type == 'task_vector' else 'TIES'} merge requires a base model.")
+        if merge_type in _NEEDS_BASE and self.base_model is None:
+            raise ValueError(f"{_NEEDS_BASE[merge_type]} merge requires a base model.")
         if merge_type == "linear":
             local = merge_linear_sharded(self.models, weights)
         elif merge_type == "task_vector":
             local = merge_task_vector_sharded(self.base_model, self.models, weights)
         elif merge_type == "ties":
             local = merge_ties_sharded(self.base_model, self.models, weights, kwargs["density"], self.d_global, self.group)
-        elif merge_type in ("dare", "pcb"):
-            raise NotImplementedError(f"Merge type '{merge_type}' has no sharded implementation.")
+        elif merge_type == "pcb":
+            local = merge_pcb_sharded(self.base_model, self.models, weights, kwargs.get("density", 0.2), self.d_global,
+                                      self.group)
+        elif merge_type == "dare":
+            if "density" not in kwargs:       # what ModelMerger's call of merge_dare raises
+                raise TypeError("merge_dare() missing 1 required positional argument: 'density'")
+            local = merge_dare_sharded(self.base_model, self.models, weights, kwargs["density"], self.d_global,
+                                       masks=kwargs.get("masks"), generator=kwargs.get("generator"), group=self.group)
         else:
             raise ValueError(f"Merge type '{merge_type}' is not supported.")
         return unflatten_model(gather_flat(local, self.d_global, self.group), self.shape_dict)
