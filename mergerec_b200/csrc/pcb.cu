@@ -46,9 +46,12 @@ struct PcbState {     // one per (slot, model); the window search uses the slot-
     int32_t pad;
 };
 
+// Order-preserving key: ~u for a set sign bit, u with the sign bit set otherwise.  Written as one xor with a mask built
+// from the sign: the select form `(u & sign) ? ~u : (u | sign)` let nvcc compute `u | sign` as the float -|x| (an FADD),
+// which turns a NaN into the canonical NaN 0x7fffffff, so +NaN weights were keyed as -0.
 __device__ __forceinline__ uint32_t pcb_key(float x) {
     const uint32_t u = __float_as_uint(x);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    return u ^ ((uint32_t)((int32_t)u >> 31) | 0x80000000u);
 }
 __device__ __forceinline__ float pcb_unkey(uint32_t k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
@@ -563,15 +566,19 @@ pcb_build_kernel(const float* __restrict__ base, PtrPack<K> m, int64_t d, const 
                 const float cl = fminf(fmaxf(task[k], s_q[k]), s_max[k]);
                 scale[k] = pcb_div_by<SAFE>(__fsub_rn(cl, s_q[k]), s_span[k], s_rspan[k]);
             }
-            const float denom = fmaxf(torch_sum_dim0<K>(scale, tail), (float)1e-12);   // in [1e-12, K]
+            // in [1e-12, K], or NaN: under IEEE divides (the rerun of status 2) a model whose range is 0 -- it equals
+            // the base -- has NaN scales, and pcb.py's clamp(sum, min=1e-12) keeps the NaN where fmaxf alone returns
+            // 1e-12.  The fast divisions only run with every divisor in range: their scales are never NaN.
+            const float ssum = torch_sum_dim0<K>(scale, tail);
+            const float denom = (!SAFE && ssum != ssum) ? ssum : fmaxf(ssum, (float)1e-12);
             const float rden = SAFE ? __frcp_rn(denom) : 0.0f;
 #pragma unroll
             for (int k = 0; k < K; ++k) {
                 // pcb.py:54-56: sign(tau) A scale / denom / n.  Round-to-nearest commutes with the sign, so the
                 // quotients are taken of the magnitude (A scale >= +0: a zero needs no special case) and the sign goes
-                // on last; sign(0) = 0 makes the whole product +0.
+                // on last; sign(0) = 0 makes the whole product +0, unless scale / denom is NaN (0 * NaN; IEEE divides only).
                 const float w = pcb_div_count<SAFE>(pcb_div_by<SAFE>(__fmul_rn(A[k], scale[k]), denom, rden), (float)K, inv_n);
-                xs[k][c] = (tau[k] != 0.0f) ? copysignf(w, tau[k]) : 0.0f;   // the input is dead: reuse its register
+                xs[k][c] = (tau[k] != 0.0f) ? copysignf(w, tau[k]) : ((!SAFE && w != w) ? w : 0.0f);   // the input is dead: reuse its register
                 if (task_out && c < nvalid) task_out[(int64_t)k * ldo + j0 + c] = task[k];
             }
         }
