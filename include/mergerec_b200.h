@@ -165,6 +165,16 @@ int mr_ties_build(const float* base, const float* const* models, int K, int64_t 
 int mr_topk_rows(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base, float* out_val,
                  int32_t* out_id, mr_stream_t stream);
 
+/* mr_topk_rows with items left out of each row: the full-ranking protocol that removes a user's history before
+ * Recall@K / NDCG@K are taken (RecBole's full-sort evaluation sets those scores to -inf).
+ *   excl_off   dev int64 (Q + 1): CSR offsets by row; row q's list is excl_ids[excl_off[q] .. excl_off[q + 1])
+ *   excl_ids   dev int32: global item ids, ascending within a row, duplicates allowed; a row may be empty
+ * Row q never lists an item of its list; a row with fewer than K other items ends in slots of id -1, score -inf.  Ids
+ * outside [id_base, id_base + N) have no effect, so every shard of a catalog takes the same lists.  Both pointers must
+ * be non-NULL (even when every row is empty). */
+int mr_topk_rows_exclude(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base, float* out_val,
+                         int32_t* out_id, const int64_t* excl_off, const int32_t* excl_ids, mr_stream_t stream);
+
 /* Merge L per-shard lists (vals / ids: dev (L, Q, K_in), sorted or not, id < 0 = empty slot) into one sorted
  * (Q, K_out) list: the exchange step after the NCCL allgather of per-GPU top-K lists (no reference
  * counterpart; the reference is single-GPU, README.md:51-53).  L * K_in <= 8192. */
@@ -207,6 +217,19 @@ int64_t mr_score_topk_workspace_bytes(int64_t Q, int64_t N, int E, int K);
 int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N, int E,
                   int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws, int64_t ws_bytes,
                   mr_stream_t stream);
+
+/* mr_score_topk with items left out of each row's list (a user's history), inside the fused kernel: an excluded item
+ * never enters the row's candidates, so the list is the exact top-K of the remaining items.
+ *   excl_off   dev int64 (Q + 1): CSR offsets by query row; row q's list is excl_ids[excl_off[q] .. excl_off[q + 1])
+ *   excl_ids   dev int32: global item ids, ascending within a row, duplicates allowed; a row may be empty
+ * Row q never lists an item of its list; a row with fewer than K other items ends in slots of id -1, score -inf.  Ids
+ * outside [id_base, id_base + N) have no effect, so every shard (and every streamed chunk) of a catalog takes the same
+ * lists.  Same arguments, workspace (mr_score_topk_workspace_bytes) and requirements as mr_score_topk otherwise, plus
+ * non-NULL excl_off / excl_ids (even when every row is empty).  Runs in the default kernel geometry whatever the
+ * MR_SCORE_BK / MR_SCORE_BF16_EPI_GROUPS experiment settings say. */
+int mr_score_topk_exclude(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                          int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
+                          int64_t ws_bytes, const int64_t* excl_off, const int32_t* excl_ids, mr_stream_t stream);
 
 /* Host-only view of the kernel's static schedule for a problem shape (no CUDA call; tests/test_schedule.py).  A unit =
  * (block of 256 queries, contiguous range of 256-item tiles); the grid's CTA pairs run the units in waves of `wave`,

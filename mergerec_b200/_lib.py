@@ -38,12 +38,15 @@ SIGNATURES = {
     "mr_ties_select_exact": ([_vp, _vp, _i32, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_ties_select_build": ([_vp, _vp, _i32, _i64, _i64, _i32, _vp, _i32, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_topk_rows": ([_vp, _i64, _i64, _i64, _i32, _i32, _vp, _vp, _vp], C.c_int),
+    "mr_topk_rows_exclude": ([_vp, _i64, _i64, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp], C.c_int),
     "mr_topk_merge": ([_vp, _vp, _i32, _i64, _i32, _i32, _vp, _vp, _vp], C.c_int),
     "mr_topk_merge_packed": ([_vp, _i32, _i64, _i32, _i32, _vp, _vp, _vp], C.c_int),
     "mr_float_sum": ([_vp, _i64, _i32], C.c_double),
     "mr_label_rank": ([_vp, _i64, _i32, _vp, _vp, _vp], C.c_int),
     "mr_score_topk_workspace_bytes": ([_i64, _i64, _i32, _i32], _i64),
     "mr_score_topk": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp], C.c_int),
+    "mr_score_topk_exclude": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _vp],
+                              C.c_int),
     "mr_score_topk_debug_buffer": ([_vp, _i64], C.c_int),
     "mr_score_topk_schedule": ([_i64, _i64, _i32, _i32, _vp, _vp, _i64], _i64),
     "mr_to_bf16": ([_vp, _i64, _vp, _vp], C.c_int),

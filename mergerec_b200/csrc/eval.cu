@@ -21,15 +21,21 @@ constexpr int kTopkThreads = 256;
 constexpr int kTopkCap = 2048;               // candidate buffer (keys), power of two
 constexpr int kTopkChunk = kTopkThreads * 4; // elements examined between two buffer checks
 
+// EXCL: items of row q's exclusion list (CSR: excl_ids[excl_off[q] .. excl_off[q + 1]), ascending global ids) never
+// enter the buffer.  A thread's columns are strided, so each key that passes the threshold is looked up in the row's
+// list by binary search.
+template <bool EXCL>
 __global__ void __launch_bounds__(kTopkThreads)
 topk_rows_kernel(const float* __restrict__ scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base,
-                 float* __restrict__ out_val, int32_t* __restrict__ out_id) {
+                 float* __restrict__ out_val, int32_t* __restrict__ out_id, const int64_t* __restrict__ excl_off,
+                 const int32_t* __restrict__ excl_ids) {
     __shared__ u64 s_keys[kTopkCap];
     __shared__ int s_cnt;
     __shared__ u64 s_thr;
     for (int64_t q = blockIdx.x; q < Q; q += gridDim.x) {
         const float* row = scores + q * ld;
         const bool vec = ((reinterpret_cast<uintptr_t>(row) & 15) == 0);
+        const int64_t ex_beg = EXCL ? excl_off[q] : 0, ex_end = EXCL ? excl_off[q + 1] : 0;
         if (threadIdx.x == 0) { s_cnt = 0; s_thr = 0; }
         __syncthreads();
         for (int64_t c0 = 0; c0 < N; c0 += kTopkChunk) {
@@ -51,6 +57,15 @@ topk_rows_kernel(const float* __restrict__ scores, int64_t Q, int64_t N, int64_t
             for (int i = 0; i < 4; ++i) {
                 if (i < nv) {
                     const u64 key = topk_key(v[i], (uint32_t)(id_base + (int32_t)(c + i)));
+                    if (EXCL && key > thr) {
+                        const int32_t id = id_base + (int32_t)(c + i);
+                        int64_t a = ex_beg, b = ex_end;
+                        while (a < b) {
+                            const int64_t m = (a + b) >> 1;
+                            if (excl_ids[m] < id) a = m + 1; else b = m;
+                        }
+                        if (a < ex_end && excl_ids[a] == id) continue;
+                    }
                     if (key > thr) {
                         const int pos = atomicAdd(&s_cnt, 1);
                         s_keys[pos] = key;
@@ -291,8 +306,9 @@ scores_fp32_kernel(const float* __restrict__ U, int64_t Q, const float* __restri
 
 }  // namespace mr
 
-extern "C" int mr_topk_rows(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base,
-                            float* out_val, int32_t* out_id, mr_stream_t stream) {
+// mr_topk_rows (excl_off == NULL) and mr_topk_rows_exclude
+static int topk_rows_launch(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base, float* out_val,
+                            int32_t* out_id, const int64_t* excl_off, const int32_t* excl_ids, mr_stream_t stream) {
     using namespace mr;
     MR_REQUIRE(Q >= 0 && N >= 0 && ld >= N, "mr_topk_rows: need Q >= 0 and ld >= N >= 0");
     MR_REQUIRE(K >= 1 && K <= MR_MAX_TOPK, "mr_topk_rows: K=%d outside [1,%d]", K, MR_MAX_TOPK);
@@ -302,9 +318,26 @@ extern "C" int mr_topk_rows(const float* scores, int64_t Q, int64_t N, int64_t l
     const int64_t cap = (int64_t)sm_count() * 8;
     const unsigned blocks = (unsigned)(Q < cap ? Q : cap);
     // rows whose start is not 16-byte aligned (ld % 4 != 0) simply take the scalar loads
-    topk_rows_kernel<<<blocks, kTopkThreads, 0, (cudaStream_t)stream>>>(scores, Q, N, ld, K, id_base, out_val, out_id);
+    if (excl_off)
+        topk_rows_kernel<true><<<blocks, kTopkThreads, 0, (cudaStream_t)stream>>>(scores, Q, N, ld, K, id_base, out_val,
+                                                                                  out_id, excl_off, excl_ids);
+    else
+        topk_rows_kernel<false><<<blocks, kTopkThreads, 0, (cudaStream_t)stream>>>(scores, Q, N, ld, K, id_base, out_val,
+                                                                                   out_id, nullptr, nullptr);
     MR_CUDA_LAUNCH_CHECK("mr_topk_rows");
     return MR_OK;
+}
+
+extern "C" int mr_topk_rows(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base,
+                            float* out_val, int32_t* out_id, mr_stream_t stream) {
+    return topk_rows_launch(scores, Q, N, ld, K, id_base, out_val, out_id, nullptr, nullptr, stream);
+}
+
+extern "C" int mr_topk_rows_exclude(const float* scores, int64_t Q, int64_t N, int64_t ld, int K, int32_t id_base,
+                                    float* out_val, int32_t* out_id, const int64_t* excl_off, const int32_t* excl_ids,
+                                    mr_stream_t stream) {
+    MR_REQUIRE(excl_off && excl_ids, "mr_topk_rows_exclude: null pointer (excl_off / excl_ids)");
+    return topk_rows_launch(scores, Q, N, ld, K, id_base, out_val, out_id, excl_off, excl_ids, stream);
 }
 
 static int topk_merge_launch(const float* vals, const int32_t* ids, int64_t list_stride, int L, int64_t Q, int K_in,

@@ -23,6 +23,8 @@
 // Two accumulator stages (2 x 256 TMEM columns) let the epilogue of tile i overlap the MMAs of tile i + 1.
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "topk_common.cuh"
 
@@ -80,6 +82,15 @@ struct Params {
     int wave;           // CTA pairs (clusters) in the grid = units that run at the same time
     int sync_giveup;    // windows after which a unit stops waiting if a member of its stream has not even started (0 = never)
 };
+// Parameters of the EXCL instantiations (mr_score_topk_exclude).  A type of their own: adding the fields to Params changes
+// the code ptxas emits for the other instantiations.
+struct ExclParams : Params {
+    // items to leave out of each row's list, CSR by global query row: row q's global item ids are
+    // excl_ids[excl_off[q] .. excl_off[q + 1]), ascending, duplicates allowed
+    const int64_t* excl_off;
+    const int32_t* excl_ids;
+};
+template <bool EXCL> using KernelParams = typename std::conditional<EXCL, ExclParams, Params>::type;
 
 // ---- PTX helpers ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -420,11 +431,17 @@ __device__ __forceinline__ void warp_write_list(const Params& p, size_t o, const
     }
 }
 
-template <int CG, int BK, bool BF16, int EG>
+// EXCL: leave the items of the row's exclusion list (ExclParams) out of its list.  Phase 2 of the
+// epilogue skips an excluded id before it enters the candidate buffer, so the running threshold stays the exact K-th
+// best of the eligible items.  Inside a unit a row meets its item ids in ascending order (tiles, chunks and bits within
+// a chunk ascend), so a lane-private cursor into the row's sorted list only moves forward: one register compare per
+// survivor of the threshold filter, at most one load per list entry and unit.  A separate instantiation, not a run-time
+// test, because the epilogue's speed depends on its code staying inside the instruction cache (DESIGN.md section 3.4).
+template <int CG, int BK, bool BF16, int EG, bool EXCL>
 __global__ void __launch_bounds__(128 + 128 * EG, 1)
 score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_constant__ CUtensorMap map_ulo,
                   const __grid_constant__ CUtensorMap map_ihi, const __grid_constant__ CUtensorMap map_ilo,
-                  const Params p) {
+                  const KernelParams<EXCL> p) {
     using C = Cfg<CG, BK, BF16>;
     constexpr int kABytes = C::kABytes;
     extern __shared__ unsigned char smem_raw[];
@@ -619,6 +636,22 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
             int cnt = 0;
             uint32_t thr = 0;                        // score key of the row's K-th best so far (0: list not full)
             float thr_f = __int_as_float(0x7FC00000);  // same threshold as a float; NaN = "everything passes"
+            // EXCL: cursor into the row's exclusion list, placed on the first id >= the unit's first item; ex_next is
+            // the id under the cursor (INT32_MAX past the end: no item id reaches it, since id_base + N < 2^31)
+            int64_t ex_cur = 0, ex_end = 0;
+            int32_t ex_next = INT32_MAX;
+            if constexpr (EXCL) {
+                if (active) {
+                    ex_cur = p.excl_off[q];
+                    ex_end = p.excl_off[q + 1];
+                    const int64_t first = (int64_t)p.id_base + (int64_t)u.t0 * kBlockN;
+                    for (int64_t hi = ex_end; ex_cur < hi;) {
+                        const int64_t mid = (ex_cur + hi) >> 1;
+                        if ((int64_t)p.excl_ids[mid] < first) ex_cur = mid + 1; else hi = mid;
+                    }
+                    if (ex_cur < ex_end) ex_next = p.excl_ids[ex_cur];
+                }
+            }
             for (int t = u.t0; t < u.t1; ++t, ++it) {
                 if (EG > 1 && (int)(it & 1) != grp) continue;   // two groups: group g drains stage g
                 const uint32_t acc = it & 1;
@@ -661,6 +694,13 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
                             bits &= 0xFFFF0000u;
                         }
                         const uint32_t key = score_key(__uint_as_float(bits));
+                        if constexpr (EXCL) {
+                            if (key > thr) {
+                                const int32_t id = (int32_t)(id0 + (uint32_t)j);
+                                while (ex_next < id) ex_next = ++ex_cur < ex_end ? p.excl_ids[ex_cur] : INT32_MAX;
+                                if (ex_next == id) continue;
+                            }
+                        }
                         if (key > thr) my_buf[cnt++] = ((u64)key << 32) | (u64)(0xFFFFFFFFu - (id0 + (uint32_t)j));
                     }
                     // rows that could overflow on the next chunk are cut back to their best K, two rows per sort
@@ -792,11 +832,13 @@ static int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
     return (v && *v) ? atoi(v) : dflt;
 }
-static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16) {
+// excl: the plan of mr_score_topk_exclude, whose kernels exist only in the default geometry (BK = 32, one epilogue
+// group): it ignores the experiment knobs MR_SCORE_BK and MR_SCORE_BF16_EPI_GROUPS.
+static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false) {
     Plan pl;
-    pl.eg = (bf16 && env_int("MR_SCORE_BF16_EPI_GROUPS", 1) == 2) ? 2 : 1;
+    pl.eg = (!excl && bf16 && env_int("MR_SCORE_BF16_EPI_GROUPS", 1) == 2) ? 2 : 1;
     pl.cg = env_int("MR_SCORE_CTA_GROUP", 2) == 1 ? 1 : 2;
-    pl.bk = env_int("MR_SCORE_BK", 32) == 16 ? 16 : 32;
+    pl.bk = (!excl && env_int("MR_SCORE_BK", 32) == 16) ? 16 : 32;
     const int sms = sm_count();
     const int clusters = sms / pl.cg;
     pl.QB = (int)((Q + (int64_t)kBlockM * pl.cg - 1) / ((int64_t)kBlockM * pl.cg));
@@ -843,11 +885,11 @@ static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16) {
     return pl;
 }
 
-template <int CG, int BK, bool BF16, int EG>
+template <int CG, int BK, bool BF16, int EG, bool EXCL = false>
 static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul, const CUtensorMap& mih, const CUtensorMap& mil,
-                  const Params& p, cudaStream_t stream) {
+                  const ExclParams& p, cudaStream_t stream) {
     using C = Cfg<CG, BK, BF16>;
-    cudaError_t e = cudaFuncSetAttribute(score_topk_kernel<CG, BK, BF16, EG>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
+    cudaError_t e = cudaFuncSetAttribute(score_topk_kernel<CG, BK, BF16, EG, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     if (e != cudaSuccess) { set_error("mr_score_topk: shared memory attribute: %s", cudaGetErrorString(e)); return (int)e; }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)pl.grid);
@@ -861,7 +903,8 @@ static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG>, muh, mul, mih, mil, p);
+    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG, EXCL>, muh, mul, mih, mil,
+                           static_cast<const KernelParams<EXCL>&>(p));
     if (e != cudaSuccess) { set_error("mr_score_topk: launch: %s", cudaGetErrorString(e)); return (int)e; }
     return MR_OK;
 }
@@ -917,10 +960,12 @@ extern "C" int64_t mr_score_topk_workspace_bytes(int64_t Q, int64_t N, int E, in
     return (a > b ? a : b) + 256;
 }
 
-extern "C" int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
-                             int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
-                             int64_t ws_bytes, mr_stream_t stream) {
+// mr_score_topk (excl_off == NULL) and mr_score_topk_exclude
+static int score_topk_impl(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                           int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
+                           int64_t ws_bytes, mr_stream_t stream, const int64_t* excl_off, const int32_t* excl_ids) {
     using namespace mr;
+    const bool excl = excl_off != nullptr;
     MR_REQUIRE(Q >= 0 && N >= 0 && E >= 1, "mr_score_topk: need Q, N >= 0 and E >= 1");
     MR_REQUIRE(K >= 1 && K <= MR_MAX_FUSED_TOPK, "mr_score_topk: K=%d outside [1,%d]", K, MR_MAX_FUSED_TOPK);
     MR_REQUIRE(mode == MR_SCORE_TF32X3 || mode == MR_SCORE_TF32X1 || mode == MR_SCORE_BF16, "mr_score_topk: unknown mode %d", mode);
@@ -940,14 +985,14 @@ extern "C" int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, cons
         if (e != cudaSuccess) { set_error("mr_score_topk: memset: %s", cudaGetErrorString(e)); return (int)e; }
         return MR_OK;
     }
-    const st::Plan pl = st::make_plan(Q, N, K, bf16);
+    const st::Plan pl = st::make_plan(Q, N, K, bf16, excl);
     const int64_t need = pl.cand_bytes + pl.part_bytes + pl.sync_bytes + 256;
     if (!ws || ws_bytes < need) {
         set_error("mr_score_topk: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
         return MR_ERR_WORKSPACE;
     }
     unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-    st::Params p;
+    st::ExclParams p;
     p.Q = Q; p.N = N; p.E = E; p.K = K; p.mode = mode; p.id_base = id_base;
     const int bk = bf16 ? 32 : pl.bk;                 // bf16 rows are 64 elements = 128 bytes: the BK = 32 geometry
     const int kelems = bf16 ? 64 : bk;
@@ -969,6 +1014,8 @@ extern "C" int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, cons
     int32_t* part_id = reinterpret_cast<int32_t*>(w + pl.cand_bytes + pl.part_bytes / 2);
     p.out_val = part_val;
     p.out_id = part_id;
+    p.excl_off = excl_off;
+    p.excl_ids = excl_ids;
 
     CUtensorMap muh, mul, mih, mil;
     const int brows = st::kBlockN / pl.cg;
@@ -979,10 +1026,28 @@ extern "C" int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, cons
     if (!ok) { set_error("mr_score_topk: cuTensorMapEncodeTiled failed (driver without TMA support?)"); return MR_ERR_UNSUPPORTED; }
 
     int rc;
-    if (bf16 && pl.eg == 2) rc = pl.cg == 1 ? st::launch<1, 32, true, 2>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 2>(pl, muh, mul, mih, mil, p, s);
+    if (excl && bf16) rc = pl.cg == 1 ? st::launch<1, 32, true, 1, true>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 1, true>(pl, muh, mul, mih, mil, p, s);
+    else if (excl) rc = pl.cg == 1 ? st::launch<1, 32, false, 1, true>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, false, 1, true>(pl, muh, mul, mih, mil, p, s);
+    else if (bf16 && pl.eg == 2) rc = pl.cg == 1 ? st::launch<1, 32, true, 2>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 2>(pl, muh, mul, mih, mil, p, s);
     else if (bf16) rc = pl.cg == 1 ? st::launch<1, 32, true, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 1>(pl, muh, mul, mih, mil, p, s);
     else if (bk == 32) rc = pl.cg == 1 ? st::launch<1, 32, false, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, false, 1>(pl, muh, mul, mih, mil, p, s);
     else rc = pl.cg == 1 ? st::launch<1, 16, false, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 16, false, 1>(pl, muh, mul, mih, mil, p, s);
     if (rc != MR_OK) return rc;
     return mr_topk_merge(part_val, part_id, pl.S * pl.eg, Q, K, K, out_val, out_id, stream);
+}
+
+extern "C" int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                             int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
+                             int64_t ws_bytes, mr_stream_t stream) {
+    return score_topk_impl(Uhi, Ulo, Q, Ihi, Ilo, N, E, K, id_base, mode, out_val, out_id, ws, ws_bytes, stream, nullptr,
+                           nullptr);
+}
+
+extern "C" int mr_score_topk_exclude(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo,
+                                     int64_t N, int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id,
+                                     void* ws, int64_t ws_bytes, const int64_t* excl_off, const int32_t* excl_ids,
+                                     mr_stream_t stream) {
+    MR_REQUIRE(excl_off && excl_ids, "mr_score_topk_exclude: null pointer (excl_off / excl_ids)");
+    return score_topk_impl(Uhi, Ulo, Q, Ihi, Ilo, N, E, K, id_base, mode, out_val, out_id, ws, ws_bytes, stream, excl_off,
+                           excl_ids);
 }

@@ -22,11 +22,44 @@ from .sharded import (MAX_FUSED_TOPK, MR_SCORE_BF16, MR_SCORE_TF32X3, ShardedIte
                       new_packed_list, split_tf32, to_bf16)
 
 MAX_TOPK = 1024
+_INT_DTYPES = (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8)
 
 
-def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+def exclusion_csr(exclude: torch.Tensor, Q: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The per-query items to leave out of the ranking -- `exclude`, a (Q, H) integer tensor of global item ids in which
+    negative entries are padding (MergeRec pads its sequences with -1) -- as the CSR the kernels take, built with torch
+    ops on `exclude`'s device: (offsets int64 (Q + 1), ids int32), row q's ids sorted ascending in
+    ids[offsets[q]:offsets[q + 1]].  Duplicates are kept and ids beyond the catalog are allowed (they exclude nothing).
+    `ids` has at least one element, so its pointer is valid even when every row is empty."""
+    if not isinstance(exclude, torch.Tensor) or exclude.dim() != 2 or exclude.shape[0] != Q:
+        raise ValueError(f"exclude must be a (Q, H) tensor with Q = {Q} rows")
+    if exclude.dtype not in _INT_DTYPES:
+        raise ValueError(f"exclude must hold integer item ids, not {exclude.dtype}")
+    x = exclude.to(torch.int64)
+    if x.numel() and int(x.max()) >= 1 << 31:
+        raise ValueError("exclude holds an item id >= 2^31")
+    keep = x >= 0
+    counts = keep.sum(dim=1)
+    rows = torch.sort(torch.where(keep, x, torch.full_like(x, 1 << 31)), dim=1).values   # padding sorts last
+    ids = rows[torch.arange(x.shape[1], device=x.device) < counts[:, None]].to(torch.int32)
+    offsets = torch.cat([counts.new_zeros(1), torch.cumsum(counts, dim=0)])
+    if ids.numel() == 0:
+        ids = torch.zeros(1, dtype=torch.int32, device=x.device)
+    return offsets, ids
+
+
+def _device_csr(exclude: Optional[torch.Tensor], Q: int, dev) -> Optional[Tuple[torch.Tensor, torch.Tensor]]:
+    if exclude is None:
+        return None
+    return tuple(t.to(dev, non_blocking=True) for t in exclusion_csr(exclude, Q))
+
+
+def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0,
+              exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """(values (Q, k) fp32, ids (Q, k) int32) of a (Q, N) score matrix: `mr_topk_rows`, the drop-in for
-    ``torch.topk(scores, k, dim=1)`` (evaluator.py:43).  CPU inputs are copied to the GPU in row chunks."""
+    ``torch.topk(scores, k, dim=1)`` (evaluator.py:43).  CPU inputs are copied to the GPU in row chunks.
+    `exclude`: (Q, H) global item ids to leave out of each row (negative = padding; `exclusion_csr`), through
+    `mr_topk_rows_exclude`; a row left with fewer than k items ends in slots of (-inf, -1)."""
     dev = _lib.require_cuda()
     lib = _lib.load()
     if scores.dim() != 2:
@@ -34,6 +67,7 @@ def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0) -> Tuple[torch.Ten
     Q, N = scores.shape
     if k > N:
         raise RuntimeError(f"selected index k out of range (k={k}, N={N})")  # torch.topk's error class
+    csr = _device_csr(exclude, Q, dev)
     out_v = torch.empty((Q, k), dtype=torch.float32, device=dev)
     out_i = torch.empty((Q, k), dtype=torch.int32, device=dev)
     rows_per_chunk = Q if scores.is_cuda else max(1, min(Q, (1 << 30) // max(4 * N, 1)))
@@ -42,17 +76,32 @@ def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0) -> Tuple[torch.Ten
         chunk = scores[q0:q1].to(device=dev, dtype=torch.float32, non_blocking=True)
         if chunk.stride(1) != 1:
             chunk = chunk.contiguous()
-        _lib.check(lib.mr_topk_rows(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base,
-                                    _lib.dptr(out_v[q0:q1]), _lib.dptr(out_i[q0:q1]), _lib.stream_handle()),
-                   "mr_topk_rows")
+        if csr is None:
+            _lib.check(lib.mr_topk_rows(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base,
+                                        _lib.dptr(out_v[q0:q1]), _lib.dptr(out_i[q0:q1]), _lib.stream_handle()),
+                       "mr_topk_rows")
+        else:   # the offsets index the whole ids array: the chunk's rows are offsets[q0 : q1 + 1]
+            _lib.check(lib.mr_topk_rows_exclude(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base,
+                                                _lib.dptr(out_v[q0:q1]), _lib.dptr(out_i[q0:q1]), _lib.dptr(csr[0][q0:]),
+                                                _lib.dptr(csr[1]), _lib.stream_handle()), "mr_topk_rows_exclude")
     return out_v, out_i
 
 
 def score_topk(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, k: int,
-               mode: int = MR_SCORE_TF32X3, out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None
-               ) -> Tuple[torch.Tensor, torch.Tensor]:
+               mode: int = MR_SCORE_TF32X3, out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+               exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Local fused scoring + top-k of pre-split queries against this rank's shard (`mr_score_topk`).  `out` =
-    (values (Q, k) fp32, ids (Q, k) int32) to write into (e.g. the planes of the exchange buffer)."""
+    (values (Q, k) fp32, ids (Q, k) int32) to write into (e.g. the planes of the exchange buffer).  `exclude`: (Q, H)
+    global item ids to leave out of each row (negative = padding), through `mr_score_topk_exclude`; a row left with
+    fewer than k items ends in slots of (-inf, -1)."""
+    dev = _lib.require_cuda()
+    return _score_topk(user_hi, user_lo, table, k, mode, out, _device_csr(exclude, user_hi.shape[0], dev))
+
+
+def _score_topk(user_hi, user_lo, table: ShardedItemTable, k: int, mode: int,
+                out: Optional[Tuple[torch.Tensor, torch.Tensor]],
+                csr: Optional[Tuple[torch.Tensor, torch.Tensor]]) -> Tuple[torch.Tensor, torch.Tensor]:
+    """`score_topk` with the exclusion lists already in device CSR form (built once, used for every shard / chunk)."""
     dev = _lib.require_cuda()
     lib = _lib.load()
     Q, E = user_hi.shape
@@ -67,9 +116,16 @@ def score_topk(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: Sh
     if ws_bytes < 0:
         _lib.check(ws_bytes, "mr_score_topk_workspace_bytes")
     ws = table.workspace(ws_bytes)
-    _lib.check(lib.mr_score_topk(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
-                                 table.n_local, E, k, table.id_base, mode, _lib.dptr(out_v), _lib.dptr(out_i),
-                                 _lib.dptr(ws), ws_bytes, _lib.stream_handle()), "mr_score_topk")
+    if csr is None:
+        _lib.check(lib.mr_score_topk(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
+                                     table.n_local, E, k, table.id_base, mode, _lib.dptr(out_v), _lib.dptr(out_i),
+                                     _lib.dptr(ws), ws_bytes, _lib.stream_handle()), "mr_score_topk")
+    else:
+        _lib.check(lib.mr_score_topk_exclude(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi),
+                                             _lib.dptr(table.lo), table.n_local, E, k, table.id_base, mode,
+                                             _lib.dptr(out_v), _lib.dptr(out_i), _lib.dptr(ws), ws_bytes,
+                                             _lib.dptr(csr[0]), _lib.dptr(csr[1]), _lib.stream_handle()),
+                   "mr_score_topk_exclude")
     return out_v, out_i
 
 
@@ -100,17 +156,22 @@ class Evaluator:
                 self._metrics.append(MetricType[metric].metric_cls(k))
 
     # ------------------------------------------------------------------ reference contract
-    def evaluate(self, scores: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "") -> Dict[str, float]:
-        return self(scores, labels, metric_prefix)
+    def evaluate(self, scores: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "",
+                 exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
+        return self(scores, labels, metric_prefix, exclude)
 
-    def __call__(self, scores: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "") -> Dict[str, float]:
-        _, ids = topk_rows(scores, self._max_k)
+    def __call__(self, scores: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "",
+                 exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
+        """`exclude` (optional): (Q, H) global item ids to leave out of each query's ranking (e.g. its history;
+        negative entries are padding), as RecBole's full-sort evaluation does.  A label in its row's `exclude`
+        cannot be hit: it counts as a miss."""
+        _, ids = topk_rows(scores, self._max_k, exclude=exclude)
         return self.metrics_from_ids(ids, labels, metric_prefix)
 
     # ------------------------------------------------------------------ fused additions
     def topk_embeddings(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
-                        k: Optional[int] = None, normalize: bool = False,
-                        mode: int = MR_SCORE_TF32X3) -> Tuple[torch.Tensor, torch.Tensor]:
+                        k: Optional[int] = None, normalize: bool = False, mode: int = MR_SCORE_TF32X3,
+                        exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """Top-k (values fp32, global ids int32), both (Q, k), of ``user_emb @ item_emb.T`` without the matrix.
 
         ``item_emb`` is an (N, E) tensor (single GPU) or a ``ShardedItemTable`` (reusable, possibly one shard of
@@ -118,7 +179,10 @@ class Evaluator:
         ``normalize`` applies the reference's cosine normalisation to the queries (and to a raw item tensor).
         ``mode``: ``MR_SCORE_TF32X3`` (default, fp32-faithful), ``MR_SCORE_TF32X1``, or ``MR_SCORE_BF16`` -- the
         bf16-compat mode that mirrors the reference's default ``precision="bf16-mixed"`` runs (bf16 operands, fp32
-        accumulation, scores rounded to bf16; configs/base.py:41) with the canonical tie rule on equal scores."""
+        accumulation, scores rounded to bf16; configs/base.py:41) with the canonical tie rule on equal scores.
+        ``exclude``: (Q, H) global item ids to leave out of each query's list (negative = padding), applied inside the
+        fused kernel; a row left with fewer than k items ends in slots of (-inf, -1).  Every rank of a sharded table
+        passes the same ``exclude``, like the queries."""
         k = self._max_k if k is None else k
         if k > MAX_FUSED_TOPK:
             raise ValueError(f"fused top-k supports k <= {MAX_FUSED_TOPK}")
@@ -132,17 +196,19 @@ class Evaluator:
         queries = user_emb if isinstance(user_emb, PreparedQueries) else PreparedQueries(user_emb, normalize, table.bf16)
         if queries.bf16 != table.bf16:
             raise ValueError("the queries were prepared for a different scoring mode than the item table")
+        csr = _device_csr(exclude, queries.shape[0], queries.hi.device)
         if table.group is None or table.world == 1:
-            return score_topk(queries.hi, queries.lo, table, k, mode)
+            return _score_topk(queries.hi, queries.lo, table, k, mode, None, csr)
         # sharded: the kernel writes this rank's list into the buffer that the single all-gather sends
         local, loc_v, loc_i = new_packed_list(queries.shape[0], k, queries.hi.device)
-        score_topk(queries.hi, queries.lo, table, k, mode, out=(loc_v, loc_i))
+        _score_topk(queries.hi, queries.lo, table, k, mode, (loc_v, loc_i), csr)
         return exchange_packed(local, k, table.group, gathered=table.gather_buffer(queries.shape[0], k))
 
     def topk_embeddings_streamed(self, user_emb: Union[torch.Tensor, "PreparedQueries"], host_items: torch.Tensor,
                                  k: Optional[int] = None, id_base: int = 0, n_total: Optional[int] = None, group=None,
                                  normalize: bool = False, mode: int = MR_SCORE_TF32X3,
-                                 first_rows: int = 32768, max_chunks: int = 12) -> Tuple[torch.Tensor, torch.Tensor]:
+                                 first_rows: int = 32768, max_chunks: int = 12,
+                                 exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """`topk_embeddings` for an item table that still lives in HOST memory (what `load_item_embeddings` /
         `ItemEncoderMixin.encode_items(...).cpu()` hand over): the rows are copied to the GPU in chunks on a copy stream
         while the previous chunk is being scored, so the transfer hides behind the tensor-core work instead of preceding
@@ -150,7 +216,8 @@ class Evaluator:
         split into its TF32 operands, scored into its own sorted list, and the lists are merged (`mr_topk_merge_packed`).
         Because a (query, item) score does not depend on how the table is cut, the result is bit-identical to the
         one-table call.  `host_items` = this rank's rows (pinned memory makes the copies asynchronous); `id_base`,
-        `n_total`, `group` as for `ShardedItemTable`."""
+        `n_total`, `group` as for `ShardedItemTable`; `exclude` as for `topk_embeddings` (global ids: every chunk
+        takes the same lists)."""
         from .sharded import exchange_packed, topk_merge_packed
         k = self._max_k if k is None else k
         if k > MAX_FUSED_TOPK:
@@ -165,6 +232,7 @@ class Evaluator:
         bf16 = mode == MR_SCORE_BF16
         queries = user_emb if isinstance(user_emb, PreparedQueries) else PreparedQueries(user_emb, normalize, bf16)
         Q = queries.shape[0]
+        csr = _device_csr(exclude, Q, dev)
         # chunk plan: geometric ramp, at most max_chunks lists (k * chunks candidates per row must stay mergeable)
         max_chunks = max(1, min(max_chunks, 8192 // max(k, 1)))
         bounds, lo, rows = [], 0, max(int(first_rows), 1)
@@ -195,9 +263,9 @@ class Evaluator:
             table = ShardedItemTable(chunk, id_base=id_base + a, n_total=n_total, normalize=normalize, bf16=bf16)
             table._ws = ws                                            # one scratch for all chunks (grown if needed)
             if b - a >= k:
-                score_topk(queries.hi, queries.lo, table, k, mode, out=(partial[c, 0].view(torch.float32), partial[c, 1]))
+                _score_topk(queries.hi, queries.lo, table, k, mode, (partial[c, 0].view(torch.float32), partial[c, 1]), csr)
             else:
-                self._score_small_chunk(queries, table, k, mode, partial[c])
+                self._score_small_chunk(queries, table, k, mode, partial[c], csr)
             ws = table._ws
         vals, ids = topk_merge_packed(partial, k) if C > 1 else (partial[0, 0].view(torch.float32), partial[0, 1])
         if group is not None:
@@ -208,19 +276,21 @@ class Evaluator:
         return vals, ids
 
     @staticmethod
-    def _score_small_chunk(queries: "PreparedQueries", table: ShardedItemTable, k: int, mode: int, out: torch.Tensor) -> None:
+    def _score_small_chunk(queries: "PreparedQueries", table: ShardedItemTable, k: int, mode: int, out: torch.Tensor,
+                           csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> None:
         """A chunk with fewer than k rows: its list has only n < k entries; the rest of the (Q, k) plane is marked empty."""
         n = table.n_local
         out[0].view(torch.float32).fill_(float("-inf"))
         out[1].fill_(-1)
         if n:
-            v, i = score_topk(queries.hi, queries.lo, table, n, mode)
+            v, i = _score_topk(queries.hi, queries.lo, table, n, mode, None, csr)
             out[0].view(torch.float32)[:, :n] = v
             out[1][:, :n] = i
 
     def evaluate_embeddings_streamed(self, user_emb, host_items: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "",
                                      **kw) -> Dict[str, float]:
-        """`evaluate_embeddings` with a host-resident item table (see `topk_embeddings_streamed`)."""
+        """`evaluate_embeddings` with a host-resident item table (see `topk_embeddings_streamed`; `exclude` is one of
+        its keywords)."""
         _, ids = self.topk_embeddings_streamed(user_emb, host_items, self._max_k, **kw)
         return self.metrics_from_ids(ids, labels, metric_prefix)
 
@@ -232,8 +302,9 @@ class Evaluator:
 
     def evaluate_embeddings(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
                             labels: torch.Tensor, metric_prefix: str = "", normalize: bool = False,
-                            mode: int = MR_SCORE_TF32X3) -> Dict[str, float]:
-        _, ids = self.topk_embeddings(user_emb, item_emb, self._max_k, normalize, mode)
+                            mode: int = MR_SCORE_TF32X3, exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
+        """Metrics of `topk_embeddings`; with `exclude`, a label in its row's `exclude` counts as a miss."""
+        _, ids = self.topk_embeddings(user_emb, item_emb, self._max_k, normalize, mode, exclude)
         return self.metrics_from_ids(ids, labels, metric_prefix)
 
     # ------------------------------------------------------------------ shared tail
