@@ -196,6 +196,17 @@ double mr_float_sum(const double* x, int64_t n, int compensated);
 /* rank[q] = position of labels[q] in ids[q, :K], or -1          ref: evaluator/metrics.py:51-59, 79-84 */
 int mr_label_rank(const int32_t* ids, int64_t Q, int K, const int64_t* labels, int32_t* rank, mr_stream_t stream);
 
+/* Rank of each row's label against the whole row of a materialised (Q, N) score matrix (row stride ld), with no list
+ * and no K: count[q] = the number of columns that sort before column labels[q] - id_base under the top-K order
+ * (score desc, id asc; -0.0 == +0.0, NaN first), leaving out the ids of row q's exclusion list, if given.  -1 when the
+ * label is not in [id_base, id_base + N).  The label's own exclusion is not applied: its count is still the number of
+ * eligible items ahead of it.
+ *   labels     dev int64 (Q): global item ids
+ *   excl_off / excl_ids   as for mr_topk_rows_exclude, both NULL (no exclusion) or both set
+ *   count      dev int32 (Q) */
+int mr_rank_rows(const float* scores, int64_t Q, int64_t N, int64_t ld, int32_t id_base, const int64_t* labels,
+                 const int64_t* excl_off, const int32_t* excl_ids, int32_t* count, mr_stream_t stream);
+
 /* Fused full-catalog scoring + per-row top-K: the tensor-core path (tcgen05.mma kind::tf32 fed by TMA, fp32
  * accumulators in TMEM) that never materialises the (Q, N) score matrix
  *                              ref: module/recommender/module.py:137 followed by evaluator/evaluator.py:43
@@ -230,6 +241,28 @@ int mr_score_topk(const float* Uhi, const float* Ulo, int64_t Q, const float* Ih
 int mr_score_topk_exclude(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
                           int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
                           int64_t ws_bytes, const int64_t* excl_off, const int32_t* excl_ids, mr_stream_t stream);
+
+/* Rank of each query's label against this GPU's rows of the item table, inside the fused scoring kernel: two
+ * passes with the operands and modes of mr_score_topk, and no list.
+ * mr_label_score: label_key[q] (dev uint32, Q) = the score key of (query q, item labels[q]) -- the order-preserving
+ *   32-bit key of the score the top-K kernel ranks, bit for bit, computed by the same kernel on the gathered label rows
+ *   -- or 0 when labels[q] is not in [id_base, id_base + N).  0 is never the key of a score.  On a sharded table,
+ *   the maximum over the ranks is the label's key.
+ * mr_score_rank: count[q] (dev int32, Q) = the number of this table's items that sort before the label under (score
+ *   key desc, id asc), leaving out the ids of row q's exclusion list (excl_off / excl_ids as for mr_score_topk_exclude,
+ *   both NULL or both set); -1 when label_key[q] == 0.  The label's own exclusion is not applied.  On a sharded table
+ *   the sum of the ranks' counts is the label's 0-based rank in the whole catalog.
+ *   labels     dev int64 (Q): global item ids
+ *   ws         dev scratch of at least mr_score_rank_workspace_bytes(Q, N, E) bytes (both passes, every mode)
+ * Requirements as for mr_score_topk (K aside).  Both run in the default kernel geometry (MR_SCORE_BK and
+ * MR_SCORE_BF16_EPI_GROUPS are ignored) and need the same MR_SCORE_CTA_GROUP. */
+int64_t mr_score_rank_workspace_bytes(int64_t Q, int64_t N, int E);
+int mr_label_score(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N, int E,
+                   int32_t id_base, int mode, const int64_t* labels, uint32_t* label_key, void* ws, int64_t ws_bytes,
+                   mr_stream_t stream);
+int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N, int E,
+                  int32_t id_base, int mode, const int64_t* labels, const uint32_t* label_key, const int64_t* excl_off,
+                  const int32_t* excl_ids, int32_t* count, void* ws, int64_t ws_bytes, mr_stream_t stream);
 
 /* Host-only view of the kernel's static schedule for a problem shape (no CUDA call; tests/test_schedule.py).  A unit =
  * (block of 256 queries, contiguous range of 256-item tiles); the grid's CTA pairs run the units in waves of `wave`,

@@ -48,6 +48,10 @@ SIGNATURES = {
     "mr_score_topk_exclude": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _vp],
                               C.c_int),
     "mr_score_topk_debug_buffer": ([_vp, _i64], C.c_int),
+    "mr_rank_rows": ([_vp, _i64, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "mr_score_rank_workspace_bytes": ([_i64, _i64, _i32], _i64),
+    "mr_label_score": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp], C.c_int),
+    "mr_score_rank": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_score_topk_schedule": ([_i64, _i64, _i32, _i32, _vp, _vp, _i64], _i64),
     "mr_to_bf16": ([_vp, _i64, _vp, _vp], C.c_int),
     "mr_split_tf32": ([_vp, _i64, _vp, _vp, _vp], C.c_int),

@@ -231,6 +231,56 @@ __global__ void label_rank_kernel(const int32_t* __restrict__ ids, int64_t Q, in
     rank[q] = r;
 }
 
+// ---- rank of the label against the whole row (no list, no K) ----------------------------------------------------
+// count[q] = number of columns whose (score, id) key sorts before the label's, minus the row's excluded ids that do:
+// the exclusion list is walked once, after the count, skipping repeated ids.  -1 when the label is not a column.
+constexpr int kRankThreads = 256;
+__global__ void __launch_bounds__(kRankThreads)
+rank_rows_kernel(const float* __restrict__ scores, int64_t Q, int64_t N, int64_t ld, int32_t id_base,
+                 const int64_t* __restrict__ labels, const int64_t* __restrict__ excl_off,
+                 const int32_t* __restrict__ excl_ids, int32_t* __restrict__ count) {
+    __shared__ int s_warp[kRankThreads / 32];
+    for (int64_t q = blockIdx.x; q < Q; q += gridDim.x) {
+        const float* row = scores + q * ld;
+        const int64_t col = labels[q] - id_base;
+        if (col < 0 || col >= N) {          // block-uniform
+            if (threadIdx.x == 0) count[q] = -1;
+            continue;
+        }
+        const u64 L = topk_key(row[col], (uint32_t)(id_base + (int32_t)col));
+        const bool vec = ((reinterpret_cast<uintptr_t>(row) & 15) == 0);
+        int c = 0;
+        for (int64_t c0 = (int64_t)threadIdx.x * 4; c0 < N; c0 += kRankThreads * 4) {
+            if (c0 + 3 < N && vec) {
+                const float4 f = ldg_stream4(row + c0);
+                const uint32_t id = (uint32_t)(id_base + (int32_t)c0);
+                c += (topk_key(f.x, id) > L) + (topk_key(f.y, id + 1) > L) + (topk_key(f.z, id + 2) > L) +
+                     (topk_key(f.w, id + 3) > L);
+            } else {
+                for (int64_t i = c0; i < c0 + 4 && i < N; ++i) c += topk_key(row[i], (uint32_t)(id_base + (int32_t)i)) > L;
+            }
+        }
+        if (excl_off) {
+            const int64_t beg = excl_off[q], end = excl_off[q + 1];
+            for (int64_t i = beg + threadIdx.x; i < end; i += kRankThreads) {
+                const int64_t x = (int64_t)excl_ids[i] - id_base;
+                if (x >= 0 && x < N && (i == beg || excl_ids[i - 1] != excl_ids[i]))
+                    c -= topk_key(row[x], (uint32_t)excl_ids[i]) > L;
+            }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) c += __shfl_xor_sync(0xffffffffu, c, off);
+        if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = c;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int t = 0;
+            for (int w = 0; w < kRankThreads / 32; ++w) t += s_warp[w];
+            count[q] = t;
+        }
+        __syncthreads();
+    }
+}
+
 // ---- hi/lo split for the 3xTF32 contraction -----------------------------------------------------------------------
 // hi = rna_tf32(x), lo = rna_tf32(x - hi): x = hi + lo up to 2^-22 |x|, both exactly representable in TF32.
 __device__ __forceinline__ float rna_tf32(float x) {
@@ -394,6 +444,23 @@ extern "C" int mr_label_rank(const int32_t* ids, int64_t Q, int K, const int64_t
     MR_REQUIRE(ids && labels && rank, "mr_label_rank: null pointer");
     label_rank_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ids, Q, K, labels, rank);
     MR_CUDA_LAUNCH_CHECK("mr_label_rank");
+    return MR_OK;
+}
+
+extern "C" int mr_rank_rows(const float* scores, int64_t Q, int64_t N, int64_t ld, int32_t id_base, const int64_t* labels,
+                            const int64_t* excl_off, const int32_t* excl_ids, int32_t* count, mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr),
+               "mr_rank_rows: excl_off and excl_ids must both be NULL or both be set");
+    MR_REQUIRE(Q >= 0 && N >= 0 && ld >= N, "mr_rank_rows: need Q >= 0 and ld >= N >= 0");
+    MR_REQUIRE((int64_t)id_base + N < (1ll << 31), "mr_rank_rows: id_base + N must fit 31 bits");
+    if (Q == 0) return MR_OK;
+    MR_REQUIRE(scores && labels && count, "mr_rank_rows: null pointer");
+    const int64_t cap = (int64_t)sm_count() * 8;
+    const unsigned blocks = (unsigned)(Q < cap ? Q : cap);
+    rank_rows_kernel<<<blocks, kRankThreads, 0, (cudaStream_t)stream>>>(scores, Q, N, ld, id_base, labels, excl_off,
+                                                                        excl_ids, count);
+    MR_CUDA_LAUNCH_CHECK("mr_rank_rows");
     return MR_OK;
 }
 

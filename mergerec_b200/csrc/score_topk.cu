@@ -90,7 +90,20 @@ struct ExclParams : Params {
     const int64_t* excl_off;
     const int32_t* excl_ids;
 };
-template <bool EXCL> using KernelParams = typename std::conditional<EXCL, ExclParams, Params>::type;
+// Epilogue of an instantiation (template parameter EPI): the top-K lists, or one of the two label-rank passes --
+// kEpiDiag (mr_label_score): the score key of each query's label; kEpiCount (mr_score_rank): per (split, row), the
+// items of the unit that sort before the row's label.
+constexpr int kEpiTopK = 0, kEpiCount = 1, kEpiDiag = 2;
+// Parameters of the label-rank instantiations, a type of their own for the same reason as ExclParams.
+struct RankParams : ExclParams {
+    const int64_t* labels;       // (Q) global item id of each query's label
+    const uint32_t* label_key;   // kEpiCount: (Q) score key of the label's score (0: no label, the row is not counted)
+    uint32_t* out_key;           // kEpiDiag: (Q) score key of the label's score, 0 when the label is not in this table
+    int32_t* part;               // kEpiCount: (S, Q) counts per item split
+};
+template <bool EXCL, int EPI = kEpiTopK>
+using KernelParams = typename std::conditional<EPI != kEpiTopK, RankParams,
+                                               typename std::conditional<EXCL, ExclParams, Params>::type>::type;
 
 // ---- PTX helpers ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -431,17 +444,137 @@ __device__ __forceinline__ void warp_write_list(const Params& p, size_t o, const
     }
 }
 
+// The score the top-K epilogue ranks: the fp32 accumulator, or in bf16-compat mode that accumulator rounded to bf16
+// (RN-even) with the same bit operations.
+template <bool BF16>
+__device__ __forceinline__ float ranked_score(uint32_t bits) {
+    if (BF16) {
+        if ((bits & 0x7F800000u) != 0x7F800000u) bits += 0x7FFFu + ((bits >> 16) & 1u);
+        bits &= 0xFFFF0000u;
+    }
+    return __uint_as_float(bits);
+}
+
+// ---- label-rank epilogues (RankParams) ----------------------------------------------------------------------------
+// kEpiDiag: every unit walks one tile, the gathered label rows of its own query rows (host side: label_score), so query
+// row `row` of CTA `rank` meets its label in accumulator column rank * 128 + row.  Two 16-column loads cover a warp's 32
+// columns; each lane selects its own.
+// kEpiCount: per 16-column chunk, bit j = "column j sorts before the row's label" under (score key desc, id asc):
+// greater score, or equal score and smaller id (an arithmetic mask of the ids below the label), minus padding and
+// excluded ids (the forward-only cursor of the EXCL top-K epilogue); the row's count grows by the popc.  No candidate
+// buffer, no sort.  The float tests are the key tests: -0 == +0, and a NaN score is above every other (gt = !(f <= L));
+// for a NaN label only the NaN columns with smaller ids count (Lg = +inf: gt = NaN, eq = never).
+template <int CG, bool BF16, bool EXCL, int EPI>
+__device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem_base, uint32_t bar_tfull,
+                                              uint32_t bar_tempty, uint32_t rank, bool leader, int cluster_id,
+                                              int num_clusters, int warp, int lane) {
+    const int ew = (warp - 4) & 3;
+    const int row = ew * 32 + lane;
+    uint32_t it = 0;
+    Unit u;
+    for (int ui = cluster_id; get_unit(p, ui, u); ui += num_clusters) {
+        const int64_t q = ((int64_t)u.qb * CG + rank) * kBlockM + row;
+        const bool active = q < p.Q;
+        uint32_t L = 0;
+        float Lf = 0.0f, Lg = 0.0f;
+        int64_t lab = 0;
+        // ex_next: the id under the exclusion cursor, INT64_MAX past the end of the row.  (An int32 sentinel could be
+        // reached: the last chunk of a table ending at 2^31 - 1 spans ids up to id0 + 15 > INT32_MAX.)
+        int64_t ex_cur = 0, ex_end = 0;
+        int64_t ex_next = INT64_MAX;
+        if (EPI == kEpiCount && active) {
+            L = p.label_key[q];
+            lab = p.labels[q];
+            Lf = key_score((u64)L << 32);
+            Lg = L == 0xFFFFFFFFu ? INFINITY : Lf;
+            if constexpr (EXCL) {
+                ex_cur = p.excl_off[q];
+                ex_end = p.excl_off[q + 1];
+                const int64_t first = (int64_t)p.id_base + (int64_t)u.t0 * kBlockN;
+                for (int64_t hi = ex_end; ex_cur < hi;) {
+                    const int64_t mid = (ex_cur + hi) >> 1;
+                    if ((int64_t)p.excl_ids[mid] < first) ex_cur = mid + 1; else hi = mid;
+                }
+                if (ex_cur < ex_end) ex_next = p.excl_ids[ex_cur];
+            }
+        }
+        const uint32_t gt_keep = L == 0xFFFFFFFFu ? 0u : 0xFFFFu;   // NaN label: the NaN columns count only below its id
+        int cnt = 0;
+        for (int t = u.t0; t < u.t1; ++t, ++it) {
+            const uint32_t acc = it & 1;
+            mbar_wait(bar_tfull + 8 * acc, (it >> 1) & 1, 4);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * kBlockN;
+            if constexpr (EPI == kEpiDiag) {
+                uint32_t a[kChunk], b[kChunk];
+                tmem_ld16(taddr + rank * kBlockM + ew * 32, a);
+                tmem_ld16(taddr + rank * kBlockM + ew * 32 + kChunk, b);
+                tmem_ld_wait();
+                // column `lane` of the warp's 32: a select tree on the bits of the lane, constant register indices only
+#pragma unroll
+                for (int j = 0; j < kChunk; ++j) a[j] = lane < kChunk ? a[j] : b[j];
+#pragma unroll
+                for (int h = kChunk / 2; h >= 1; h >>= 1)
+#pragma unroll
+                    for (int j = 0; j < h; ++j) a[j] = (lane & h) ? a[j + h] : a[j];
+                const uint32_t bits = a[0];
+                if (active) {
+                    const int64_t l = p.labels[q];
+                    const bool mine = l >= (int64_t)p.id_base && l < (int64_t)p.id_base + p.N;
+                    p.out_key[q] = mine ? score_key(ranked_score<BF16>(bits)) : 0u;
+                }
+            } else {
+                const int64_t n0 = (int64_t)t * kBlockN;
+                const int nvalid = (int)((p.N - n0) < kBlockN ? (p.N - n0) : kBlockN);
+#pragma unroll 1
+                for (int c = 0; c < nvalid; c += kChunk) {
+                    uint32_t v[kChunk];
+                    tmem_ld16(taddr + c, v);
+                    tmem_ld_wait();
+                    uint32_t gt = 0, eq = 0;
+#pragma unroll
+                    for (int j = 0; j < kChunk; ++j) {
+                        const float f = ranked_score<BF16>(v[j]);
+                        gt |= !(f <= Lg) ? (1u << j) : 0u;
+                        eq |= (f == Lf) ? (1u << j) : 0u;
+                    }
+                    const int64_t id0 = (int64_t)p.id_base + n0 + c;
+                    const int64_t d = lab - id0;                          // columns of the chunk with ids below the label
+                    const uint32_t below = d <= 0 ? 0u : d >= kChunk ? 0xFFFFu : (1u << d) - 1u;
+                    uint32_t m = (gt & (gt_keep | below)) | (eq & below);
+                    if (nvalid - c < kChunk) m &= (1u << (nvalid - c)) - 1u;
+                    if constexpr (EXCL) {
+                        while (ex_next < id0 + kChunk) {
+                            if (ex_next >= id0) m &= ~(1u << (int)(ex_next - id0));
+                            ex_next = ++ex_cur < ex_end ? (int64_t)p.excl_ids[ex_cur] : INT64_MAX;
+                        }
+                    }
+                    cnt += __popc(m);
+                }
+            }
+            // accumulator stage drained: hand it back to the MMA issuer
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) {
+                if (CG == 1 || leader) mbar_arrive_local(bar_tempty + 8 * acc);
+                else mbar_arrive_remote(bar_tempty + 8 * acc, 0);
+            }
+        }
+        if (EPI == kEpiCount && active) p.part[(size_t)u.split * p.Q + q] = cnt;
+    }
+}
+
 // EXCL: leave the items of the row's exclusion list (ExclParams) out of its list.  Phase 2 of the
 // epilogue skips an excluded id before it enters the candidate buffer, so the running threshold stays the exact K-th
 // best of the eligible items.  Inside a unit a row meets its item ids in ascending order (tiles, chunks and bits within
 // a chunk ascend), so a lane-private cursor into the row's sorted list only moves forward: one register compare per
 // survivor of the threshold filter, at most one load per list entry and unit.  A separate instantiation, not a run-time
 // test, because the epilogue's speed depends on its code staying inside the instruction cache (DESIGN.md section 3.4).
-template <int CG, int BK, bool BF16, int EG, bool EXCL>
+template <int CG, int BK, bool BF16, int EG, bool EXCL, int EPI = kEpiTopK>
 __global__ void __launch_bounds__(128 + 128 * EG, 1)
 score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_constant__ CUtensorMap map_ulo,
                   const __grid_constant__ CUtensorMap map_ihi, const __grid_constant__ CUtensorMap map_ilo,
-                  const KernelParams<EXCL> p) {
+                  const KernelParams<EXCL, EPI> p) {
     using C = Cfg<CG, BK, BF16>;
     constexpr int kABytes = C::kABytes;
     extern __shared__ unsigned char smem_raw[];
@@ -517,7 +650,8 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
                 // timeout at every window.
                 bool peers = true;
                 for (int t = u.t0; t < u.t1; ++t) {
-                    const int nrow = t * kBlockN + (int)rank * C::kBRows;
+                    // kEpiDiag: the unit's one tile is the gathered label rows of its own query rows
+                    const int nrow = (EPI == kEpiDiag ? u.qb * CG * kBlockM : t * kBlockN) + (int)rank * C::kBRows;
                     if (pace && u.members > 1) {
                         const int r = t - u.t0;
                         if (r > 0 && r % p.sync_w == 0) {
@@ -617,6 +751,11 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
                 }
             }
         }
+    } else if (EPI != kEpiTopK && warp >= 4) {
+        // ===== label-rank epilogue (a discarded branch in the top-K instantiations, whose Params have no label fields)
+        if constexpr (EPI != kEpiTopK)
+            rank_epilogue<CG, BF16, EXCL, EPI>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id, num_clusters,
+                                               warp, lane);
     } else if (warp >= 4) {
         // ===== epilogue: TMEM -> threshold filter -> per-row candidate buffers -> sorted top-K =====
         // Group g = (warp - 4) / 4 owns accumulator stage g, i.e. every second tile; warp ew of a group reads TMEM
@@ -834,8 +973,11 @@ static int env_int(const char* name, int dflt) {
 }
 // excl: the plan of mr_score_topk_exclude, whose kernels exist only in the default geometry (BK = 32, one epilogue
 // group): it ignores the experiment knobs MR_SCORE_BK and MR_SCORE_BF16_EPI_GROUPS.
-static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false) {
+// rank: the plan of the counting pass (mr_score_rank; K is ignored), same geometry: no top-K warm-up, no merge to
+// bound S, and one int32 per (split, row) instead of the lists and candidate buffers.
+static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false, bool rank = false) {
     Plan pl;
+    if (rank) { excl = true; K = 1; }
     pl.eg = (!excl && bf16 && env_int("MR_SCORE_BF16_EPI_GROUPS", 1) == 2) ? 2 : 1;
     pl.cg = env_int("MR_SCORE_CTA_GROUP", 2) == 1 ? 1 : 2;
     pl.bk = (!excl && env_int("MR_SCORE_BK", 32) == 16) ? 16 : 32;
@@ -847,12 +989,14 @@ static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false)
     // item splits: each unit pays a top-K warm-up (its first tiles pass everything and trigger bursts of row sorts),
     // measured at roughly (8 + K / 5) tile-times; units are executed in waves of `clusters`.  Pick the S that
     // minimises waves * (tiles per unit + warm-up).
-    int smax = 8192 / (pl.eg * (K > 0 ? K : 1));  // mr_topk_merge takes at most 8192 candidates per row
+    int smax = rank ? pl.T : 8192 / (pl.eg * (K > 0 ? K : 1));  // mr_topk_merge takes at most 8192 candidates per row
     if (smax > pl.T) smax = pl.T;
     if (smax < 1) smax = 1;
     int s = env_int("MR_SCORE_SPLITS", 0);
     if (s <= 0) {
-        const double warm = 8.0 + K / 5.0;
+        // the counting pass keeps the K-independent part: it also stands for the L2 sharing that many small units
+        // lose (a wave walks S item streams, each shared by wave / S query blocks)
+        const double warm = rank ? 8.0 : 8.0 + K / 5.0;
         double best = 1e300;
         s = 1;
         for (int c = 1; c <= smax; ++c) {
@@ -873,8 +1017,8 @@ static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false)
     const int64_t units = (int64_t)pl.QB * pl.S;
     pl.grid = (int)((units < clusters ? units : clusters) * pl.cg);
     if (pl.grid < pl.cg) pl.grid = pl.cg;
-    pl.cand_bytes = (int64_t)sms * pl.eg * kBlockM * kCap * 8;
-    pl.part_bytes = (int64_t)pl.S * pl.eg * Q * K * 8;
+    pl.cand_bytes = rank ? 0 : (int64_t)sms * pl.eg * kBlockM * kCap * 8;
+    pl.part_bytes = rank ? (((int64_t)pl.S * Q * 4 + 255) & ~(int64_t)255) : (int64_t)pl.S * pl.eg * Q * K * 8;
     // pacing counters: (query groups x splits) streams x windows of sync_w tiles
     pl.sync_w = env_int("MR_SCORE_PACE_TILES", 1);
     if (pl.sync_w < 1) pl.sync_w = 0;
@@ -885,11 +1029,11 @@ static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false)
     return pl;
 }
 
-template <int CG, int BK, bool BF16, int EG, bool EXCL = false>
+template <int CG, int BK, bool BF16, int EG, bool EXCL = false, int EPI = kEpiTopK, class P = ExclParams>
 static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul, const CUtensorMap& mih, const CUtensorMap& mil,
-                  const ExclParams& p, cudaStream_t stream) {
+                  const P& p, cudaStream_t stream) {
     using C = Cfg<CG, BK, BF16>;
-    cudaError_t e = cudaFuncSetAttribute(score_topk_kernel<CG, BK, BF16, EG, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
+    cudaError_t e = cudaFuncSetAttribute(score_topk_kernel<CG, BK, BF16, EG, EXCL, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     if (e != cudaSuccess) { set_error("mr_score_topk: shared memory attribute: %s", cudaGetErrorString(e)); return (int)e; }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)pl.grid);
@@ -903,11 +1047,67 @@ static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG, EXCL>, muh, mul, mih, mil,
-                           static_cast<const KernelParams<EXCL>&>(p));
+    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG, EXCL, EPI>, muh, mul, mih, mil,
+                           static_cast<const KernelParams<EXCL, EPI>&>(p));
     if (e != cudaSuccess) { set_error("mr_score_topk: launch: %s", cudaGetErrorString(e)); return (int)e; }
     return MR_OK;
 }
+
+// kEpiDiag operand: dst row q = the item row of labels[q] (src row labels[q] - id_base), zeros when the label is not in
+// [id_base, id_base + N); rows of `row_words` 16-byte words.
+__global__ void gather_label_rows_kernel(const uint4* __restrict__ src, uint4* __restrict__ dst, int64_t Q, int64_t N,
+                                         int row_words, int32_t id_base, const int64_t* __restrict__ labels) {
+    const int64_t total = Q * row_words, gsz = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gsz) {
+        const int64_t q = i / row_words, w = i - q * row_words;
+        const int64_t l = labels[q] - id_base;
+        dst[i] = (l >= 0 && l < N) ? src[l * row_words + w] : make_uint4(0, 0, 0, 0);
+    }
+}
+// count[q] = the (split, q) counts of kEpiCount summed in split order, -1 for a row without a label key
+__global__ void rank_finish_kernel(const int32_t* __restrict__ part, int S, int64_t Q, const uint32_t* __restrict__ label_key,
+                                   int32_t* __restrict__ count) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= Q) return;
+    int32_t c = 0;
+    for (int s = 0; s < S; ++s) c += part[(int64_t)s * Q + q];
+    count[q] = label_key[q] ? c : -1;
+}
+
+// Fields and tensor maps shared by the two label-rank passes.  `items` / `items_lo` are the item operand of the pass
+// (the table, or the gathered label rows) with `item_rows` rows.
+static int rank_params(RankParams& p, CUtensorMap (&maps)[4], const Plan& pl, const float* Uhi, const float* Ulo, int64_t Q,
+                       const void* items, const void* items_lo, int64_t item_rows, int64_t N, int E, int32_t id_base,
+                       int mode, const int64_t* labels) {
+    const bool bf16 = mode == MR_SCORE_BF16;
+    p = RankParams{};
+    p.Q = Q; p.N = N; p.E = E; p.K = 1; p.mode = mode; p.id_base = id_base;
+    p.KB = (E + (bf16 ? 63 : 31)) / (bf16 ? 64 : 32);
+    p.T = pl.T; p.QB = pl.QB; p.S = pl.S; p.QG = pl.QG; p.wave = pl.grid / pl.cg;
+    p.l2_hint = env_int("MR_SCORE_L2HINT", 1);
+    p.sync_w = pl.sync_w; p.sync_windows = pl.sync_windows;
+    p.sync_lead = env_int("MR_SCORE_PACE_LEAD", 1);
+    if (p.sync_lead < 1) p.sync_lead = 1;
+    p.sync_giveup = env_int("MR_SCORE_PACE_GIVEUP", 8);
+    p.labels = labels;
+    const int brows = kBlockN / pl.cg;
+    bool ok = make_map(&maps[0], Uhi, Q, E, kBlockM, 32, bf16) && make_map(&maps[2], items, item_rows, E, brows, 32, bf16);
+    if (ok && mode == MR_SCORE_TF32X3)
+        ok = make_map(&maps[1], Ulo, Q, E, kBlockM, 32, false) && make_map(&maps[3], items_lo, item_rows, E, brows, 32, false);
+    else if (ok) { maps[1] = maps[0]; maps[3] = maps[2]; }
+    if (!ok) { set_error("mr_score_rank: cuTensorMapEncodeTiled failed (driver without TMA support?)"); return MR_ERR_UNSUPPORTED; }
+    return MR_OK;
+}
+template <int EPI, bool EXCL>
+static int launch_rank(const Plan& pl, const CUtensorMap (&m)[4], const RankParams& p, bool bf16, cudaStream_t s) {
+    if (bf16) return pl.cg == 1 ? launch<1, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
+                                : launch<2, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s);
+    return pl.cg == 1 ? launch<1, 32, false, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
+                      : launch<2, 32, false, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s);
+}
+static int64_t align256(int64_t n) { return (n + 255) & ~(int64_t)255; }
+// workspace of the label-score pass: the gathered (hi, lo) label rows
+static int64_t diag_bytes(int64_t Q, int E, bool bf16) { return (bf16 ? 1 : 2) * align256(Q * E * (bf16 ? 2 : 4)); }
 
 }  // namespace st
 }  // namespace mr
@@ -1050,4 +1250,127 @@ extern "C" int mr_score_topk_exclude(const float* Uhi, const float* Ulo, int64_t
     MR_REQUIRE(excl_off && excl_ids, "mr_score_topk_exclude: null pointer (excl_off / excl_ids)");
     return score_topk_impl(Uhi, Ulo, Q, Ihi, Ilo, N, E, K, id_base, mode, out_val, out_id, ws, ws_bytes, stream, excl_off,
                            excl_ids);
+}
+
+// ---- label rank against the whole catalog ------------------------------------------------------------------------
+static int rank_check(const char* who, const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo,
+                      int64_t N, int E, int32_t id_base, int mode) {
+    using namespace mr;
+    MR_REQUIRE(Q >= 0 && N >= 0 && E >= 1, "%s: need Q, N >= 0 and E >= 1", who);
+    MR_REQUIRE(mode == MR_SCORE_TF32X3 || mode == MR_SCORE_TF32X1 || mode == MR_SCORE_BF16, "%s: unknown mode %d", who, mode);
+    const bool bf16 = mode == MR_SCORE_BF16;
+    MR_REQUIRE(E % (bf16 ? 8 : 4) == 0, "%s: E=%d must be a multiple of %d (16-byte rows for TMA)", who, E, bf16 ? 8 : 4);
+    MR_REQUIRE(Q < (1ll << 31) - 512 && N < (1ll << 31) - 512 && (int64_t)id_base + N < (1ll << 31),
+               "%s: Q, N and id_base + N must fit 31 bits", who);
+    if (Q == 0) return MR_OK;
+    MR_REQUIRE(Uhi && Ihi, "%s: null pointer", who);
+    MR_REQUIRE(mode != MR_SCORE_TF32X3 || (Ulo && Ilo), "%s: the 3xTF32 mode needs the lo operands", who);
+    MR_REQUIRE(host_aligned16(Uhi) && host_aligned16(Ihi) && host_aligned16(Ulo) && host_aligned16(Ilo),
+               "%s: operands must be 16-byte aligned", who);
+    return MR_OK;
+}
+
+extern "C" int64_t mr_score_rank_workspace_bytes(int64_t Q, int64_t N, int E) {
+    using namespace mr;
+    if (Q < 0 || N < 0 || E < 1) {
+        set_error("mr_score_rank_workspace_bytes: need Q, N >= 0 and E >= 1");
+        return MR_ERR_INVALID_ARG;
+    }
+    if (Q == 0) return 0;
+    // one scratch for both passes and every mode: the gathered fp32 (hi, lo) label rows, or the counting pass's counts
+    // (the plan mr_score_rank builds: N = 0 plans as N = 1)
+    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, false, true, true);
+    const int64_t a = st::diag_bytes(Q, E, false), b = pl.part_bytes + pl.sync_bytes;
+    return (a > b ? a : b) + 256;
+}
+
+extern "C" int mr_label_score(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                              int E, int32_t id_base, int mode, const int64_t* labels, uint32_t* label_key, void* ws,
+                              int64_t ws_bytes, mr_stream_t stream) {
+    using namespace mr;
+    int rc = rank_check("mr_label_score", Uhi, Ulo, Q, Ihi, Ilo, N, E, id_base, mode);
+    if (rc != MR_OK || Q == 0) return rc;
+    MR_REQUIRE(labels && label_key, "mr_label_score: null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (N == 0) {
+        cudaError_t e = cudaMemsetAsync(label_key, 0, (size_t)Q * 4, s);
+        if (e != cudaSuccess) { set_error("mr_label_score: memset: %s", cudaGetErrorString(e)); return (int)e; }
+        return MR_OK;
+    }
+    const bool bf16 = mode == MR_SCORE_BF16;
+    const int64_t need = st::diag_bytes(Q, E, bf16) + 256;
+    if (!ws || ws_bytes < need) {
+        set_error("mr_label_score: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
+        return MR_ERR_WORKSPACE;
+    }
+    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    const int row_bytes = E * (bf16 ? 2 : 4);
+    void* ghi = w;
+    void* glo = w + st::align256(Q * row_bytes);
+    int64_t blocks = (Q * (row_bytes / 16) + 255) / 256;
+    const int64_t cap = (int64_t)sm_count() * 16;
+    if (blocks > cap) blocks = cap;
+    st::gather_label_rows_kernel<<<(unsigned)blocks, 256, 0, s>>>(reinterpret_cast<const uint4*>(Ihi), reinterpret_cast<uint4*>(ghi),
+                                                                  Q, N, row_bytes / 16, id_base, labels);
+    if (mode == MR_SCORE_TF32X3)
+        st::gather_label_rows_kernel<<<(unsigned)blocks, 256, 0, s>>>(reinterpret_cast<const uint4*>(Ilo),
+                                                                      reinterpret_cast<uint4*>(glo), Q, N, row_bytes / 16,
+                                                                      id_base, labels);
+    MR_CUDA_LAUNCH_CHECK("mr_label_score");
+    // one unit per query block, one tile each: the block's own gathered label rows
+    st::Plan pl{};
+    pl.cg = st::env_int("MR_SCORE_CTA_GROUP", 2) == 1 ? 1 : 2;
+    pl.bk = 32; pl.eg = 1;
+    pl.QB = (int)((Q + (int64_t)st::kBlockM * pl.cg - 1) / ((int64_t)st::kBlockM * pl.cg));
+    pl.T = 1; pl.S = 1; pl.QG = 0;
+    const int clusters = sm_count() / pl.cg;
+    pl.grid = (pl.QB < clusters ? pl.QB : clusters) * pl.cg;
+    st::RankParams p;
+    CUtensorMap maps[4];
+    rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, ghi, glo, Q, N, E, id_base, mode, labels);
+    if (rc != MR_OK) return rc;
+    p.out_key = label_key;
+    return st::launch_rank<st::kEpiDiag, false>(pl, maps, p, bf16, s);
+}
+
+extern "C" int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                             int E, int32_t id_base, int mode, const int64_t* labels, const uint32_t* label_key,
+                             const int64_t* excl_off, const int32_t* excl_ids, int32_t* count, void* ws, int64_t ws_bytes,
+                             mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr),
+               "mr_score_rank: excl_off and excl_ids must both be NULL or both be set");
+    int rc = rank_check("mr_score_rank", Uhi, Ulo, Q, Ihi, Ilo, N, E, id_base, mode);
+    if (rc != MR_OK || Q == 0) return rc;
+    MR_REQUIRE(labels && label_key && count, "mr_score_rank: null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, mode == MR_SCORE_BF16, true, true);
+    const int64_t need = pl.part_bytes + pl.sync_bytes + 256;
+    if (!ws || ws_bytes < need) {
+        set_error("mr_score_rank: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
+        return MR_ERR_WORKSPACE;
+    }
+    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    int32_t* part = reinterpret_cast<int32_t*>(w);
+    if (N > 0) {
+        st::RankParams p;
+        CUtensorMap maps[4];
+        rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, Ihi, Ilo, N, N, E, id_base, mode, labels);
+        if (rc != MR_OK) return rc;
+        p.label_key = label_key;
+        p.part = part;
+        p.excl_off = excl_off;
+        p.excl_ids = excl_ids;
+        if (pl.sync_bytes) {
+            p.sync = reinterpret_cast<int32_t*>(w + pl.part_bytes);
+            cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
+            if (e != cudaSuccess) { set_error("mr_score_rank: memset: %s", cudaGetErrorString(e)); return (int)e; }
+        }
+        rc = excl_off ? st::launch_rank<st::kEpiCount, true>(pl, maps, p, mode == MR_SCORE_BF16, s)
+                      : st::launch_rank<st::kEpiCount, false>(pl, maps, p, mode == MR_SCORE_BF16, s);
+        if (rc != MR_OK) return rc;
+    }
+    st::rank_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(part, N > 0 ? pl.S : 0, Q, label_key, count);
+    MR_CUDA_LAUNCH_CHECK("mr_score_rank");
+    return MR_OK;
 }

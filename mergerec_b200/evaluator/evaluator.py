@@ -13,6 +13,7 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Tuple, Union
 
+import numpy as np
 import torch
 
 from .. import _lib
@@ -87,6 +88,48 @@ def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0,
     return out_v, out_i
 
 
+def _exclusion_miss(rank: torch.Tensor, labels: torch.Tensor, exclude: Optional[torch.Tensor]) -> torch.Tensor:
+    """The miss rule of every evaluator path: a label inside its own `exclude` row has rank -1."""
+    if exclude is None:
+        return rank
+    own = (exclude.to(device=rank.device, dtype=torch.int64) == labels[:, None]).any(dim=1)
+    return torch.where(own, torch.full_like(rank, -1), rank)
+
+
+def _device_labels(labels: torch.Tensor, Q: int, dev) -> torch.Tensor:
+    labels = labels.to(device=dev, dtype=torch.int64).contiguous()
+    if labels.dim() != 1 or labels.numel() != Q:
+        raise ValueError(f"labels must be a (Q,) tensor with Q = {Q}")
+    return labels
+
+
+def rank_rows(scores: torch.Tensor, labels: torch.Tensor, id_base: int = 0,
+              exclude: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """(Q,) int32 on the GPU: rank[q] = the number of items of row q of a (Q, N) score matrix, minus `exclude[q]`,
+    that sort before item labels[q] under the top-K order (score desc, id asc), i.e. the label's 0-based position in
+    the full ranking (`mr_rank_rows`); -1 when the label is not an item id of the matrix (id_base + column) or is in
+    its own `exclude` row.  CPU inputs are copied to the GPU in row chunks, as in `topk_rows`."""
+    dev = _lib.require_cuda()
+    lib = _lib.load()
+    if scores.dim() != 2:
+        raise ValueError("scores must be (Q, N)")
+    Q, N = scores.shape
+    labels = _device_labels(labels, Q, dev)
+    csr = _device_csr(exclude, Q, dev)
+    rank = torch.empty(Q, dtype=torch.int32, device=dev)
+    rows_per_chunk = Q if scores.is_cuda else max(1, min(Q, (1 << 30) // max(4 * N, 1)))
+    for q0 in range(0, Q, max(rows_per_chunk, 1)):
+        q1 = min(Q, q0 + rows_per_chunk)
+        chunk = scores[q0:q1].to(device=dev, dtype=torch.float32, non_blocking=True)
+        if chunk.stride(1) != 1:
+            chunk = chunk.contiguous()
+        off, ids = (None, None) if csr is None else (csr[0][q0:], csr[1])   # the offsets index the whole ids array
+        _lib.check(lib.mr_rank_rows(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), id_base, _lib.dptr(labels[q0:q1]),
+                                    _lib.dptr(off), _lib.dptr(ids), _lib.dptr(rank[q0:q1]), _lib.stream_handle()),
+                   "mr_rank_rows")
+    return _exclusion_miss(rank, labels, exclude)
+
+
 def score_topk(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, k: int,
                mode: int = MR_SCORE_TF32X3, out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
                exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -129,6 +172,46 @@ def _score_topk(user_hi, user_lo, table: ShardedItemTable, k: int, mode: int,
     return out_v, out_i
 
 
+def label_score(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, labels: torch.Tensor,
+                mode: int = MR_SCORE_TF32X3) -> torch.Tensor:
+    """(Q,) int32 holding the uint32 score keys of (query q, item labels[q]) against this rank's shard, bit for bit
+    the key of the score `score_topk` ranks, or 0 when this shard does not hold the label (`mr_label_score`).  Over
+    the shards of a catalog, the maximum key (unsigned) is the label's key.  `labels`: (Q,) int64 on the device."""
+    lib = _lib.load()
+    Q, E = user_hi.shape
+    key = torch.empty(Q, dtype=torch.int32, device=user_hi.device)
+    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, table.n_local, E))
+    if ws_bytes < 0:
+        _lib.check(ws_bytes, "mr_score_rank_workspace_bytes")
+    ws = table.workspace(ws_bytes)
+    _lib.check(lib.mr_label_score(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
+                                  table.n_local, E, table.id_base, mode, _lib.dptr(labels), _lib.dptr(key), _lib.dptr(ws),
+                                  ws_bytes, _lib.stream_handle()), "mr_label_score")
+    return key
+
+
+def score_rank(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, labels: torch.Tensor,
+               label_key: torch.Tensor, mode: int = MR_SCORE_TF32X3,
+               csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> torch.Tensor:
+    """(Q,) int32: the number of this shard's items, minus the row's exclusion list (`csr`, from `exclusion_csr`), that
+    sort before the label whose key is `label_key` (`label_score`, maximised over the shards), or -1 where that key is
+    0 (`mr_score_rank`).  Over the shards of a catalog the counts add up to the label's rank; the label's own exclusion
+    is not applied here."""
+    lib = _lib.load()
+    Q, E = user_hi.shape
+    count = torch.empty(Q, dtype=torch.int32, device=user_hi.device)
+    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, table.n_local, E))
+    if ws_bytes < 0:
+        _lib.check(ws_bytes, "mr_score_rank_workspace_bytes")
+    ws = table.workspace(ws_bytes)
+    off, ids = (None, None) if csr is None else csr
+    _lib.check(lib.mr_score_rank(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
+                                 table.n_local, E, table.id_base, mode, _lib.dptr(labels), _lib.dptr(label_key),
+                                 _lib.dptr(off), _lib.dptr(ids), _lib.dptr(count), _lib.dptr(ws), ws_bytes,
+                                 _lib.stream_handle()), "mr_score_rank")
+    return count
+
+
 class PreparedQueries:
     """Query embeddings in the operand format of the scoring kernel ((hi, lo) TF32 split, or bf16), prepared once and
     reusable against any number of item tables / evaluations (`Evaluator.prepare_queries`)."""
@@ -164,7 +247,11 @@ class Evaluator:
                  exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
         """`exclude` (optional): (Q, H) global item ids to leave out of each query's ranking (e.g. its history;
         negative entries are padding), as RecBole's full-sort evaluation does.  A label in its row's `exclude`
-        cannot be hit: it counts as a miss."""
+        cannot be hit: it counts as a miss.  Beyond `topk_rows`'s k <= 1024, the ranks come from `rank_rows`."""
+        if self._max_k > MAX_TOPK:
+            if self._max_k > scores.shape[-1]:
+                raise RuntimeError(f"selected index k out of range (k={self._max_k}, N={scores.shape[-1]})")
+            return self.metrics_from_ranks(rank_rows(scores, labels, exclude=exclude), metric_prefix)
         _, ids = topk_rows(scores, self._max_k, exclude=exclude)
         return self.metrics_from_ids(ids, labels, metric_prefix)
 
@@ -186,6 +273,17 @@ class Evaluator:
         k = self._max_k if k is None else k
         if k > MAX_FUSED_TOPK:
             raise ValueError(f"fused top-k supports k <= {MAX_FUSED_TOPK}")
+        queries, table = self._operands(user_emb, item_emb, normalize, mode, k)
+        csr = _device_csr(exclude, queries.shape[0], queries.hi.device)
+        if table.group is None or table.world == 1:
+            return _score_topk(queries.hi, queries.lo, table, k, mode, None, csr)
+        # sharded: the kernel writes this rank's list into the buffer that the single all-gather sends
+        local, loc_v, loc_i = new_packed_list(queries.shape[0], k, queries.hi.device)
+        _score_topk(queries.hi, queries.lo, table, k, mode, (loc_v, loc_i), csr)
+        return exchange_packed(local, k, table.group, gathered=table.gather_buffer(queries.shape[0], k))
+
+    @staticmethod
+    def _operands(user_emb, item_emb, normalize: bool, mode: int, k: int) -> Tuple["PreparedQueries", ShardedItemTable]:
         _lib.require_cuda()
         table = item_emb if isinstance(item_emb, ShardedItemTable) else ShardedItemTable(
             item_emb, normalize=normalize, bf16=(mode == MR_SCORE_BF16))
@@ -196,13 +294,35 @@ class Evaluator:
         queries = user_emb if isinstance(user_emb, PreparedQueries) else PreparedQueries(user_emb, normalize, table.bf16)
         if queries.bf16 != table.bf16:
             raise ValueError("the queries were prepared for a different scoring mode than the item table")
-        csr = _device_csr(exclude, queries.shape[0], queries.hi.device)
-        if table.group is None or table.world == 1:
-            return _score_topk(queries.hi, queries.lo, table, k, mode, None, csr)
-        # sharded: the kernel writes this rank's list into the buffer that the single all-gather sends
-        local, loc_v, loc_i = new_packed_list(queries.shape[0], k, queries.hi.device)
-        _score_topk(queries.hi, queries.lo, table, k, mode, (loc_v, loc_i), csr)
-        return exchange_packed(local, k, table.group, gathered=table.gather_buffer(queries.shape[0], k))
+        return queries, table
+
+    def label_ranks(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
+                    labels: torch.Tensor, normalize: bool = False, mode: int = MR_SCORE_TF32X3,
+                    exclude: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """(Q,) int32 on the device: rank[q] = the number of items of the whole catalog, minus `exclude[q]`, that sort
+        before item labels[q] in query q's ranking (score desc, id asc) -- the label's 0-based position, with no
+        ceiling on k.  -1 when the label is not an item id of the catalog or is in its own `exclude` row.  Arguments as
+        for `topk_embeddings`.  Computed inside the fused scoring kernel: one pass scores each label (`label_score`),
+        one counts the items ahead of it (`score_rank`).  On a sharded table every rank passes the same queries,
+        labels and `exclude` and receives the same ranks, after two all-reduces of Q words (MAX of the keys, SUM of
+        the counts)."""
+        queries, table = self._operands(user_emb, item_emb, normalize, mode, 1)
+        Q = queries.shape[0]
+        dev = queries.hi.device
+        labels = _device_labels(labels, Q, dev)
+        csr = _device_csr(exclude, Q, dev)
+        key = label_score(queries.hi, queries.lo, table, labels, mode)
+        sharded = table.group is not None and table.world > 1
+        if sharded:   # unsigned maximum as a signed one: flip the sign bit
+            import torch.distributed as dist
+            key ^= -(1 << 31)
+            dist.all_reduce(key, op=dist.ReduceOp.MAX, group=table.group)
+            key ^= -(1 << 31)
+        count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
+        if sharded:
+            dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
+            count = torch.where(key == 0, torch.full_like(count, -1), count)
+        return _exclusion_miss(count, labels, exclude)
 
     def topk_embeddings_streamed(self, user_emb: Union[torch.Tensor, "PreparedQueries"], host_items: torch.Tensor,
                                  k: Optional[int] = None, id_base: int = 0, n_total: Optional[int] = None, group=None,
@@ -303,14 +423,23 @@ class Evaluator:
     def evaluate_embeddings(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
                             labels: torch.Tensor, metric_prefix: str = "", normalize: bool = False,
                             mode: int = MR_SCORE_TF32X3, exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
-        """Metrics of `topk_embeddings`; with `exclude`, a label in its row's `exclude` counts as a miss."""
+        """Metrics of `topk_embeddings`; with `exclude`, a label in its row's `exclude` counts as a miss.  Beyond the
+        fused top-K's k <= 128, the ranks come from `label_ranks`."""
+        if self._max_k > MAX_FUSED_TOPK:
+            queries, table = self._operands(user_emb, item_emb, normalize, mode, self._max_k)
+            return self.metrics_from_ranks(self.label_ranks(queries, table, labels, mode=mode, exclude=exclude),
+                                           metric_prefix)
         _, ids = self.topk_embeddings(user_emb, item_emb, self._max_k, normalize, mode, exclude)
         return self.metrics_from_ids(ids, labels, metric_prefix)
 
     # ------------------------------------------------------------------ shared tail
     def metrics_from_ids(self, ids: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "") -> Dict[str, float]:
         """One rank lookup on the GPU (Q int32 back to the host), then every (metric, k) from the same ranks."""
-        ranks = label_rank(ids, labels).cpu().numpy()
+        return self.metrics_from_ranks(label_rank(ids, labels), metric_prefix)
+
+    def metrics_from_ranks(self, ranks: torch.Tensor, metric_prefix: str = "") -> Dict[str, float]:
+        """Every (metric, k) from each query's 0-based label rank (-1 = miss), e.g. `label_ranks` or `rank_rows`."""
+        ranks = ranks.cpu().numpy() if isinstance(ranks, torch.Tensor) else np.asarray(ranks)
         found = ranks.compress(ranks >= 0)     # compressed once; row order (= the reference's summation order) is kept
         n = int(ranks.shape[0])
         return {metric_prefix + m.name: m.from_found(found, n) for m in self._metrics}

@@ -9,7 +9,6 @@ table built with the very expression the reference evaluates per hit row (metric
 from __future__ import annotations
 
 import sys
-from functools import lru_cache
 from typing import List, Optional
 
 import numpy as np
@@ -18,10 +17,24 @@ import torch
 from .. import _lib
 
 
-@lru_cache(maxsize=None)
+_GAINS = np.zeros(0, dtype=np.float64)
+
+
 def _gain_table(n: int) -> np.ndarray:
-    """gain[r] = 1 / (torch.log2(torch.tensor(r + 2)).item())  -- int64 -> fp32 log2 -> python float."""
-    return np.asarray([1 / (torch.log2(torch.tensor(r + 2)).item()) for r in range(n)], dtype=np.float64)
+    """gain[r] = 1 / (torch.log2(torch.tensor(r + 2)).item())  -- int64 -> fp32 log2 -> python float -- for r < n.
+    One table, extended on demand: each entry costs a torch call, so callers ask only for the ranks that hit."""
+    global _GAINS
+    if _GAINS.size < n:
+        more = [1 / (torch.log2(torch.tensor(r + 2)).item()) for r in range(_GAINS.size, n)]
+        _GAINS = np.concatenate([_GAINS, np.asarray(more, dtype=np.float64)])
+    return _GAINS[:n]
+
+
+def _gains(hit_ranks: np.ndarray) -> np.ndarray:
+    """The gains of the hit rows' ranks, in row order, from a table only as long as the largest of them needs."""
+    if hit_ranks.size == 0:
+        return np.zeros(0, dtype=np.float64)
+    return np.ascontiguousarray(np.take(_gain_table(int(hit_ranks.max()) + 1), hit_ranks), dtype=np.float64)
 
 
 def label_rank(ids: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
@@ -71,8 +84,7 @@ def ndcg_from_ranks(ranks: np.ndarray, k: int) -> float:
     if n == 0:
         return 0.0
     hit = (ranks >= 0) & (ranks < k)
-    table = _gain_table(max(int(k), 1))
-    vals = np.ascontiguousarray(np.take(table, ranks.compress(hit)), dtype=np.float64)
+    vals = _gains(ranks.compress(hit))
     if vals.size == 0:
         return 0 / n
     return _python_float_sum(vals) / n
@@ -90,7 +102,7 @@ def ndcg_from_found(found: np.ndarray, n: int, k: int) -> float:
     """`ndcg_from_ranks` on the compressed form (row order is preserved by the compression, so the summation order is)."""
     if n == 0:
         return 0.0
-    vals = np.ascontiguousarray(np.take(_gain_table(max(int(k), 1)), found.compress(found < k)), dtype=np.float64)
+    vals = _gains(found.compress(found < k))
     if vals.size == 0:
         return 0 / n
     return _python_float_sum(vals) / n

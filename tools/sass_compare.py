@@ -2,9 +2,10 @@
 
     python tools/sass_compare.py OLD.so NEW.so
 
-Kernels are matched by demangled name.  A trailing `false` template argument that a newer build added to a kernel
-(the exclusion flag of score_topk_kernel / topk_rows_kernel) is dropped first, so an existing instantiation is compared
-with its own successor.  Only instruction lines are compared.  Prints one line per kernel; exits 1 when a kernel of OLD
+Kernels are matched by demangled name.  Trailing template arguments that newer builds added to a kernel, at their
+values for the existing instantiations, are dropped first (the exclusion flag `false` of score_topk_kernel /
+topk_rows_kernel, then the epilogue `0` of score_topk_kernel), so an existing instantiation is compared with its own
+successor.  Only instruction lines are compared.  Prints one line per kernel; exits 1 when a kernel of OLD
 is missing from NEW or compiles differently."""
 import os
 import re
@@ -18,6 +19,7 @@ def kernel_name(mangled):
     d = subprocess.run([os.path.join(CUDA_BIN, "cu++filt"), mangled], capture_output=True, text=True, check=True).stdout
     d = re.sub(r"\((int|bool)\)", "", d.strip())
     d = re.match(r"(?:void )?([\w:]+(<[^>]*>)?)", d).group(1).replace(" ", "")
+    d = re.sub(r"^(mr::st::score_topk_kernel<\d+,\d+,\d+,\d+,\d+),0>$", r"\1>", d)
     d = re.sub(r"^(mr::st::score_topk_kernel<\d+,\d+,\d+,\d+),0>$", r"\1>", d)
     return d.replace("topk_rows_kernel<0>", "topk_rows_kernel")
 
