@@ -264,6 +264,25 @@ int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, const float* Ih
                   int32_t id_base, int mode, const int64_t* labels, const uint32_t* label_key, const int64_t* excl_off,
                   const int32_t* excl_ids, int32_t* count, void* ws, int64_t ws_bytes, mr_stream_t stream);
 
+/* Log-softmax of each query's label over the whole catalog, inside the fused scoring kernel: a pass of its own with
+ * the operands, modes and schedule of mr_score_rank, and no list.  The logit of score f is f / temperature; f is the
+ * score the top-K kernel ranks (bf16-rounded in MR_SCORE_BF16).  Supported while |f / temperature| < 1.1e7.
+ * mr_score_lse: this table's partial (shift[q] dev int32, sum[q] dev fp64, Q each) = the sum over row q's eligible
+ *   items (not in its exclusion list; excl_off / excl_ids as for mr_score_rank, both NULL or both set) of
+ *   exp(f / temperature), as sum * 2^shift.  As torch.logsumexp: an eligible NaN gives sum = NaN, an eligible +inf
+ *   gives +inf; no eligible item, or only -inf, gives the empty partial (shift = -2^24, sum = 0), also written for N = 0.
+ *   temperature must be finite and > 0.  ws: dev scratch of at least mr_score_lse_workspace_bytes(Q, N, E) bytes.
+ * mr_lse_finish: merges the (P, Q) partials (shift, sum: row-major, partial p of row q at p * Q + q) of the P shards of
+ *   a catalog in index order, then logp[q] (dev fp32, Q) = min(0, log p) with log p = L / temperature - log(total), L
+ *   the score of label_key[q] (mr_label_score, maximised over the shards), computed in fp64; NaN when label_key[q] is
+ *   0.  The same temperature as mr_score_lse.  Every GPU that merges the same partials gets the same bits. */
+int64_t mr_score_lse_workspace_bytes(int64_t Q, int64_t N, int E);
+int mr_score_lse(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N, int E,
+                 int32_t id_base, int mode, float temperature, const int64_t* excl_off, const int32_t* excl_ids,
+                 int32_t* shift, double* sum, void* ws, int64_t ws_bytes, mr_stream_t stream);
+int mr_lse_finish(const int32_t* shift, const double* sum, int64_t P, int64_t Q, const uint32_t* label_key,
+                  float temperature, float* logp, mr_stream_t stream);
+
 /* Host-only view of the kernel's static schedule for a problem shape (no CUDA call; tests/test_schedule.py).  A unit =
  * (block of 256 queries, contiguous range of 256-item tiles); the grid's CTA pairs run the units in waves of `wave`,
  * unit u on pair u % wave.  plan_out (8 int32): query blocks, item tiles, item splits S, wave, CTAs per pair, item

@@ -52,6 +52,10 @@ SIGNATURES = {
     "mr_score_rank_workspace_bytes": ([_i64, _i64, _i32], _i64),
     "mr_label_score": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_score_rank": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp], C.c_int),
+    "mr_score_lse_workspace_bytes": ([_i64, _i64, _i32], _i64),
+    "mr_score_lse": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
+                     C.c_int),
+    "mr_lse_finish": ([_vp, _vp, _i64, _i64, _vp, C.c_float, _vp, _vp], C.c_int),
     "mr_score_topk_schedule": ([_i64, _i64, _i32, _i32, _vp, _vp, _i64], _i64),
     "mr_to_bf16": ([_vp, _i64, _vp, _vp], C.c_int),
     "mr_split_tf32": ([_vp, _i64, _vp, _vp, _vp], C.c_int),

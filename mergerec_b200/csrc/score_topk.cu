@@ -101,9 +101,22 @@ struct RankParams : ExclParams {
     uint32_t* out_key;           // kEpiDiag: (Q) score key of the label's score, 0 when the label is not in this table
     int32_t* part;               // kEpiCount: (S, Q) counts per item split
 };
+// kEpiLse (mr_score_lse): per (split, row), the exponential sum of the unit's eligible scores as a pair (shift k,
+// sum s) with value s * 2^k in log2 units.  A type of its own, for the same reason again; labels are not read.
+constexpr int kEpiLse = 3;
+struct LseParams : RankParams {
+    float lse_c;                 // log2(e) / temperature: the logit of score f is f * lse_c in log2 units
+    int32_t* lse_shift;          // (S, Q)
+    double* lse_sum;             // (S, Q)
+};
+// Shift range of a (shift, sum) pair: an empty sum is (kLseMinShift, 0).  Logits stay exact in the fp32 fma of the
+// epilogue while |shift| <= 2^24, which bounds the supported |score / temperature| to about 1.1e7.
+constexpr int kLseMinShift = -(1 << 24), kLseMaxShift = 1 << 24;
 template <bool EXCL, int EPI = kEpiTopK>
-using KernelParams = typename std::conditional<EPI != kEpiTopK, RankParams,
-                                               typename std::conditional<EXCL, ExclParams, Params>::type>::type;
+using KernelParams = typename std::conditional<
+    EPI == kEpiLse, LseParams,
+    typename std::conditional<EPI != kEpiTopK, RankParams,
+                              typename std::conditional<EXCL, ExclParams, Params>::type>::type>::type;
 
 // ---- PTX helpers ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -564,6 +577,103 @@ __device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem
     }
 }
 
+__device__ __forceinline__ float ex2_approx(float x) {
+    float y;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+
+// ---- log-sum-exp epilogue (LseParams) -----------------------------------------------------------------------------
+// kEpiLse: the counting pass's schedule and exclusion cursor; per row, the sum of 2^(f c) over the eligible columns
+// (not padding, not in the row's exclusion list) of the unit, f = the score top-K ranks, as acc * 2^k.  Each chunk adds
+// its 16 terms 2^(f c - k), summed in fp32, to the fp64 accumulator.  The integer shift k only rises, and only when a
+// chunk's max(f) c exceeds k + 64, to ceil(max(f) c): the terms stay below 2^64, the first term that set the shift is
+// in (1/2, 1], and the rescale of acc by ldexp is exact, however many chunks raise the shift.  Special values as
+// torch.logsumexp: an eligible NaN gives NaN (its term is NaN; fmaxf, which drops it, only places the shift), an
+// eligible +inf gives +inf (its term is +inf; the shift stays), and a row of -inf or of no eligible item gives the
+// empty pair (kLseMinShift, 0).
+template <int CG, bool BF16, bool EXCL>
+__device__ __forceinline__ void lse_epilogue(const LseParams& p, uint32_t tmem_base, uint32_t bar_tfull,
+                                             uint32_t bar_tempty, uint32_t rank, bool leader, int cluster_id,
+                                             int num_clusters, int warp, int lane) {
+    const int ew = (warp - 4) & 3;
+    const int row = ew * 32 + lane;
+    const float lc = p.lse_c;
+    uint32_t it = 0;
+    Unit u;
+    for (int ui = cluster_id; get_unit(p, ui, u); ui += num_clusters) {
+        const int64_t q = ((int64_t)u.qb * CG + rank) * kBlockM + row;
+        const bool active = q < p.Q;
+        int64_t ex_cur = 0, ex_end = 0;
+        int64_t ex_next = INT64_MAX;   // as in rank_epilogue
+        if constexpr (EXCL) {
+            if (active) {
+                ex_cur = p.excl_off[q];
+                ex_end = p.excl_off[q + 1];
+                const int64_t first = (int64_t)p.id_base + (int64_t)u.t0 * kBlockN;
+                for (int64_t hi = ex_end; ex_cur < hi;) {
+                    const int64_t mid = (ex_cur + hi) >> 1;
+                    if ((int64_t)p.excl_ids[mid] < first) ex_cur = mid + 1; else hi = mid;
+                }
+                if (ex_cur < ex_end) ex_next = p.excl_ids[ex_cur];
+            }
+        }
+        int k = kLseMinShift;
+        double acc = 0.0;
+        for (int t = u.t0; t < u.t1; ++t, ++it) {
+            const uint32_t stage = it & 1;
+            mbar_wait(bar_tfull + 8 * stage, (it >> 1) & 1, 4);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + stage * kBlockN;
+            const int64_t n0 = (int64_t)t * kBlockN;
+            const int nvalid = (int)((p.N - n0) < kBlockN ? (p.N - n0) : kBlockN);
+#pragma unroll 1
+            for (int c = 0; c < nvalid; c += kChunk) {
+                uint32_t v[kChunk];
+                tmem_ld16(taddr + c, v);
+                tmem_ld_wait();
+                uint32_t m = nvalid - c < kChunk ? (1u << (nvalid - c)) - 1u : 0xFFFFu;
+                if constexpr (EXCL) {
+                    const int64_t id0 = (int64_t)p.id_base + n0 + c;
+                    while (ex_next < id0 + kChunk) {
+                        if (ex_next >= id0) m &= ~(1u << (int)(ex_next - id0));
+                        ex_next = ++ex_cur < ex_end ? (int64_t)p.excl_ids[ex_cur] : INT64_MAX;
+                    }
+                }
+                float f[kChunk];
+                float mx = -INFINITY;
+#pragma unroll
+                for (int j = 0; j < kChunk; ++j) {
+                    f[j] = (m >> j) & 1u ? ranked_score<BF16>(v[j]) : -INFINITY;
+                    mx = fmaxf(mx, f[j]);
+                }
+                const float top = mx * lc;
+                if (top > (float)(k + 64) && top < INFINITY) {
+                    const int nk = top < (float)kLseMaxShift ? (int)ceilf(top) : kLseMaxShift;
+                    acc = ldexp(acc, k - nk);
+                    k = nk;
+                }
+                const float nkf = -(float)k;
+                float s = 0.0f;
+#pragma unroll
+                for (int j = 0; j < kChunk; ++j) s += ex2_approx(fmaf(f[j], lc, nkf));
+                acc += (double)s;
+            }
+            // accumulator stage drained: hand it back to the MMA issuer
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) {
+                if (CG == 1 || leader) mbar_arrive_local(bar_tempty + 8 * stage);
+                else mbar_arrive_remote(bar_tempty + 8 * stage, 0);
+            }
+        }
+        if (active) {
+            p.lse_shift[(size_t)u.split * p.Q + q] = k;
+            p.lse_sum[(size_t)u.split * p.Q + q] = acc;
+        }
+    }
+}
+
 // EXCL: leave the items of the row's exclusion list (ExclParams) out of its list.  Phase 2 of the
 // epilogue skips an excluded id before it enters the candidate buffer, so the running threshold stays the exact K-th
 // best of the eligible items.  Inside a unit a row meets its item ids in ascending order (tiles, chunks and bits within
@@ -753,7 +863,10 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
         }
     } else if (EPI != kEpiTopK && warp >= 4) {
         // ===== label-rank epilogue (a discarded branch in the top-K instantiations, whose Params have no label fields)
-        if constexpr (EPI != kEpiTopK)
+        if constexpr (EPI == kEpiLse)
+            lse_epilogue<CG, BF16, EXCL>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id, num_clusters,
+                                         warp, lane);
+        else if constexpr (EPI != kEpiTopK)
             rank_epilogue<CG, BF16, EXCL, EPI>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id, num_clusters,
                                                warp, lane);
     } else if (warp >= 4) {
@@ -1073,6 +1186,35 @@ __global__ void rank_finish_kernel(const int32_t* __restrict__ part, int S, int6
     for (int s = 0; s < S; ++s) c += part[(int64_t)s * Q + q];
     count[q] = label_key[q] ? c : -1;
 }
+// Merges P (shift, sum) partials of kEpiLse per row, in index order: K = the largest shift, total = the sums aligned to
+// it by ldexp (exact) and added in order.  label_key == NULL: writes the merged pair (out_shift, out_sum).  Otherwise
+// writes logp[q] = min(0, (L c - K - log2(total)) ln 2) in fp64, stored as fp32, with L the score of the label's key:
+// the label's log-probability under the softmax of the merged scores, NaN where the key is 0 (no label).  The min only
+// removes the rounding above 0 (the label's own term is inside total) and keeps NaN.
+__global__ void lse_finish_kernel(const int32_t* __restrict__ shift, const double* __restrict__ sum, int P, int64_t Q,
+                                  const uint32_t* __restrict__ label_key, float lc, int32_t* __restrict__ out_shift,
+                                  double* __restrict__ out_sum, float* __restrict__ logp) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= Q) return;
+    int K = kLseMinShift;
+    for (int i = 0; i < P; ++i) K = max(K, shift[(int64_t)i * Q + q]);
+    double total = 0.0;
+    for (int i = 0; i < P; ++i) total += ldexp(sum[(int64_t)i * Q + q], shift[(int64_t)i * Q + q] - K);
+    if (!label_key) {
+        out_shift[q] = K;
+        out_sum[q] = total;
+        return;
+    }
+    const uint32_t L = label_key[q];
+    if (L == 0) {
+        logp[q] = __int_as_float(0x7FC00000);
+        return;
+    }
+    const double x = ((double)key_score((u64)L << 32) * (double)lc - (double)K - log2(total)) * 0.6931471805599453;
+    logp[q] = (float)(x > 0.0 ? 0.0 : x);
+}
+// log2(e) / temperature, rounded once to fp32: the same scale in the epilogue and in the finish
+static float lse_scale(float temperature) { return (float)(1.4426950408889634 / (double)temperature); }
 
 // Fields and tensor maps shared by the two label-rank passes.  `items` / `items_lo` are the item operand of the pass
 // (the table, or the gathered label rows) with `item_rows` rows.
@@ -1098,8 +1240,8 @@ static int rank_params(RankParams& p, CUtensorMap (&maps)[4], const Plan& pl, co
     if (!ok) { set_error("mr_score_rank: cuTensorMapEncodeTiled failed (driver without TMA support?)"); return MR_ERR_UNSUPPORTED; }
     return MR_OK;
 }
-template <int EPI, bool EXCL>
-static int launch_rank(const Plan& pl, const CUtensorMap (&m)[4], const RankParams& p, bool bf16, cudaStream_t s) {
+template <int EPI, bool EXCL, class P>
+static int launch_rank(const Plan& pl, const CUtensorMap (&m)[4], const P& p, bool bf16, cudaStream_t s) {
     if (bf16) return pl.cg == 1 ? launch<1, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
                                 : launch<2, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s);
     return pl.cg == 1 ? launch<1, 32, false, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
@@ -1108,6 +1250,8 @@ static int launch_rank(const Plan& pl, const CUtensorMap (&m)[4], const RankPara
 static int64_t align256(int64_t n) { return (n + 255) & ~(int64_t)255; }
 // workspace of the label-score pass: the gathered (hi, lo) label rows
 static int64_t diag_bytes(int64_t Q, int E, bool bf16) { return (bf16 ? 1 : 2) * align256(Q * E * (bf16 ? 2 : 4)); }
+// partials of the log-sum-exp pass on the counting pass's plan: (S, Q) fp64 sums, then (S, Q) int32 shifts
+static int64_t lse_part_bytes(const Plan& pl, int64_t Q) { return align256(pl.S * Q * 8) + align256(pl.S * Q * 4); }
 
 }  // namespace st
 }  // namespace mr
@@ -1372,5 +1516,81 @@ extern "C" int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, cons
     }
     st::rank_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(part, N > 0 ? pl.S : 0, Q, label_key, count);
     MR_CUDA_LAUNCH_CHECK("mr_score_rank");
+    return MR_OK;
+}
+
+// ---- log-sum-exp of each query's scores over the whole catalog ----------------------------------------------------
+extern "C" int64_t mr_score_lse_workspace_bytes(int64_t Q, int64_t N, int E) {
+    using namespace mr;
+    if (Q < 0 || N < 0 || E < 1) {
+        set_error("mr_score_lse_workspace_bytes: need Q, N >= 0 and E >= 1");
+        return MR_ERR_INVALID_ARG;
+    }
+    if (Q == 0) return 0;
+    // the plan mr_score_lse builds (N = 0 plans as N = 1); the sync counters do not depend on the mode
+    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, false, true, true);
+    return st::lse_part_bytes(pl, Q) + pl.sync_bytes + 256;
+}
+
+extern "C" int mr_score_lse(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
+                            int E, int32_t id_base, int mode, float temperature, const int64_t* excl_off,
+                            const int32_t* excl_ids, int32_t* shift, double* sum, void* ws, int64_t ws_bytes,
+                            mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr),
+               "mr_score_lse: excl_off and excl_ids must both be NULL or both be set");
+    MR_REQUIRE(temperature > 0.0f && temperature < INFINITY, "mr_score_lse: temperature must be finite and > 0");
+    // N = 0: no item operand is read (an empty table may hand in NULL), only the empty partials are written
+    int rc = rank_check("mr_score_lse", Uhi, Ulo, Q, N > 0 ? Ihi : Uhi, N > 0 ? Ilo : Ulo, N, E, id_base, mode);
+    if (rc != MR_OK || Q == 0) return rc;
+    MR_REQUIRE(shift && sum, "mr_score_lse: null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, mode == MR_SCORE_BF16, true, true);
+    const int64_t part_bytes = st::lse_part_bytes(pl, Q);
+    const int64_t need = part_bytes + pl.sync_bytes + 256;
+    if (!ws || ws_bytes < need) {
+        set_error("mr_score_lse: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
+        return MR_ERR_WORKSPACE;
+    }
+    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    double* psum = reinterpret_cast<double*>(w);
+    int32_t* pshift = reinterpret_cast<int32_t*>(w + st::align256(pl.S * Q * 8));
+    const float lc = st::lse_scale(temperature);
+    if (N > 0) {
+        st::LseParams p;
+        CUtensorMap maps[4];
+        rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, Ihi, Ilo, N, N, E, id_base, mode, nullptr);
+        if (rc != MR_OK) return rc;
+        p.lse_c = lc;
+        p.lse_shift = pshift;
+        p.lse_sum = psum;
+        p.excl_off = excl_off;
+        p.excl_ids = excl_ids;
+        if (pl.sync_bytes) {
+            p.sync = reinterpret_cast<int32_t*>(w + part_bytes);
+            cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
+            if (e != cudaSuccess) { set_error("mr_score_lse: memset: %s", cudaGetErrorString(e)); return (int)e; }
+        }
+        rc = excl_off ? st::launch_rank<st::kEpiLse, true>(pl, maps, p, mode == MR_SCORE_BF16, s)
+                      : st::launch_rank<st::kEpiLse, false>(pl, maps, p, mode == MR_SCORE_BF16, s);
+        if (rc != MR_OK) return rc;
+    }
+    // the S splits merged in split order (none for N = 0: the empty pair)
+    st::lse_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(pshift, psum, N > 0 ? pl.S : 0, Q, nullptr, lc,
+                                                                       shift, sum, nullptr);
+    MR_CUDA_LAUNCH_CHECK("mr_score_lse");
+    return MR_OK;
+}
+
+extern "C" int mr_lse_finish(const int32_t* shift, const double* sum, int64_t P, int64_t Q, const uint32_t* label_key,
+                             float temperature, float* logp, mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE(P >= 0 && P < (1 << 20) && Q >= 0 && Q < (1ll << 40), "mr_lse_finish: need 0 <= P < 2^20 and Q >= 0");
+    MR_REQUIRE(temperature > 0.0f && temperature < INFINITY, "mr_lse_finish: temperature must be finite and > 0");
+    if (Q == 0) return MR_OK;
+    MR_REQUIRE(label_key && logp && (P == 0 || (shift && sum)), "mr_lse_finish: null pointer");
+    st::lse_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        shift, sum, (int)P, Q, label_key, st::lse_scale(temperature), nullptr, nullptr, logp);
+    MR_CUDA_LAUNCH_CHECK("mr_lse_finish");
     return MR_OK;
 }

@@ -212,6 +212,46 @@ def score_rank(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: Sh
     return count
 
 
+def score_lse(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, temperature: float,
+              mode: int = MR_SCORE_TF32X3, csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+              out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """This shard's log-sum-exp partial, (shift (Q,) int32, sum (Q,) fp64): the sum over row q's items, minus its
+    exclusion list (`csr`, from `exclusion_csr`), of exp(score / temperature), as sum * 2^shift (`mr_score_lse`).
+    `out`: optional (shift, sum) tensors to write into.  `lse_finish` merges the partials of the shards."""
+    lib = _lib.load()
+    Q, E = user_hi.shape
+    if out is None:
+        out = (torch.empty(Q, dtype=torch.int32, device=user_hi.device),
+               torch.empty(Q, dtype=torch.float64, device=user_hi.device))
+    ws_bytes = int(lib.mr_score_lse_workspace_bytes(Q, table.n_local, E))
+    if ws_bytes < 0:
+        _lib.check(ws_bytes, "mr_score_lse_workspace_bytes")
+    ws = table.workspace(ws_bytes)
+    off, ids = (None, None) if csr is None else csr
+    _lib.check(lib.mr_score_lse(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
+                                table.n_local, E, table.id_base, mode, float(temperature), _lib.dptr(off), _lib.dptr(ids),
+                                _lib.dptr(out[0]), _lib.dptr(out[1]), _lib.dptr(ws), ws_bytes, _lib.stream_handle()),
+               "mr_score_lse")
+    return out
+
+
+def lse_finish(shift: torch.Tensor, sum_: torch.Tensor, label_key: torch.Tensor, temperature: float) -> torch.Tensor:
+    """(Q,) fp32: the label's log-softmax over the catalog whose shards' `score_lse` partials are the rows of `shift`
+    (P, Q) int32 and `sum_` (P, Q) fp64, merged in row order (`mr_lse_finish`), with `label_key` the label keys of
+    `label_score` maximised over the shards; NaN where a key is 0."""
+    lib = _lib.load()
+    if shift.dim() != 2 or sum_.shape != shift.shape or shift.dtype != torch.int32 or sum_.dtype != torch.float64 \
+            or not (shift.is_contiguous() and sum_.is_contiguous()):
+        raise ValueError("expected contiguous (P, Q) int32 shifts and (P, Q) float64 sums")
+    P, Q = shift.shape
+    if label_key.shape != (Q,):
+        raise ValueError(f"label_key must be a (Q,) tensor with Q = {Q}")
+    logp = torch.empty(Q, dtype=torch.float32, device=shift.device)
+    _lib.check(lib.mr_lse_finish(_lib.dptr(shift), _lib.dptr(sum_), P, Q, _lib.dptr(label_key), float(temperature),
+                                 _lib.dptr(logp), _lib.stream_handle()), "mr_lse_finish")
+    return logp
+
+
 class PreparedQueries:
     """Query embeddings in the operand format of the scoring kernel ((hi, lo) TF32 split, or bf16), prepared once and
     reusable against any number of item tables / evaluations (`Evaluator.prepare_queries`)."""
@@ -311,18 +351,60 @@ class Evaluator:
         dev = queries.hi.device
         labels = _device_labels(labels, Q, dev)
         csr = _device_csr(exclude, Q, dev)
+        key = self._label_key(queries, table, labels, mode)
+        count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
+        if table.group is not None and table.world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
+            count = torch.where(key == 0, torch.full_like(count, -1), count)
+        return _exclusion_miss(count, labels, exclude)
+
+    @staticmethod
+    def _label_key(queries: PreparedQueries, table: ShardedItemTable, labels: torch.Tensor, mode: int) -> torch.Tensor:
+        """`label_score`; on a sharded table the all-reduce MAX over the ranks, so every rank holds the label's key."""
         key = label_score(queries.hi, queries.lo, table, labels, mode)
-        sharded = table.group is not None and table.world > 1
-        if sharded:   # unsigned maximum as a signed one: flip the sign bit
+        if table.group is not None and table.world > 1:   # unsigned maximum as a signed one: flip the sign bit
             import torch.distributed as dist
             key ^= -(1 << 31)
             dist.all_reduce(key, op=dist.ReduceOp.MAX, group=table.group)
             key ^= -(1 << 31)
-        count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
-        if sharded:
-            dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
-            count = torch.where(key == 0, torch.full_like(count, -1), count)
-        return _exclusion_miss(count, labels, exclude)
+        return key
+
+    @staticmethod
+    def label_log_softmax(user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
+                          labels: torch.Tensor, temperature: float = 1.0, normalize: bool = False,
+                          mode: int = MR_SCORE_TF32X3, exclude: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """(Q,) fp32 on the device: log_softmax(scores[q] / temperature)[labels[q]] over the whole catalog minus
+        `exclude[q]`, without the score matrix -- the per-query log-likelihood of the label, whose negative mean is
+        the catalog cross-entropy.  NaN when the label is not an item id of the catalog, -inf when it is in its own
+        `exclude` row (probability 0 among the eligible items).  Arguments as for `topk_embeddings`; the scores are
+        those the lists rank (bf16-rounded in `MR_SCORE_BF16`).  Computed inside the fused scoring kernel: one pass
+        scores each label (`label_score`), one sums exp(score / temperature) per row (`score_lse`).  On a sharded table
+        every rank passes the same arguments and receives the same bits, after one all-reduce MAX of the label keys and
+        one all-gather of the (shift, sum) partials, merged in rank order (`lse_finish`)."""
+        queries, table = Evaluator._operands(user_emb, item_emb, normalize, mode, 1)
+        Q = queries.shape[0]
+        dev = queries.hi.device
+        labels = _device_labels(labels, Q, dev)
+        csr = _device_csr(exclude, Q, dev)
+        key = Evaluator._label_key(queries, table, labels, mode)
+        if table.group is None or table.world == 1:
+            shift, sums = score_lse(queries.hi, queries.lo, table, temperature, mode, csr)
+            logp = lse_finish(shift[None], sums[None], key, temperature)
+        else:
+            # one buffer per rank, (sums fp64 | shifts int32) as 3Q words, written by the kernel and sent by ONE all-gather
+            import torch.distributed as dist
+            local = torch.empty(3 * Q, dtype=torch.int32, device=dev)
+            score_lse(queries.hi, queries.lo, table, temperature, mode, csr,
+                      out=(local[2 * Q:], local[:2 * Q].view(torch.float64)))
+            gathered = torch.empty((table.world, 3 * Q), dtype=torch.int32, device=dev)
+            dist.all_gather_into_tensor(gathered.view(-1), local, group=table.group)
+            logp = lse_finish(gathered[:, 2 * Q:].contiguous(), gathered[:, :2 * Q].contiguous().view(torch.float64),
+                              key, temperature)
+        if exclude is not None:   # the miss rule of `_exclusion_miss`, for labels of the catalog
+            own = (exclude.to(device=dev, dtype=torch.int64) == labels[:, None]).any(dim=1) & (key != 0)
+            logp = torch.where(own, torch.full_like(logp, -float("inf")), logp)
+        return logp
 
     def topk_embeddings_streamed(self, user_emb: Union[torch.Tensor, "PreparedQueries"], host_items: torch.Tensor,
                                  k: Optional[int] = None, id_base: int = 0, n_total: Optional[int] = None, group=None,

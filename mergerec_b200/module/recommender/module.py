@@ -19,7 +19,8 @@ is UNPINNED (no Lightning to run), the per-batch metric floats themselves are bi
 
 The encoder forward stays PyTorch; scoring + top-K + Recall / NDCG go through ``Evaluator.evaluate_embeddings``
 (``mr_score_topk``: tcgen05 3xTF32 by default, ``MR_SCORE_BF16`` to mirror the reference's bf16-mixed runs), the
-catalog cross-entropy through ``mr_scores_fp32`` + torch's ``cross_entropy`` on one batch of logits at a time.
+catalog cross-entropy through ``Evaluator.label_log_softmax`` in 3xTF32 whatever the metrics' mode, so that the loss
+stays the fp32 cross-entropy of the reference.
 """
 from __future__ import annotations
 
@@ -29,40 +30,25 @@ from typing import Dict, List, Literal, Optional, Sequence, Union
 import torch
 from torch import nn
 
-from ... import _lib
 from ...evaluator import Evaluator, ShardedItemTable
+from ...evaluator.evaluator import PreparedQueries
 from ...evaluator.sharded import MR_SCORE_BF16, MR_SCORE_TF32X3
 
 __all__ = ["RecEvaluation", "RecJointEvaluation", "WeightedMeanLog", "catalog_cross_entropy"]
 
 
-def _scores_fp32(user: torch.Tensor, items: torch.Tensor) -> torch.Tensor:
-    """(B, N) fp32 scores of one batch on CUDA cores (`mr_scores_fp32`), for the loss only."""
-    lib = _lib.load()
-    B, E = user.shape
-    N = items.shape[0]
-    out = torch.empty((B, N), dtype=torch.float32, device=user.device)
-    if B and N:
-        _lib.check(lib.mr_scores_fp32(_lib.dptr(user), B, _lib.dptr(items), N, E, _lib.dptr(out), N, _lib.stream_handle()),
-                   "mr_scores_fp32")
-    return out
-
-
-def catalog_cross_entropy(user_encoding: torch.Tensor, item_embeddings: torch.Tensor, labels: torch.Tensor,
-                          temperature: float, rows_per_chunk: int = 4096) -> torch.Tensor:
+def catalog_cross_entropy(user_encoding: Union[torch.Tensor, PreparedQueries],
+                          item_embeddings: Union[torch.Tensor, ShardedItemTable], labels: torch.Tensor,
+                          temperature: float) -> torch.Tensor:
     """``nn.functional.cross_entropy(scores / temperature, labels)`` with ``scores = user @ items.T`` (module.py:307, :363),
-    evaluated in row chunks so that at most ``rows_per_chunk x num_items`` logits exist at a time.  Returns the mean loss
-    (a 0-d tensor on the device)."""
-    dev = _lib.require_cuda()
-    user = user_encoding.to(device=dev, dtype=torch.float32).contiguous()
-    items = item_embeddings.to(device=dev, dtype=torch.float32).contiguous()
-    labels = labels.to(device=dev, dtype=torch.int64)
-    total = torch.zeros((), dtype=torch.float32, device=dev)
-    for r0 in range(0, user.shape[0], rows_per_chunk):
-        r1 = min(user.shape[0], r0 + rows_per_chunk)
-        logits = _scores_fp32(user[r0:r1], items) / temperature
-        total = total + nn.functional.cross_entropy(logits, labels[r0:r1], reduction="sum")
-    return total / max(user.shape[0], 1)
+    as ``-Evaluator.label_log_softmax(...).mean()`` in 3xTF32: the fused scoring kernel, no logits in memory.  The mean is
+    taken in fp64 and returned as a 0-d fp32 tensor on the device.  The operands may also be prepared for 3xTF32
+    (``PreparedQueries`` / a ``ShardedItemTable`` without bf16).  Labels outside ``[0, num_items)`` raise ``ValueError``."""
+    n_items = item_embeddings.n_total if isinstance(item_embeddings, ShardedItemTable) else int(item_embeddings.shape[0])
+    if labels.numel() and not bool(((labels >= 0) & (labels < n_items)).all()):
+        raise ValueError(f"labels must be item ids in [0, {n_items})")
+    logp = Evaluator.label_log_softmax(user_encoding, item_embeddings, labels, temperature, mode=MR_SCORE_TF32X3)
+    return (-logp.to(torch.float64).sum() / max(logp.shape[0], 1)).to(torch.float32)
 
 
 class WeightedMeanLog:
@@ -107,6 +93,16 @@ class _EvalBase:
             return items
         return ShardedItemTable(items.detach(), bf16=(self.mode == MR_SCORE_BF16))
 
+    @staticmethod
+    def _loss_table(items: torch.Tensor, table: ShardedItemTable) -> ShardedItemTable:
+        """The 3xTF32 operand of the loss: the metric table itself, or a TF32-split table when that one is bf16."""
+        return ShardedItemTable(items.detach()) if table.bf16 else table
+
+    @staticmethod
+    def _queries(users: torch.Tensor, table: ShardedItemTable) -> Union[torch.Tensor, PreparedQueries]:
+        """Queries prepared once for the metrics and the loss when both take the TF32 split, else left raw."""
+        return users if table.bf16 else PreparedQueries(users)
+
 
 class RecEvaluation(_EvalBase):
     """``RecModule``'s validation / test epoch (module.py:284-359) without the score matrices."""
@@ -116,12 +112,14 @@ class RecEvaluation(_EvalBase):
         super().__init__(evaluator, similarity, temperature, mode)
         self.item_embeddings: Optional[torch.Tensor] = None      # injected like ItemEncodingCallback does
         self._table_cache: Optional[ShardedItemTable] = None
+        self._loss_table_cache: Optional[ShardedItemTable] = None
         self.eval_user_embeddings: List[torch.Tensor] = []
         self.eval_labels: List[torch.Tensor] = []
 
     def set_item_embeddings(self, item_embeddings: torch.Tensor) -> None:
         self.item_embeddings = item_embeddings
         self._table_cache = None
+        self._loss_table_cache = None
 
     def on_epoch_start(self) -> None:
         self.eval_user_embeddings, self.eval_labels = [], []
@@ -139,8 +137,10 @@ class RecEvaluation(_EvalBase):
         labels = torch.cat(self.eval_labels, dim=0)
         if self._table_cache is None:
             self._table_cache = self._table(self.item_embeddings)
-        metrics = self.evaluator.evaluate_embeddings(users, self._table_cache, labels, metric_prefix=f"{stage}/", mode=self.mode)
-        loss = catalog_cross_entropy(users, self.item_embeddings, labels, self.temperature)
+            self._loss_table_cache = self._loss_table(self.item_embeddings, self._table_cache)
+        queries = self._queries(users, self._table_cache)
+        metrics = self.evaluator.evaluate_embeddings(queries, self._table_cache, labels, metric_prefix=f"{stage}/", mode=self.mode)
+        loss = catalog_cross_entropy(queries, self._loss_table_cache, labels, self.temperature)
         metrics[f"{stage}/epoch_loss" if stage == "val" else f"{stage}/loss"] = loss.item()
         return metrics
 
@@ -153,6 +153,7 @@ class RecJointEvaluation(_EvalBase):
         super().__init__(evaluator, similarity, temperature, mode)
         self.item_embeddings: Optional[Sequence[torch.Tensor]] = None    # one table per dataloader (callbacks.py:85-118)
         self._tables: Dict[int, ShardedItemTable] = {}
+        self._loss_tables: Dict[int, ShardedItemTable] = {}
         self._log = WeightedMeanLog()
         self.eval_labels = defaultdict(list)
         self.eval_user_embeddings = defaultdict(list)
@@ -160,6 +161,7 @@ class RecJointEvaluation(_EvalBase):
     def set_item_embeddings(self, item_embeddings: Sequence[torch.Tensor]) -> None:
         self.item_embeddings = item_embeddings
         self._tables = {}
+        self._loss_tables = {}
 
     def on_epoch_start(self) -> None:
         """module.py:421-423, :459-462."""
@@ -173,13 +175,17 @@ class RecJointEvaluation(_EvalBase):
         if self.item_embeddings is None:
             raise RuntimeError("item_embeddings have not been injected")
         if dataloader_idx not in self._tables:
-            self._tables[dataloader_idx] = self._table(self.item_embeddings[dataloader_idx])
+            items = self.item_embeddings[dataloader_idx]
+            self._tables[dataloader_idx] = self._table(items)
+            self._loss_tables[dataloader_idx] = self._loss_table(items, self._tables[dataloader_idx])
+        table = self._tables[dataloader_idx]
         users = self._maybe_normalize(user_encoding.detach()).to(torch.float32)
         self.eval_labels[dataloader_idx].append(labels.detach())
         self.eval_user_embeddings[dataloader_idx].append(users)
         n = int(labels.shape[0])
-        metrics = self.evaluator.evaluate_embeddings(users, self._tables[dataloader_idx], labels, metric_prefix=f"{stage}/", mode=self.mode)
-        loss = catalog_cross_entropy(users, self.item_embeddings[dataloader_idx], labels, self.temperature)
+        queries = self._queries(users, table)
+        metrics = self.evaluator.evaluate_embeddings(queries, table, labels, metric_prefix=f"{stage}/", mode=self.mode)
+        loss = catalog_cross_entropy(queries, self._loss_tables[dataloader_idx], labels, self.temperature)
         suffix = f"/dataloader_idx_{dataloader_idx}"      # what Lightning appends with several dataloaders
         self._log.log_dict({k + suffix: v for k, v in metrics.items()}, batch_size=n)
         self._log.log(f"{stage}/loss{suffix}", loss, batch_size=n)
