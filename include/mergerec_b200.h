@@ -264,6 +264,26 @@ int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, const float* Ih
                   int32_t id_base, int mode, const int64_t* labels, const uint32_t* label_key, const int64_t* excl_off,
                   const int32_t* excl_ids, int32_t* count, void* ws, int64_t ws_bytes, mr_stream_t stream);
 
+/* Label ranks bounded by a cap (exact below it, some value >= cap above it): mr_score_rank on a first slice of the
+ * table (the probe) already finishes every row whose count reached the cap, so the rest of the table is counted only
+ * for the rows still below it, gathered into a compact query set.
+ * mr_rank_compact: one launch; selects the rows q with label_key[q] != 0 && probe[q] < cap in ascending q and writes
+ *   *live (dev int32) = their number n, idx[i] (dev int32, Q) = their rows, out_labels / out_key (Q) = their labels and
+ *   keys, and, when excl_off is set, out_excl_off (dev int64, Q + 1) = the offsets of their exclusion lists packed in
+ *   the same order (out_excl_off[0] = 0; the ids follow with mr_rank_gather).
+ * mr_rank_gather: compacted row i < n = row idx[i] of the query operands hi (and lo, or NULL in the bf16-compat mode),
+ *   rows of row_bytes (a multiple of 16) into out_hi / out_lo, and its exclusion ids into out_excl_ids at
+ *   out_excl_off[i] (the four exclusion pointers all NULL or all set).  n is the host's copy of *live.
+ * mr_rank_add: count[idx[i]] += part[i] for i < n where part[i] >= 0 (count[i] without idx): the rest's counts onto the
+ *   probe's. */
+int mr_rank_compact(int64_t Q, const int32_t* probe, int32_t cap, const uint32_t* label_key, const int64_t* labels,
+                    const int64_t* excl_off, int32_t* live, int32_t* idx, int64_t* out_labels, uint32_t* out_key,
+                    int64_t* out_excl_off, mr_stream_t stream);
+int mr_rank_gather(int64_t n, const int32_t* idx, int64_t row_bytes, const void* hi, const void* lo, void* out_hi,
+                   void* out_lo, const int64_t* excl_off, const int32_t* excl_ids, const int64_t* out_excl_off,
+                   int32_t* out_excl_ids, mr_stream_t stream);
+int mr_rank_add(int64_t n, const int32_t* idx, const int32_t* part, int32_t* count, mr_stream_t stream);
+
 /* Log-softmax of each query's label over the whole catalog, inside the fused scoring kernel: a pass of its own with
  * the operands, modes and schedule of mr_score_rank, and no list.  The logit of score f is f / temperature; f is the
  * score the top-K kernel ranks (bf16-rounded in MR_SCORE_BF16).  Supported while |f / temperature| < 1.1e7.

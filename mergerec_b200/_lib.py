@@ -52,6 +52,9 @@ SIGNATURES = {
     "mr_score_rank_workspace_bytes": ([_i64, _i64, _i32], _i64),
     "mr_label_score": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _i64, _vp], C.c_int),
     "mr_score_rank": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp], C.c_int),
+    "mr_rank_compact": ([_i64, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "mr_rank_gather": ([_i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "mr_rank_add": ([_i64, _vp, _vp, _vp, _vp], C.c_int),
     "mr_score_lse_workspace_bytes": ([_i64, _i64, _i32], _i64),
     "mr_score_lse": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
                      C.c_int),

@@ -1186,6 +1186,79 @@ __global__ void rank_finish_kernel(const int32_t* __restrict__ part, int S, int6
     for (int s = 0; s < S; ++s) c += part[(int64_t)s * Q + q];
     count[q] = label_key[q] ? c : -1;
 }
+// mr_rank_compact, one block: the rows with label_key != 0 && probe < cap in ascending order (each thread scans a
+// contiguous run of rows twice: count, then write at its exclusive prefix), their labels and keys, and the offsets of
+// their exclusion lists in the compacted CSR.
+constexpr int kCompactThreads = 1024;
+__global__ void __launch_bounds__(kCompactThreads) rank_compact_kernel(
+    int64_t Q, const int32_t* __restrict__ probe, int32_t cap, const uint32_t* __restrict__ label_key,
+    const int64_t* __restrict__ labels, const int64_t* __restrict__ excl_off, int32_t* __restrict__ live,
+    int32_t* __restrict__ idx, int64_t* __restrict__ out_labels, uint32_t* __restrict__ out_key,
+    int64_t* __restrict__ out_off) {
+    __shared__ int64_t s_n[kCompactThreads], s_len[kCompactThreads];
+    const int t = threadIdx.x;
+    const int64_t run = (Q + kCompactThreads - 1) / kCompactThreads;
+    const int64_t q0 = min(Q, t * run), q1 = min(Q, q0 + run);
+    auto alive = [&](int64_t q) { return label_key[q] != 0 && probe[q] < cap; };
+    int64_t n = 0, len = 0;
+    for (int64_t q = q0; q < q1; ++q)
+        if (alive(q)) {
+            ++n;
+            if (excl_off) len += excl_off[q + 1] - excl_off[q];
+        }
+    s_n[t] = n;
+    s_len[t] = len;
+    __syncthreads();
+    for (int d = 1; d < kCompactThreads; d <<= 1) {   // inclusive scan (Hillis-Steele)
+        const int64_t a = t >= d ? s_n[t - d] : 0, b = t >= d ? s_len[t - d] : 0;
+        __syncthreads();
+        s_n[t] += a;
+        s_len[t] += b;
+        __syncthreads();
+    }
+    int64_t i = s_n[t] - n, o = s_len[t] - len;
+    for (int64_t q = q0; q < q1; ++q) {
+        if (!alive(q)) continue;
+        idx[i] = (int32_t)q;
+        out_labels[i] = labels[q];
+        out_key[i] = label_key[q];
+        if (excl_off) {
+            o += excl_off[q + 1] - excl_off[q];
+            out_off[i + 1] = o;
+        }
+        ++i;
+    }
+    if (t == kCompactThreads - 1) {
+        *live = (int32_t)s_n[t];
+        if (excl_off) out_off[0] = 0;
+    }
+}
+// mr_rank_gather: compacted row i = source row idx[i] (one block per row): `row_words` 16-byte words of each operand,
+// and the row's exclusion ids.
+__global__ void rank_gather_kernel(int64_t n, const int32_t* __restrict__ idx, int row_words,
+                                   const uint4* __restrict__ hi, const uint4* __restrict__ lo, uint4* __restrict__ out_hi,
+                                   uint4* __restrict__ out_lo, const int64_t* __restrict__ excl_off,
+                                   const int32_t* __restrict__ excl_ids, const int64_t* __restrict__ out_off,
+                                   int32_t* __restrict__ out_ids) {
+    for (int64_t i = blockIdx.x; i < n; i += gridDim.x) {
+        const int64_t q = idx[i];
+        for (int w = threadIdx.x; w < row_words; w += blockDim.x) {
+            out_hi[i * row_words + w] = hi[q * row_words + w];
+            if (lo) out_lo[i * row_words + w] = lo[q * row_words + w];
+        }
+        if (excl_off) {
+            const int64_t a = excl_off[q], m = excl_off[q + 1] - a, d = out_off[i];
+            for (int64_t j = threadIdx.x; j < m; j += blockDim.x) out_ids[d + j] = excl_ids[a + j];
+        }
+    }
+}
+// mr_rank_add: count[q] += part[i] with q = idx[i] (i itself without idx), where part[i] is a count (>= 0)
+__global__ void rank_add_kernel(int64_t n, const int32_t* __restrict__ idx, const int32_t* __restrict__ part,
+                                int32_t* __restrict__ count) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || part[i] < 0) return;
+    count[idx ? idx[i] : i] += part[i];
+}
 // Merges P (shift, sum) partials of kEpiLse per row, in index order: K = the largest shift, total = the sums aligned to
 // it by ldexp (exact) and added in order.  label_key == NULL: writes the merged pair (out_shift, out_sum).  Otherwise
 // writes logp[q] = min(0, (L c - K - log2(total)) ln 2) in fp64, stored as fp32, with L the score of the label's key:
@@ -1516,6 +1589,53 @@ extern "C" int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, cons
     }
     st::rank_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(part, N > 0 ? pl.S : 0, Q, label_key, count);
     MR_CUDA_LAUNCH_CHECK("mr_score_rank");
+    return MR_OK;
+}
+
+// ---- label ranks bounded by a cap: probe a slice of the catalog, count the rest for the rows still below the cap ----
+extern "C" int mr_rank_compact(int64_t Q, const int32_t* probe, int32_t cap, const uint32_t* label_key,
+                               const int64_t* labels, const int64_t* excl_off, int32_t* live, int32_t* idx,
+                               int64_t* out_labels, uint32_t* out_key, int64_t* out_excl_off, mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE(Q >= 0 && Q < (1ll << 31), "mr_rank_compact: need 0 <= Q < 2^31");
+    MR_REQUIRE(probe && label_key && labels && live && idx && out_labels && out_key && (!excl_off || out_excl_off),
+               "mr_rank_compact: null pointer");
+    st::rank_compact_kernel<<<1, st::kCompactThreads, 0, (cudaStream_t)stream>>>(
+        Q, probe, cap, label_key, labels, excl_off, live, idx, out_labels, out_key, out_excl_off);
+    MR_CUDA_LAUNCH_CHECK("mr_rank_compact");
+    return MR_OK;
+}
+
+extern "C" int mr_rank_gather(int64_t n, const int32_t* idx, int64_t row_bytes, const void* hi, const void* lo,
+                              void* out_hi, void* out_lo, const int64_t* excl_off, const int32_t* excl_ids,
+                              const int64_t* out_excl_off, int32_t* out_excl_ids, mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE(n >= 0 && row_bytes > 0 && row_bytes % 16 == 0 && row_bytes < (1ll << 31),
+               "mr_rank_gather: need n >= 0 and rows of a positive multiple of 16 bytes");
+    MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr) && (excl_off == nullptr) == (out_excl_off == nullptr) &&
+                   (excl_off == nullptr) == (out_excl_ids == nullptr),
+               "mr_rank_gather: the four exclusion pointers must all be NULL or all be set");
+    MR_REQUIRE((lo == nullptr) == (out_lo == nullptr), "mr_rank_gather: lo and out_lo must both be NULL or both be set");
+    if (n == 0) return MR_OK;
+    MR_REQUIRE(idx && hi && out_hi, "mr_rank_gather: null pointer");
+    MR_REQUIRE(host_aligned16(hi) && host_aligned16(lo) && host_aligned16(out_hi) && host_aligned16(out_lo),
+               "mr_rank_gather: rows must be 16-byte aligned");
+    const int64_t cap = (int64_t)sm_count() * 16;
+    st::rank_gather_kernel<<<(unsigned)(n < cap ? n : cap), 128, 0, (cudaStream_t)stream>>>(
+        n, idx, (int)(row_bytes / 16), reinterpret_cast<const uint4*>(hi), reinterpret_cast<const uint4*>(lo),
+        reinterpret_cast<uint4*>(out_hi), reinterpret_cast<uint4*>(out_lo), excl_off, excl_ids, out_excl_off,
+        out_excl_ids);
+    MR_CUDA_LAUNCH_CHECK("mr_rank_gather");
+    return MR_OK;
+}
+
+extern "C" int mr_rank_add(int64_t n, const int32_t* idx, const int32_t* part, int32_t* count, mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE(n >= 0 && n < (1ll << 40), "mr_rank_add: need n >= 0");
+    if (n == 0) return MR_OK;
+    MR_REQUIRE(part && count, "mr_rank_add: null pointer");
+    st::rank_add_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, idx, part, count);
+    MR_CUDA_LAUNCH_CHECK("mr_rank_add");
     return MR_OK;
 }
 

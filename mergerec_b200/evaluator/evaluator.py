@@ -11,6 +11,7 @@ Top-K order is (score desc, item id asc): ``torch.topk``'s order among equal sco
 """
 from __future__ import annotations
 
+import os
 from typing import Dict, List, Optional, Tuple, Union
 
 import numpy as np
@@ -192,23 +193,101 @@ def label_score(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: S
 
 def score_rank(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, labels: torch.Tensor,
                label_key: torch.Tensor, mode: int = MR_SCORE_TF32X3,
-               csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> torch.Tensor:
+               csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+               rows: Optional[Tuple[int, int]] = None) -> torch.Tensor:
     """(Q,) int32: the number of this shard's items, minus the row's exclusion list (`csr`, from `exclusion_csr`), that
     sort before the label whose key is `label_key` (`label_score`, maximised over the shards), or -1 where that key is
     0 (`mr_score_rank`).  Over the shards of a catalog the counts add up to the label's rank; the label's own exclusion
-    is not applied here."""
+    is not applied here.  `rows` = (a, b): count only the shard's local rows [a, b) (a count adds up over any split of
+    the catalog, since a score does not depend on where its item sits)."""
     lib = _lib.load()
     Q, E = user_hi.shape
+    a, b = (0, table.n_local) if rows is None else rows
+    if not 0 <= a <= b <= table.n_local:
+        raise ValueError(f"rows [{a}, {b}) outside the shard's {table.n_local} rows")
+    hi, lo = table.hi[a:b], None if table.lo is None else table.lo[a:b]
     count = torch.empty(Q, dtype=torch.int32, device=user_hi.device)
-    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, table.n_local, E))
+    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, b - a, E))
     if ws_bytes < 0:
         _lib.check(ws_bytes, "mr_score_rank_workspace_bytes")
     ws = table.workspace(ws_bytes)
     off, ids = (None, None) if csr is None else csr
-    _lib.check(lib.mr_score_rank(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
-                                 table.n_local, E, table.id_base, mode, _lib.dptr(labels), _lib.dptr(label_key),
+    _lib.check(lib.mr_score_rank(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(hi), _lib.dptr(lo),
+                                 b - a, E, table.id_base + a, mode, _lib.dptr(labels), _lib.dptr(label_key),
                                  _lib.dptr(off), _lib.dptr(ids), _lib.dptr(count), _lib.dptr(ws), ws_bytes,
                                  _lib.stream_handle()), "mr_score_rank")
+    return count
+
+
+# Bounded ranks (`label_ranks(cap=...)`): the probe counts the first 1/PROBE_DIV of each shard (whole 256-item tiles);
+# the rest of the shard is counted only for the rows whose probe count is still below the cap, gathered into a compact
+# query set -- unless more than COMPACT_MAX_LIVE of the rows are live, when the gather would not pay and every row is
+# counted in place.  MR_SCORE_PROBE_DIV overrides the probe size (sweeps).
+PROBE_DIV = 64
+COMPACT_MAX_LIVE = 0.9
+
+
+def _probe_rows(n_local: int) -> int:
+    div = int(os.environ.get("MR_SCORE_PROBE_DIV", "") or PROBE_DIV)
+    return min(n_local, 256 * max(1, round(n_local / (256 * max(div, 1)))))
+
+
+def bounded_count(queries: "PreparedQueries", table: ShardedItemTable, labels: torch.Tensor, key: torch.Tensor,
+                  mode: int, csr: Optional[Tuple[torch.Tensor, torch.Tensor]], cap: int) -> torch.Tensor:
+    """`score_rank` summed over the catalog's shards where that sum is below `cap`, and some count >= `cap` elsewhere
+    (the label's own exclusion not applied; -world on a sharded table where `key` is 0).  A probe over the first
+    `_probe_rows` of each shard finishes every row whose count there already reaches `cap`; `mr_rank_compact` /
+    `mr_rank_gather` gather the others, the rest of the shard is counted for them alone and added (`mr_rank_add`).
+    One host sync (the live count).  On a sharded table: one all-reduce SUM of the Q probe counts, one of the live
+    rows' rest counts; every rank gets the same live rows and the same result."""
+    lib = _lib.load()
+    Q, E = queries.shape
+    dev = queries.hi.device
+    n_local = table.n_local
+    sharded = table.group is not None and table.world > 1
+    if sharded:
+        import torch.distributed as dist
+    n1 = _probe_rows(n_local)
+    count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr, rows=(0, n1))
+    if sharded:
+        dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
+    elif n1 == n_local:
+        return count                    # the probe was the whole table: the counts are exact
+    live = torch.empty(1, dtype=torch.int32, device=dev)
+    idx = torch.empty(Q, dtype=torch.int32, device=dev)
+    labels_c = torch.empty(Q, dtype=torch.int64, device=dev)
+    key_c = torch.empty(Q, dtype=torch.int32, device=dev)
+    off_c = None if csr is None else torch.empty(Q + 1, dtype=torch.int64, device=dev)
+    _lib.check(lib.mr_rank_compact(Q, _lib.dptr(count), cap, _lib.dptr(key), _lib.dptr(labels),
+                                   _lib.dptr(None if csr is None else csr[0]), _lib.dptr(live), _lib.dptr(idx),
+                                   _lib.dptr(labels_c), _lib.dptr(key_c), _lib.dptr(off_c), _lib.stream_handle()),
+               "mr_rank_compact")
+    n = int(live.item())
+    if n == 0:
+        return count
+    rows = (n1, n_local)
+    in_place = n > COMPACT_MAX_LIVE * Q
+    if n1 == n_local:                   # this shard is done; the all-reduce below still needs its (zero) counts
+        rest = torch.zeros(Q if in_place else n, dtype=torch.int32, device=dev)
+    elif in_place:
+        rest = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr, rows=rows)
+    else:
+        hi = torch.empty((n, E), dtype=queries.hi.dtype, device=dev)
+        lo = None if queries.lo is None else torch.empty((n, E), dtype=queries.lo.dtype, device=dev)
+        csr_c = None if csr is None else (off_c[:n + 1], torch.empty_like(csr[1]))
+        _lib.check(lib.mr_rank_gather(n, _lib.dptr(idx), E * queries.hi.element_size(), _lib.dptr(queries.hi),
+                                      _lib.dptr(queries.lo), _lib.dptr(hi), _lib.dptr(lo),
+                                      _lib.dptr(None if csr is None else csr[0]), _lib.dptr(None if csr is None else csr[1]),
+                                      _lib.dptr(None if csr is None else csr_c[0]),
+                                      _lib.dptr(None if csr is None else csr_c[1]), _lib.stream_handle()),
+                   "mr_rank_gather")
+        rest = score_rank(hi, lo, table, labels_c[:n], key_c[:n], mode, csr_c, rows=rows)
+    if sharded:
+        dist.all_reduce(rest, op=dist.ReduceOp.SUM, group=table.group)
+    if in_place:
+        idx, n = None, Q
+    _lib.check(lib.mr_rank_add(n, _lib.dptr(idx), _lib.dptr(rest), _lib.dptr(count), _lib.stream_handle()),
+               "mr_rank_add")
     return count
 
 
@@ -338,24 +417,35 @@ class Evaluator:
 
     def label_ranks(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
                     labels: torch.Tensor, normalize: bool = False, mode: int = MR_SCORE_TF32X3,
-                    exclude: Optional[torch.Tensor] = None) -> torch.Tensor:
+                    exclude: Optional[torch.Tensor] = None, cap: Optional[int] = None) -> torch.Tensor:
         """(Q,) int32 on the device: rank[q] = the number of items of the whole catalog, minus `exclude[q]`, that sort
         before item labels[q] in query q's ranking (score desc, id asc) -- the label's 0-based position, with no
         ceiling on k.  -1 when the label is not an item id of the catalog or is in its own `exclude` row.  Arguments as
         for `topk_embeddings`.  Computed inside the fused scoring kernel: one pass scores each label (`label_score`),
         one counts the items ahead of it (`score_rank`).  On a sharded table every rank passes the same queries,
         labels and `exclude` and receives the same ranks, after two all-reduces of Q words (MAX of the keys, SUM of
-        the counts)."""
+        the counts).
+
+        `cap` (>= 1): a rank is exact where it is below `cap` and is some value >= `cap` elsewhere -- all that Recall@k
+        and NDCG@k need for k <= cap.  Rows whose label is already behind `cap` items of a slice of the catalog are not
+        scored against the rest of it (`bounded_count`); the ranks below `cap` are the same bits as without it."""
         queries, table = self._operands(user_emb, item_emb, normalize, mode, 1)
         Q = queries.shape[0]
         dev = queries.hi.device
         labels = _device_labels(labels, Q, dev)
         csr = _device_csr(exclude, Q, dev)
         key = self._label_key(queries, table, labels, mode)
-        count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
-        if table.group is not None and table.world > 1:
-            import torch.distributed as dist
-            dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
+        sharded = table.group is not None and table.world > 1
+        if cap is not None:
+            if not 1 <= int(cap) < 1 << 31:
+                raise ValueError(f"cap must be in [1, 2^31), not {cap}")
+            count = bounded_count(queries, table, labels, key, mode, csr, int(cap))
+        else:
+            count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
+            if sharded:
+                import torch.distributed as dist
+                dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
+        if sharded:
             count = torch.where(key == 0, torch.full_like(count, -1), count)
         return _exclusion_miss(count, labels, exclude)
 
@@ -505,14 +595,13 @@ class Evaluator:
     def evaluate_embeddings(self, user_emb: Union[torch.Tensor, PreparedQueries], item_emb: Union[torch.Tensor, ShardedItemTable],
                             labels: torch.Tensor, metric_prefix: str = "", normalize: bool = False,
                             mode: int = MR_SCORE_TF32X3, exclude: Optional[torch.Tensor] = None) -> Dict[str, float]:
-        """Metrics of `topk_embeddings`; with `exclude`, a label in its row's `exclude` counts as a miss.  Beyond the
-        fused top-K's k <= 128, the ranks come from `label_ranks`."""
-        if self._max_k > MAX_FUSED_TOPK:
-            queries, table = self._operands(user_emb, item_emb, normalize, mode, self._max_k)
-            return self.metrics_from_ranks(self.label_ranks(queries, table, labels, mode=mode, exclude=exclude),
-                                           metric_prefix)
-        _, ids = self.topk_embeddings(user_emb, item_emb, self._max_k, normalize, mode, exclude)
-        return self.metrics_from_ids(ids, labels, metric_prefix)
+        """Metrics of `topk_embeddings`; with `exclude`, a label in its row's `exclude` counts as a miss.  The ranks
+        come from `label_ranks` with `cap = max(ks)`: a rank at or past max(ks) is a miss for every k, so only the rows
+        whose label is still ahead of max(ks) items after a slice of the catalog are scored against the rest of it.
+        The floats are those of the top-K lists (`metrics_from_ids(topk_embeddings(...))`), bit for bit."""
+        queries, table = self._operands(user_emb, item_emb, normalize, mode, self._max_k)
+        return self.metrics_from_ranks(self.label_ranks(queries, table, labels, mode=mode, exclude=exclude,
+                                                        cap=self._max_k), metric_prefix)
 
     # ------------------------------------------------------------------ shared tail
     def metrics_from_ids(self, ids: torch.Tensor, labels: torch.Tensor, metric_prefix: str = "") -> Dict[str, float]:
