@@ -468,19 +468,33 @@ __device__ __forceinline__ float ranked_score(uint32_t bits) {
     return __uint_as_float(bits);
 }
 
-// ---- label-rank epilogues (RankParams) ----------------------------------------------------------------------------
+__device__ __forceinline__ float ex2_approx(float x) {
+    float y;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+
+// ---- label-pass epilogue (RankParams, LseParams) ------------------------------------------------------------------
 // kEpiDiag: every unit walks one tile, the gathered label rows of its own query rows (host side: label_score), so query
 // row `row` of CTA `rank` meets its label in accumulator column rank * 128 + row.  Two 16-column loads cover a warp's 32
 // columns; each lane selects its own.
-// kEpiCount: per 16-column chunk, bit j = "column j sorts before the row's label" under (score key desc, id asc):
-// greater score, or equal score and smaller id (an arithmetic mask of the ids below the label), minus padding and
-// excluded ids (the forward-only cursor of the EXCL top-K epilogue); the row's count grows by the popc.  No candidate
-// buffer, no sort.  The float tests are the key tests: -0 == +0, and a NaN score is above every other (gt = !(f <= L));
-// for a NaN label only the NaN columns with smaller ids count (Lg = +inf: gt = NaN, eq = never).
-template <int CG, bool BF16, bool EXCL, int EPI>
-__device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem_base, uint32_t bar_tfull,
-                                              uint32_t bar_tempty, uint32_t rank, bool leader, int cluster_id,
-                                              int num_clusters, int warp, int lane) {
+// kEpiCount and kEpiLse walk the unit's tiles in 16-column chunks; a chunk's mask holds the eligible columns: not
+// padding, and not in the row's exclusion list (the forward-only cursor of the EXCL top-K epilogue).
+// kEpiCount: bit j of the mask starts as "column j sorts before the row's label" under (score key desc, id asc):
+// greater score, or equal score and smaller id (an arithmetic mask of the ids below the label); the row's count grows by
+// the popc.  No candidate buffer, no sort.  The float tests are the key tests: -0 == +0, and a NaN score is above every
+// other (gt = !(f <= L)); for a NaN label only the NaN columns with smaller ids count (Lg = +inf: gt = NaN, eq = never).
+// kEpiLse: per row, the sum of 2^(f c) over the eligible columns of the unit, f = the score top-K ranks, as acc * 2^k.
+// Each chunk adds its 16 terms 2^(f c - k), summed in fp32, to the fp64 accumulator.  The integer shift k only rises,
+// and only when a chunk's max(f) c exceeds k + 64, to ceil(max(f) c): the terms stay below 2^64, the first term that set
+// the shift is in (1/2, 1], and the rescale of acc by ldexp is exact, however many chunks raise the shift.  Special
+// values as torch.logsumexp: an eligible NaN gives NaN (its term is NaN; fmaxf, which drops it, only places the shift),
+// an eligible +inf gives +inf (its term is +inf; the shift stays), and a row of -inf or of no eligible item gives the
+// empty pair (kLseMinShift, 0).
+template <int CG, bool BF16, bool EXCL, int EPI, class P>
+__device__ __forceinline__ void label_epilogue(const P& p, uint32_t tmem_base, uint32_t bar_tfull, uint32_t bar_tempty,
+                                               uint32_t rank, bool leader, int cluster_id, int num_clusters, int warp,
+                                               int lane) {
     const int ew = (warp - 4) & 3;
     const int row = ew * 32 + lane;
     uint32_t it = 0;
@@ -495,12 +509,14 @@ __device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem
         // reached: the last chunk of a table ending at 2^31 - 1 spans ids up to id0 + 15 > INT32_MAX.)
         int64_t ex_cur = 0, ex_end = 0;
         int64_t ex_next = INT64_MAX;
-        if (EPI == kEpiCount && active) {
-            L = p.label_key[q];
-            lab = p.labels[q];
-            Lf = key_score((u64)L << 32);
-            Lg = L == 0xFFFFFFFFu ? INFINITY : Lf;
-            if constexpr (EXCL) {
+        if ((EPI == kEpiCount || EXCL) && active) {
+            if (EPI == kEpiCount) {
+                L = p.label_key[q];
+                lab = p.labels[q];
+                Lf = key_score((u64)L << 32);
+                Lg = L == 0xFFFFFFFFu ? INFINITY : Lf;
+            }
+            if (EXCL) {   // the cursor starts at the row's first excluded id >= the unit's first id
                 ex_cur = p.excl_off[q];
                 ex_end = p.excl_off[q + 1];
                 const int64_t first = (int64_t)p.id_base + (int64_t)u.t0 * kBlockN;
@@ -513,11 +529,13 @@ __device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem
         }
         const uint32_t gt_keep = L == 0xFFFFFFFFu ? 0u : 0xFFFFu;   // NaN label: the NaN columns count only below its id
         int cnt = 0;
+        int k = kLseMinShift;
+        double acc = 0.0;
         for (int t = u.t0; t < u.t1; ++t, ++it) {
-            const uint32_t acc = it & 1;
-            mbar_wait(bar_tfull + 8 * acc, (it >> 1) & 1, 4);
+            const uint32_t stage = it & 1;
+            mbar_wait(bar_tfull + 8 * stage, (it >> 1) & 1, 4);
             tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * kBlockN;
+            const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + stage * kBlockN;
             if constexpr (EPI == kEpiDiag) {
                 uint32_t a[kChunk], b[kChunk];
                 tmem_ld16(taddr + rank * kBlockM + ew * 32, a);
@@ -544,17 +562,22 @@ __device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem
                     uint32_t v[kChunk];
                     tmem_ld16(taddr + c, v);
                     tmem_ld_wait();
+                    uint32_t m = 0xFFFFu;   // the eligible columns of the chunk
                     uint32_t gt = 0, eq = 0;
+                    if constexpr (EPI == kEpiCount) {
 #pragma unroll
-                    for (int j = 0; j < kChunk; ++j) {
-                        const float f = ranked_score<BF16>(v[j]);
-                        gt |= !(f <= Lg) ? (1u << j) : 0u;
-                        eq |= (f == Lf) ? (1u << j) : 0u;
+                        for (int j = 0; j < kChunk; ++j) {
+                            const float f = ranked_score<BF16>(v[j]);
+                            gt |= !(f <= Lg) ? (1u << j) : 0u;
+                            eq |= (f == Lf) ? (1u << j) : 0u;
+                        }
                     }
                     const int64_t id0 = (int64_t)p.id_base + n0 + c;
-                    const int64_t d = lab - id0;                          // columns of the chunk with ids below the label
-                    const uint32_t below = d <= 0 ? 0u : d >= kChunk ? 0xFFFFu : (1u << d) - 1u;
-                    uint32_t m = (gt & (gt_keep | below)) | (eq & below);
+                    if constexpr (EPI == kEpiCount) {
+                        const int64_t d = lab - id0;                          // columns of the chunk with ids below the label
+                        const uint32_t below = d <= 0 ? 0u : d >= kChunk ? 0xFFFFu : (1u << d) - 1u;
+                        m = (gt & (gt_keep | below)) | (eq & below);
+                    }
                     if (nvalid - c < kChunk) m &= (1u << (nvalid - c)) - 1u;
                     if constexpr (EXCL) {
                         while (ex_next < id0 + kChunk) {
@@ -562,102 +585,30 @@ __device__ __forceinline__ void rank_epilogue(const RankParams& p, uint32_t tmem
                             ex_next = ++ex_cur < ex_end ? (int64_t)p.excl_ids[ex_cur] : INT64_MAX;
                         }
                     }
-                    cnt += __popc(m);
-                }
-            }
-            // accumulator stage drained: hand it back to the MMA issuer
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-                if (CG == 1 || leader) mbar_arrive_local(bar_tempty + 8 * acc);
-                else mbar_arrive_remote(bar_tempty + 8 * acc, 0);
-            }
-        }
-        if (EPI == kEpiCount && active) p.part[(size_t)u.split * p.Q + q] = cnt;
-    }
-}
-
-__device__ __forceinline__ float ex2_approx(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-
-// ---- log-sum-exp epilogue (LseParams) -----------------------------------------------------------------------------
-// kEpiLse: the counting pass's schedule and exclusion cursor; per row, the sum of 2^(f c) over the eligible columns
-// (not padding, not in the row's exclusion list) of the unit, f = the score top-K ranks, as acc * 2^k.  Each chunk adds
-// its 16 terms 2^(f c - k), summed in fp32, to the fp64 accumulator.  The integer shift k only rises, and only when a
-// chunk's max(f) c exceeds k + 64, to ceil(max(f) c): the terms stay below 2^64, the first term that set the shift is
-// in (1/2, 1], and the rescale of acc by ldexp is exact, however many chunks raise the shift.  Special values as
-// torch.logsumexp: an eligible NaN gives NaN (its term is NaN; fmaxf, which drops it, only places the shift), an
-// eligible +inf gives +inf (its term is +inf; the shift stays), and a row of -inf or of no eligible item gives the
-// empty pair (kLseMinShift, 0).
-template <int CG, bool BF16, bool EXCL>
-__device__ __forceinline__ void lse_epilogue(const LseParams& p, uint32_t tmem_base, uint32_t bar_tfull,
-                                             uint32_t bar_tempty, uint32_t rank, bool leader, int cluster_id,
-                                             int num_clusters, int warp, int lane) {
-    const int ew = (warp - 4) & 3;
-    const int row = ew * 32 + lane;
-    const float lc = p.lse_c;
-    uint32_t it = 0;
-    Unit u;
-    for (int ui = cluster_id; get_unit(p, ui, u); ui += num_clusters) {
-        const int64_t q = ((int64_t)u.qb * CG + rank) * kBlockM + row;
-        const bool active = q < p.Q;
-        int64_t ex_cur = 0, ex_end = 0;
-        int64_t ex_next = INT64_MAX;   // as in rank_epilogue
-        if constexpr (EXCL) {
-            if (active) {
-                ex_cur = p.excl_off[q];
-                ex_end = p.excl_off[q + 1];
-                const int64_t first = (int64_t)p.id_base + (int64_t)u.t0 * kBlockN;
-                for (int64_t hi = ex_end; ex_cur < hi;) {
-                    const int64_t mid = (ex_cur + hi) >> 1;
-                    if ((int64_t)p.excl_ids[mid] < first) ex_cur = mid + 1; else hi = mid;
-                }
-                if (ex_cur < ex_end) ex_next = p.excl_ids[ex_cur];
-            }
-        }
-        int k = kLseMinShift;
-        double acc = 0.0;
-        for (int t = u.t0; t < u.t1; ++t, ++it) {
-            const uint32_t stage = it & 1;
-            mbar_wait(bar_tfull + 8 * stage, (it >> 1) & 1, 4);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + stage * kBlockN;
-            const int64_t n0 = (int64_t)t * kBlockN;
-            const int nvalid = (int)((p.N - n0) < kBlockN ? (p.N - n0) : kBlockN);
-#pragma unroll 1
-            for (int c = 0; c < nvalid; c += kChunk) {
-                uint32_t v[kChunk];
-                tmem_ld16(taddr + c, v);
-                tmem_ld_wait();
-                uint32_t m = nvalid - c < kChunk ? (1u << (nvalid - c)) - 1u : 0xFFFFu;
-                if constexpr (EXCL) {
-                    const int64_t id0 = (int64_t)p.id_base + n0 + c;
-                    while (ex_next < id0 + kChunk) {
-                        if (ex_next >= id0) m &= ~(1u << (int)(ex_next - id0));
-                        ex_next = ++ex_cur < ex_end ? (int64_t)p.excl_ids[ex_cur] : INT64_MAX;
+                    if constexpr (EPI == kEpiCount) {
+                        cnt += __popc(m);
+                    } else {
+                        const float lc = p.lse_c;
+                        float f[kChunk];
+                        float mx = -INFINITY;
+#pragma unroll
+                        for (int j = 0; j < kChunk; ++j) {
+                            f[j] = (m >> j) & 1u ? ranked_score<BF16>(v[j]) : -INFINITY;
+                            mx = fmaxf(mx, f[j]);
+                        }
+                        const float top = mx * lc;
+                        if (top > (float)(k + 64) && top < INFINITY) {
+                            const int nk = top < (float)kLseMaxShift ? (int)ceilf(top) : kLseMaxShift;
+                            acc = ldexp(acc, k - nk);
+                            k = nk;
+                        }
+                        const float nkf = -(float)k;
+                        float s = 0.0f;
+#pragma unroll
+                        for (int j = 0; j < kChunk; ++j) s += ex2_approx(fmaf(f[j], lc, nkf));
+                        acc += (double)s;
                     }
                 }
-                float f[kChunk];
-                float mx = -INFINITY;
-#pragma unroll
-                for (int j = 0; j < kChunk; ++j) {
-                    f[j] = (m >> j) & 1u ? ranked_score<BF16>(v[j]) : -INFINITY;
-                    mx = fmaxf(mx, f[j]);
-                }
-                const float top = mx * lc;
-                if (top > (float)(k + 64) && top < INFINITY) {
-                    const int nk = top < (float)kLseMaxShift ? (int)ceilf(top) : kLseMaxShift;
-                    acc = ldexp(acc, k - nk);
-                    k = nk;
-                }
-                const float nkf = -(float)k;
-                float s = 0.0f;
-#pragma unroll
-                for (int j = 0; j < kChunk; ++j) s += ex2_approx(fmaf(f[j], lc, nkf));
-                acc += (double)s;
             }
             // accumulator stage drained: hand it back to the MMA issuer
             tc_fence_before();
@@ -667,9 +618,13 @@ __device__ __forceinline__ void lse_epilogue(const LseParams& p, uint32_t tmem_b
                 else mbar_arrive_remote(bar_tempty + 8 * stage, 0);
             }
         }
-        if (active) {
-            p.lse_shift[(size_t)u.split * p.Q + q] = k;
-            p.lse_sum[(size_t)u.split * p.Q + q] = acc;
+        if constexpr (EPI == kEpiCount) {
+            if (active) p.part[(size_t)u.split * p.Q + q] = cnt;
+        } else if constexpr (EPI == kEpiLse) {
+            if (active) {
+                p.lse_shift[(size_t)u.split * p.Q + q] = k;
+                p.lse_sum[(size_t)u.split * p.Q + q] = acc;
+            }
         }
     }
 }
@@ -862,13 +817,10 @@ score_topk_kernel(const __grid_constant__ CUtensorMap map_uhi, const __grid_cons
             }
         }
     } else if (EPI != kEpiTopK && warp >= 4) {
-        // ===== label-rank epilogue (a discarded branch in the top-K instantiations, whose Params have no label fields)
-        if constexpr (EPI == kEpiLse)
-            lse_epilogue<CG, BF16, EXCL>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id, num_clusters,
-                                         warp, lane);
-        else if constexpr (EPI != kEpiTopK)
-            rank_epilogue<CG, BF16, EXCL, EPI>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id, num_clusters,
-                                               warp, lane);
+        // ===== label-pass epilogue (a discarded branch in the top-K instantiations, whose Params have no label fields)
+        if constexpr (EPI != kEpiTopK)
+            label_epilogue<CG, BF16, EXCL, EPI>(p, tmem_base, bar_tfull, bar_tempty, rank, leader, cluster_id,
+                                                num_clusters, warp, lane);
     } else if (warp >= 4) {
         // ===== epilogue: TMEM -> threshold filter -> per-row candidate buffers -> sorted top-K =====
         // Group g = (warp - 4) / 4 owns accumulator stage g, i.e. every second tile; warp ew of a group reads TMEM
@@ -1075,76 +1027,143 @@ static bool make_map(CUtensorMap* map, const void* ptr, int64_t rows, int E, int
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// The passes of the kernel: the top-K lists (without and with exclusion lists) and the label passes of mr_label_score
+// (kEpiDiag), mr_score_rank (kEpiCount) and mr_score_lse (kEpiLse).
+enum class Pass { TopK, TopKExcl, Diag, Count, Lse };
 struct Plan {
+    Pass pass;
+    bool bf16;
     int cg, bk, eg, QB, T, S, QG, grid;
     int64_t cand_bytes, part_bytes, sync_bytes;
     int sync_w, sync_windows;
+    int streams;   // item streams = query groups x splits, each with sync_windows pacing counters
 };
 static int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
     return (v && *v) ? atoi(v) : dflt;
 }
-// excl: the plan of mr_score_topk_exclude, whose kernels exist only in the default geometry (BK = 32, one epilogue
-// group): it ignores the experiment knobs MR_SCORE_BK and MR_SCORE_BF16_EPI_GROUPS.
-// rank: the plan of the counting pass (mr_score_rank; K is ignored), same geometry: no top-K warm-up, no merge to
-// bound S, and one int32 per (split, row) instead of the lists and candidate buffers.
-static Plan make_plan(int64_t Q, int64_t N, int K, bool bf16, bool excl = false, bool rank = false) {
-    Plan pl;
-    if (rank) { excl = true; K = 1; }
-    pl.eg = (!excl && bf16 && env_int("MR_SCORE_BF16_EPI_GROUPS", 1) == 2) ? 2 : 1;
+static int64_t align256(int64_t n) { return (n + 255) & ~(int64_t)255; }
+// The plan of one pass over Q queries, N items of E elements (the top-K passes do not depend on E, the label passes not
+// on K).  Only the top-K pass without exclusion has the experiment geometries (MR_SCORE_BK = 16 for fp32 operands,
+// MR_SCORE_BF16_EPI_GROUPS = 2 in bf16-compat mode); every other pass exists only with BK = 32 and one epilogue group.
+// The counting and log-sum-exp passes plan as K = 1: no top-K warm-up, no merge to bound S, and partials of one or two
+// words per (split, row) instead of the lists and candidate buffers.  The label-score pass is one unit per query block,
+// one tile each (the block's own gathered label rows): no splits, no query groups, no pacing.
+static Plan make_plan(Pass pass, int64_t Q, int64_t N, int E, int K, bool bf16) {
+    Plan pl{};
+    pl.pass = pass;
+    pl.bf16 = bf16;
+    const bool topk = pass == Pass::TopK || pass == Pass::TopKExcl, label = !topk;
+    if (label) K = 1;
+    pl.eg = (pass == Pass::TopK && bf16 && env_int("MR_SCORE_BF16_EPI_GROUPS", 1) == 2) ? 2 : 1;
     pl.cg = env_int("MR_SCORE_CTA_GROUP", 2) == 1 ? 1 : 2;
-    pl.bk = (!excl && env_int("MR_SCORE_BK", 32) == 16) ? 16 : 32;
+    // bf16 rows are 64 elements = 128 bytes: the BK = 32 geometry
+    pl.bk = (pass == Pass::TopK && !bf16 && env_int("MR_SCORE_BK", 32) == 16) ? 16 : 32;
     const int sms = sm_count();
     const int clusters = sms / pl.cg;
     pl.QB = (int)((Q + (int64_t)kBlockM * pl.cg - 1) / ((int64_t)kBlockM * pl.cg));
-    pl.T = (int)((N + kBlockN - 1) / kBlockN);
-    pl.QG = 0;   // set below, once the number of splits is known
-    // item splits: each unit pays a top-K warm-up (its first tiles pass everything and trigger bursts of row sorts),
-    // measured at roughly (8 + K / 5) tile-times; units are executed in waves of `clusters`.  Pick the S that
-    // minimises waves * (tiles per unit + warm-up).
-    int smax = rank ? pl.T : 8192 / (pl.eg * (K > 0 ? K : 1));  // mr_topk_merge takes at most 8192 candidates per row
-    if (smax > pl.T) smax = pl.T;
-    if (smax < 1) smax = 1;
-    int s = env_int("MR_SCORE_SPLITS", 0);
-    if (s <= 0) {
-        // the counting pass keeps the K-independent part: it also stands for the L2 sharing that many small units
-        // lose (a wave walks S item streams, each shared by wave / S query blocks)
-        const double warm = rank ? 8.0 : 8.0 + K / 5.0;
-        double best = 1e300;
-        s = 1;
-        for (int c = 1; c <= smax; ++c) {
-            const int64_t units = (int64_t)pl.QB * c;
-            const int64_t waves = (units + clusters - 1) / clusters;
-            const double cost = (double)waves * ((double)((pl.T + c - 1) / c) + warm);
-            if (cost < best * (1.0 - 1e-9)) { best = cost; s = c; }
+    if (pass == Pass::Diag) {
+        pl.T = 1;
+        pl.S = 1;
+    } else {
+        pl.T = (int)((N + kBlockN - 1) / kBlockN);
+        // item splits: each unit pays a top-K warm-up (its first tiles pass everything and trigger bursts of row sorts),
+        // measured at roughly (8 + K / 5) tile-times; units are executed in waves of `clusters`.  Pick the S that
+        // minimises waves * (tiles per unit + warm-up).
+        int smax = label ? pl.T : 8192 / (pl.eg * (K > 0 ? K : 1));  // mr_topk_merge takes at most 8192 candidates per row
+        if (smax > pl.T) smax = pl.T;
+        if (smax < 1) smax = 1;
+        int s = env_int("MR_SCORE_SPLITS", 0);
+        if (s <= 0) {
+            // the label passes keep the K-independent part: it also stands for the L2 sharing that many small units
+            // lose (a wave walks S item streams, each shared by wave / S query blocks)
+            const double warm = label ? 8.0 : 8.0 + K / 5.0;
+            double best = 1e300;
+            s = 1;
+            for (int c = 1; c <= smax; ++c) {
+                const int64_t units = (int64_t)pl.QB * c;
+                const int64_t waves = (units + clusters - 1) / clusters;
+                const double cost = (double)waves * ((double)((pl.T + c - 1) / c) + warm);
+                if (cost < best * (1.0 - 1e-9)) { best = cost; s = c; }
+            }
         }
+        if (s > smax) s = smax;
+        pl.S = s;
+        // One wave of CTA pairs walks only S item streams (get_unit's wave-aligned order), so an item tile is shared by
+        // wave / S query blocks and the query operands of a wave fit L2 next to the item streams (measured at BASELINE
+        // config 5 with the L2 eviction hints, as explicit groups QG x S: 37 x 2 -> 443 ms; 16 x 2 -> 447; 18 x 4 -> 466;
+        // 8 x 9 -> 481; 74 x 2 -> 548).  MR_SCORE_QGROUP = explicit query groups of that many blocks (experiments).
+        pl.QG = env_int("MR_SCORE_QGROUP", 0);
+        if (pl.QG < 0) pl.QG = 0;
+        // pacing counters: (query groups x splits) streams x windows of sync_w tiles
+        pl.sync_w = env_int("MR_SCORE_PACE_TILES", 1);
+        if (pl.sync_w < 1) pl.sync_w = 0;
     }
-    if (s > smax) s = smax;
-    pl.S = s;
-    // One wave of CTA pairs walks only S item streams (get_unit's wave-aligned order), so an item tile is shared by
-    // wave / S query blocks and the query operands of a wave fit L2 next to the item streams (measured at BASELINE
-    // config 5 with the L2 eviction hints, as explicit groups QG x S: 37 x 2 -> 443 ms; 16 x 2 -> 447; 18 x 4 -> 466;
-    // 8 x 9 -> 481; 74 x 2 -> 548).  MR_SCORE_QGROUP = explicit query groups of that many blocks (experiments).
-    pl.QG = env_int("MR_SCORE_QGROUP", 0);
-    if (pl.QG < 0) pl.QG = 0;
     const int64_t units = (int64_t)pl.QB * pl.S;
     pl.grid = (int)((units < clusters ? units : clusters) * pl.cg);
     if (pl.grid < pl.cg) pl.grid = pl.cg;
-    pl.cand_bytes = rank ? 0 : (int64_t)sms * pl.eg * kBlockM * kCap * 8;
-    pl.part_bytes = rank ? (((int64_t)pl.S * Q * 4 + 255) & ~(int64_t)255) : (int64_t)pl.S * pl.eg * Q * K * 8;
-    // pacing counters: (query groups x splits) streams x windows of sync_w tiles
-    pl.sync_w = env_int("MR_SCORE_PACE_TILES", 1);
-    if (pl.sync_w < 1) pl.sync_w = 0;
     const int wave = pl.grid / pl.cg;
-    const int groups = pl.QG ? (pl.QB + pl.QG - 1) / pl.QG : (int)((units + wave - 1) / wave);   // streams = groups x S
+    const int groups = pl.QG ? (pl.QB + pl.QG - 1) / pl.QG : (int)((units + wave - 1) / wave);
+    pl.streams = groups * pl.S;
     pl.sync_windows = pl.sync_w ? ((pl.T + pl.S - 1) / pl.S + pl.sync_w - 1) / pl.sync_w + 2 : 0;
-    pl.sync_bytes = pl.sync_w ? (((int64_t)groups * pl.S * pl.sync_windows * 4 + 255) & ~(int64_t)255) : 0;
+    pl.sync_bytes = pl.sync_w ? align256((int64_t)groups * pl.S * pl.sync_windows * 4) : 0;
+    pl.cand_bytes = topk ? (int64_t)sms * pl.eg * kBlockM * kCap * 8 : 0;
+    switch (pass) {
+    case Pass::TopK:
+    case Pass::TopKExcl: pl.part_bytes = (int64_t)pl.S * pl.eg * Q * K * 8; break;   // (S * EG, Q, K) values, then ids
+    case Pass::Diag: pl.part_bytes = (bf16 ? 1 : 2) * align256(Q * E * (bf16 ? 2 : 4)); break;   // gathered (hi, lo) rows
+    case Pass::Count: pl.part_bytes = align256(pl.S * Q * 4); break;   // (S, Q) int32 counts
+    case Pass::Lse: pl.part_bytes = align256(pl.S * Q * 8) + align256(pl.S * Q * 4); break;   // (S, Q) fp64 sums, int32 shifts
+    }
     return pl;
 }
+// scratch of a pass: 256 bytes of alignment slack, then candidate buffers, partials and pacing counters
+static int64_t ws_need(const Plan& pl) { return pl.cand_bytes + pl.part_bytes + pl.sync_bytes + 256; }
+static unsigned char* ws_base(void* ws) {
+    return reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+}
 
-template <int CG, int BK, bool BF16, int EG, bool EXCL = false, int EPI = kEpiTopK, class P = ExclParams>
-static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul, const CUtensorMap& mih, const CUtensorMap& mil,
-                  const P& p, cudaStream_t stream) {
+// What every pass does before its launch: check the workspace (`w`: its 256-byte aligned start), fill the Params fields
+// the passes share, zero the pacing counters and encode the four tensor maps.  `Ihi` / `Ilo` are the item operand of the
+// pass: the table of N rows, or for kEpiDiag the Q gathered label rows.  With N = 0 only the workspace is checked.
+template <class P>
+static int setup_pass(const char* who, const Plan& pl, P& p, CUtensorMap (&m)[4], unsigned char*& w, const float* Uhi,
+                      const float* Ulo, int64_t Q, const void* Ihi, const void* Ilo, int64_t N, int E, int K,
+                      int32_t id_base, int mode, void* ws, int64_t ws_bytes, cudaStream_t s) {
+    const int64_t need = ws_need(pl);
+    if (!ws || ws_bytes < need) {
+        set_error("%s: workspace of %lld bytes needed, %lld given", who, (long long)need, (long long)ws_bytes);
+        return MR_ERR_WORKSPACE;
+    }
+    w = ws_base(ws);
+    if (N == 0) return MR_OK;
+    p = P{};
+    p.Q = Q; p.N = N; p.E = E; p.K = K; p.mode = mode; p.id_base = id_base;
+    const int kelems = pl.bf16 ? 64 : pl.bk;
+    p.KB = (E + kelems - 1) / kelems;
+    p.T = pl.T; p.QB = pl.QB; p.S = pl.S; p.QG = pl.QG; p.wave = pl.grid / pl.cg;
+    p.l2_hint = env_int("MR_SCORE_L2HINT", 1);
+    p.sync_w = pl.sync_w; p.sync_windows = pl.sync_windows;
+    p.sync_lead = env_int("MR_SCORE_PACE_LEAD", 1);   // lead 1 / 2 / 3 at config 5: 376.5 / 379.6 / 381.2 ms
+    if (p.sync_lead < 1) p.sync_lead = 1;
+    p.sync_giveup = env_int("MR_SCORE_PACE_GIVEUP", 8);
+    if (pl.sync_bytes) {
+        p.sync = reinterpret_cast<int32_t*>(w + pl.cand_bytes + pl.part_bytes);
+        cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
+        if (e != cudaSuccess) { set_error("%s: memset: %s", who, cudaGetErrorString(e)); return (int)e; }
+    }
+    const int64_t item_rows = pl.pass == Pass::Diag ? Q : N;
+    const int brows = kBlockN / pl.cg;
+    bool ok = make_map(&m[0], Uhi, Q, E, kBlockM, pl.bk, pl.bf16) && make_map(&m[2], Ihi, item_rows, E, brows, pl.bk, pl.bf16);
+    if (ok && mode == MR_SCORE_TF32X3)
+        ok = make_map(&m[1], Ulo, Q, E, kBlockM, pl.bk, false) && make_map(&m[3], Ilo, item_rows, E, brows, pl.bk, false);
+    else if (ok) { m[1] = m[0]; m[3] = m[2]; }
+    if (!ok) { set_error("%s: cuTensorMapEncodeTiled failed (driver without TMA support?)", who); return MR_ERR_UNSUPPORTED; }
+    return MR_OK;
+}
+
+template <int CG, int BK, bool BF16, int EG, bool EXCL, int EPI, class P>
+static int launch(const Plan& pl, const CUtensorMap (&m)[4], const P& p, cudaStream_t stream) {
     using C = Cfg<CG, BK, BF16>;
     cudaError_t e = cudaFuncSetAttribute(score_topk_kernel<CG, BK, BF16, EG, EXCL, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     if (e != cudaSuccess) { set_error("mr_score_topk: shared memory attribute: %s", cudaGetErrorString(e)); return (int)e; }
@@ -1160,10 +1179,29 @@ static int launch(const Plan& pl, const CUtensorMap& muh, const CUtensorMap& mul
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG, EXCL, EPI>, muh, mul, mih, mil,
+    e = cudaLaunchKernelEx(&cfg, score_topk_kernel<CG, BK, BF16, EG, EXCL, EPI>, m[0], m[1], m[2], m[3],
                            static_cast<const KernelParams<EXCL, EPI>&>(p));
     if (e != cudaSuccess) { set_error("mr_score_topk: launch: %s", cudaGetErrorString(e)); return (int)e; }
     return MR_OK;
+}
+template <int BK, bool BF16, int EG, bool EXCL, int EPI, class P>
+static int launch_cg(const Plan& pl, const CUtensorMap (&m)[4], const P& p, cudaStream_t s) {
+    return pl.cg == 1 ? launch<1, BK, BF16, EG, EXCL, EPI>(pl, m, p, s) : launch<2, BK, BF16, EG, EXCL, EPI>(pl, m, p, s);
+}
+// The instantiation of the plan's geometry for epilogue EPI, with exclusion when the params carry exclusion lists.  The
+// experiment geometries exist for the top-K pass without exclusion only (make_plan selects them for no other pass), and
+// the label-score pass has no exclusion.
+template <int EPI, class P>
+static int launch_pass(const Plan& pl, const CUtensorMap (&m)[4], const P& p, cudaStream_t s) {
+    if constexpr (EPI == kEpiTopK) {
+        if (pl.eg == 2) return launch_cg<32, true, 2, false, EPI>(pl, m, p, s);
+        if (pl.bk == 16) return launch_cg<16, false, 1, false, EPI>(pl, m, p, s);
+    }
+    if constexpr (EPI != kEpiDiag) {
+        if (p.excl_off)
+            return pl.bf16 ? launch_cg<32, true, 1, true, EPI>(pl, m, p, s) : launch_cg<32, false, 1, true, EPI>(pl, m, p, s);
+    }
+    return pl.bf16 ? launch_cg<32, true, 1, false, EPI>(pl, m, p, s) : launch_cg<32, false, 1, false, EPI>(pl, m, p, s);
 }
 
 // kEpiDiag operand: dst row q = the item row of labels[q] (src row labels[q] - id_base), zeros when the label is not in
@@ -1289,43 +1327,6 @@ __global__ void lse_finish_kernel(const int32_t* __restrict__ shift, const doubl
 // log2(e) / temperature, rounded once to fp32: the same scale in the epilogue and in the finish
 static float lse_scale(float temperature) { return (float)(1.4426950408889634 / (double)temperature); }
 
-// Fields and tensor maps shared by the two label-rank passes.  `items` / `items_lo` are the item operand of the pass
-// (the table, or the gathered label rows) with `item_rows` rows.
-static int rank_params(RankParams& p, CUtensorMap (&maps)[4], const Plan& pl, const float* Uhi, const float* Ulo, int64_t Q,
-                       const void* items, const void* items_lo, int64_t item_rows, int64_t N, int E, int32_t id_base,
-                       int mode, const int64_t* labels) {
-    const bool bf16 = mode == MR_SCORE_BF16;
-    p = RankParams{};
-    p.Q = Q; p.N = N; p.E = E; p.K = 1; p.mode = mode; p.id_base = id_base;
-    p.KB = (E + (bf16 ? 63 : 31)) / (bf16 ? 64 : 32);
-    p.T = pl.T; p.QB = pl.QB; p.S = pl.S; p.QG = pl.QG; p.wave = pl.grid / pl.cg;
-    p.l2_hint = env_int("MR_SCORE_L2HINT", 1);
-    p.sync_w = pl.sync_w; p.sync_windows = pl.sync_windows;
-    p.sync_lead = env_int("MR_SCORE_PACE_LEAD", 1);
-    if (p.sync_lead < 1) p.sync_lead = 1;
-    p.sync_giveup = env_int("MR_SCORE_PACE_GIVEUP", 8);
-    p.labels = labels;
-    const int brows = kBlockN / pl.cg;
-    bool ok = make_map(&maps[0], Uhi, Q, E, kBlockM, 32, bf16) && make_map(&maps[2], items, item_rows, E, brows, 32, bf16);
-    if (ok && mode == MR_SCORE_TF32X3)
-        ok = make_map(&maps[1], Ulo, Q, E, kBlockM, 32, false) && make_map(&maps[3], items_lo, item_rows, E, brows, 32, false);
-    else if (ok) { maps[1] = maps[0]; maps[3] = maps[2]; }
-    if (!ok) { set_error("mr_score_rank: cuTensorMapEncodeTiled failed (driver without TMA support?)"); return MR_ERR_UNSUPPORTED; }
-    return MR_OK;
-}
-template <int EPI, bool EXCL, class P>
-static int launch_rank(const Plan& pl, const CUtensorMap (&m)[4], const P& p, bool bf16, cudaStream_t s) {
-    if (bf16) return pl.cg == 1 ? launch<1, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
-                                : launch<2, 32, true, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s);
-    return pl.cg == 1 ? launch<1, 32, false, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s)
-                      : launch<2, 32, false, 1, EXCL, EPI>(pl, m[0], m[1], m[2], m[3], p, s);
-}
-static int64_t align256(int64_t n) { return (n + 255) & ~(int64_t)255; }
-// workspace of the label-score pass: the gathered (hi, lo) label rows
-static int64_t diag_bytes(int64_t Q, int E, bool bf16) { return (bf16 ? 1 : 2) * align256(Q * E * (bf16 ? 2 : 4)); }
-// partials of the log-sum-exp pass on the counting pass's plan: (S, Q) fp64 sums, then (S, Q) int32 shifts
-static int64_t lse_part_bytes(const Plan& pl, int64_t Q) { return align256(pl.S * Q * 8) + align256(pl.S * Q * 4); }
-
 }  // namespace st
 }  // namespace mr
 
@@ -1346,12 +1347,11 @@ extern "C" int64_t mr_score_topk_schedule(int64_t Q, int64_t N, int K, int mode,
         set_error("mr_score_topk_schedule: need Q, N >= 1, 1 <= K <= %d and plan_out", MR_MAX_FUSED_TOPK);
         return MR_ERR_INVALID_ARG;
     }
-    const st::Plan pl = st::make_plan(Q, N, K, mode == MR_SCORE_BF16);
+    const st::Plan pl = st::make_plan(st::Pass::TopK, Q, N, 0, K, mode == MR_SCORE_BF16);
     st::Params p{};
     p.T = pl.T; p.QB = pl.QB; p.S = pl.S; p.QG = pl.QG; p.wave = pl.grid / pl.cg;
     const int64_t U = (int64_t)pl.QB * pl.S;
-    const int groups = pl.QG ? (pl.QB + pl.QG - 1) / pl.QG : (int)((U + p.wave - 1) / p.wave);
-    const int32_t plan[8] = {pl.QB, pl.T, pl.S, p.wave, pl.cg, groups * pl.S, pl.sync_windows, pl.sync_w};
+    const int32_t plan[8] = {pl.QB, pl.T, pl.S, p.wave, pl.cg, pl.streams, pl.sync_windows, pl.sync_w};
     for (int i = 0; i < 8; ++i) plan_out[i] = plan[i];
     if (units_out) {
         for (int64_t u = 0; u < U && u < max_units; ++u) {
@@ -1372,9 +1372,30 @@ extern "C" int64_t mr_score_topk_workspace_bytes(int64_t Q, int64_t N, int E, in
     }
     if (Q == 0) return 0;
     // sized for the mode that needs the most scratch (bf16-compat: two epilogue groups), so one query serves every mode
-    const st::Plan pa = st::make_plan(Q, N, K, false), pb = st::make_plan(Q, N, K, true);
-    const int64_t a = pa.cand_bytes + pa.part_bytes + pa.sync_bytes, b = pb.cand_bytes + pb.part_bytes + pb.sync_bytes;
-    return (a > b ? a : b) + 256;
+    const int64_t a = st::ws_need(st::make_plan(st::Pass::TopK, Q, N, E, K, false));
+    const int64_t b = st::ws_need(st::make_plan(st::Pass::TopK, Q, N, E, K, true));
+    return a > b ? a : b;
+}
+
+// The argument checks of every scoring pass, in one order, with `who` as the message prefix.  K is the list length of
+// the top-K passes (1 for the label passes); `outs`: the caller's output pointers are set.  MR_OK for Q = 0 before the
+// pointer checks.
+static int score_check(const char* who, const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo,
+                       int64_t N, int E, int K, int32_t id_base, int mode, bool outs) {
+    using namespace mr;
+    MR_REQUIRE(Q >= 0 && N >= 0 && E >= 1, "%s: need Q, N >= 0 and E >= 1", who);
+    MR_REQUIRE(K >= 1 && K <= MR_MAX_FUSED_TOPK, "%s: K=%d outside [1,%d]", who, K, MR_MAX_FUSED_TOPK);
+    MR_REQUIRE(mode == MR_SCORE_TF32X3 || mode == MR_SCORE_TF32X1 || mode == MR_SCORE_BF16, "%s: unknown mode %d", who, mode);
+    const bool bf16 = mode == MR_SCORE_BF16;
+    MR_REQUIRE(E % (bf16 ? 8 : 4) == 0, "%s: E=%d must be a multiple of %d (16-byte rows for TMA)", who, E, bf16 ? 8 : 4);
+    MR_REQUIRE(Q < (1ll << 31) - 512 && N < (1ll << 31) - 512 && (int64_t)id_base + N < (1ll << 31),
+               "%s: Q, N and id_base + N must fit 31 bits", who);
+    if (Q == 0) return MR_OK;
+    MR_REQUIRE(Uhi && Ihi && outs, "%s: null pointer", who);
+    MR_REQUIRE(mode != MR_SCORE_TF32X3 || (Ulo && Ilo), "%s: the 3xTF32 mode needs the lo operands", who);
+    MR_REQUIRE(host_aligned16(Uhi) && host_aligned16(Ihi) && host_aligned16(Ulo) && host_aligned16(Ilo),
+               "%s: operands must be 16-byte aligned", who);
+    return MR_OK;
 }
 
 // mr_score_topk (excl_off == NULL) and mr_score_topk_exclude
@@ -1382,19 +1403,8 @@ static int score_topk_impl(const float* Uhi, const float* Ulo, int64_t Q, const 
                            int E, int K, int32_t id_base, int mode, float* out_val, int32_t* out_id, void* ws,
                            int64_t ws_bytes, mr_stream_t stream, const int64_t* excl_off, const int32_t* excl_ids) {
     using namespace mr;
-    const bool excl = excl_off != nullptr;
-    MR_REQUIRE(Q >= 0 && N >= 0 && E >= 1, "mr_score_topk: need Q, N >= 0 and E >= 1");
-    MR_REQUIRE(K >= 1 && K <= MR_MAX_FUSED_TOPK, "mr_score_topk: K=%d outside [1,%d]", K, MR_MAX_FUSED_TOPK);
-    MR_REQUIRE(mode == MR_SCORE_TF32X3 || mode == MR_SCORE_TF32X1 || mode == MR_SCORE_BF16, "mr_score_topk: unknown mode %d", mode);
-    const bool bf16 = mode == MR_SCORE_BF16;
-    MR_REQUIRE(E % (bf16 ? 8 : 4) == 0, "mr_score_topk: E=%d must be a multiple of %d (16-byte rows for TMA)", E, bf16 ? 8 : 4);
-    MR_REQUIRE(Q < (1ll << 31) - 512 && N < (1ll << 31) - 512 && (int64_t)id_base + N < (1ll << 31),
-               "mr_score_topk: Q, N and id_base + N must fit 31 bits");
-    if (Q == 0) return MR_OK;
-    MR_REQUIRE(Uhi && Ihi && out_val && out_id, "mr_score_topk: null pointer");
-    MR_REQUIRE(mode != MR_SCORE_TF32X3 || (Ulo && Ilo), "mr_score_topk: the 3xTF32 mode needs the lo operands");
-    MR_REQUIRE(host_aligned16(Uhi) && host_aligned16(Ihi) && host_aligned16(Ulo) && host_aligned16(Ilo),
-               "mr_score_topk: operands must be 16-byte aligned");
+    int rc = score_check("mr_score_topk", Uhi, Ulo, Q, Ihi, Ilo, N, E, K, id_base, mode, out_val && out_id);
+    if (rc != MR_OK || Q == 0) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (N == 0) {  // nothing to score: every list is empty
         cudaError_t e = cudaMemsetAsync(out_id, 0xFF, (size_t)Q * K * 4, s);
@@ -1402,53 +1412,21 @@ static int score_topk_impl(const float* Uhi, const float* Ulo, int64_t Q, const 
         if (e != cudaSuccess) { set_error("mr_score_topk: memset: %s", cudaGetErrorString(e)); return (int)e; }
         return MR_OK;
     }
-    const st::Plan pl = st::make_plan(Q, N, K, bf16, excl);
-    const int64_t need = pl.cand_bytes + pl.part_bytes + pl.sync_bytes + 256;
-    if (!ws || ws_bytes < need) {
-        set_error("mr_score_topk: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
-        return MR_ERR_WORKSPACE;
-    }
-    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    const st::Plan pl = st::make_plan(excl_off ? st::Pass::TopKExcl : st::Pass::TopK, Q, N, E, K, mode == MR_SCORE_BF16);
     st::ExclParams p;
-    p.Q = Q; p.N = N; p.E = E; p.K = K; p.mode = mode; p.id_base = id_base;
-    const int bk = bf16 ? 32 : pl.bk;                 // bf16 rows are 64 elements = 128 bytes: the BK = 32 geometry
-    const int kelems = bf16 ? 64 : bk;
-    p.KB = (E + kelems - 1) / kelems;
-    p.T = pl.T; p.QB = pl.QB; p.S = pl.S; p.QG = pl.QG; p.wave = pl.grid / pl.cg;
-    p.cand = reinterpret_cast<mr::u64*>(w);
-    p.dbg = g_score_dbg;
-    p.l2_hint = st::env_int("MR_SCORE_L2HINT", 1);
-    p.sync = nullptr; p.sync_w = pl.sync_w; p.sync_windows = pl.sync_windows;
-    p.sync_lead = st::env_int("MR_SCORE_PACE_LEAD", 1);   // lead 1 / 2 / 3 at config 5: 376.5 / 379.6 / 381.2 ms
-    if (p.sync_lead < 1) p.sync_lead = 1;
-    p.sync_giveup = st::env_int("MR_SCORE_PACE_GIVEUP", 8);
-    if (pl.sync_bytes) {
-        p.sync = reinterpret_cast<int32_t*>(w + pl.cand_bytes + pl.part_bytes);
-        cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
-        if (e != cudaSuccess) { set_error("mr_score_topk: memset: %s", cudaGetErrorString(e)); return (int)e; }
-    }
+    CUtensorMap maps[4];
+    unsigned char* w;
+    rc = st::setup_pass("mr_score_topk", pl, p, maps, w, Uhi, Ulo, Q, Ihi, Ilo, N, E, K, id_base, mode, ws, ws_bytes, s);
+    if (rc != MR_OK) return rc;
     float* part_val = reinterpret_cast<float*>(w + pl.cand_bytes);
     int32_t* part_id = reinterpret_cast<int32_t*>(w + pl.cand_bytes + pl.part_bytes / 2);
+    p.cand = reinterpret_cast<mr::u64*>(w);
+    p.dbg = g_score_dbg;
     p.out_val = part_val;
     p.out_id = part_id;
     p.excl_off = excl_off;
     p.excl_ids = excl_ids;
-
-    CUtensorMap muh, mul, mih, mil;
-    const int brows = st::kBlockN / pl.cg;
-    bool ok = st::make_map(&muh, Uhi, Q, E, st::kBlockM, bk, bf16) && st::make_map(&mih, Ihi, N, E, brows, bk, bf16);
-    if (ok && mode == MR_SCORE_TF32X3)
-        ok = st::make_map(&mul, Ulo, Q, E, st::kBlockM, bk, false) && st::make_map(&mil, Ilo, N, E, brows, bk, false);
-    else if (ok) { mul = muh; mil = mih; }
-    if (!ok) { set_error("mr_score_topk: cuTensorMapEncodeTiled failed (driver without TMA support?)"); return MR_ERR_UNSUPPORTED; }
-
-    int rc;
-    if (excl && bf16) rc = pl.cg == 1 ? st::launch<1, 32, true, 1, true>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 1, true>(pl, muh, mul, mih, mil, p, s);
-    else if (excl) rc = pl.cg == 1 ? st::launch<1, 32, false, 1, true>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, false, 1, true>(pl, muh, mul, mih, mil, p, s);
-    else if (bf16 && pl.eg == 2) rc = pl.cg == 1 ? st::launch<1, 32, true, 2>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 2>(pl, muh, mul, mih, mil, p, s);
-    else if (bf16) rc = pl.cg == 1 ? st::launch<1, 32, true, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, true, 1>(pl, muh, mul, mih, mil, p, s);
-    else if (bk == 32) rc = pl.cg == 1 ? st::launch<1, 32, false, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 32, false, 1>(pl, muh, mul, mih, mil, p, s);
-    else rc = pl.cg == 1 ? st::launch<1, 16, false, 1>(pl, muh, mul, mih, mil, p, s) : st::launch<2, 16, false, 1>(pl, muh, mul, mih, mil, p, s);
+    rc = st::launch_pass<st::kEpiTopK>(pl, maps, p, s);
     if (rc != MR_OK) return rc;
     return mr_topk_merge(part_val, part_id, pl.S * pl.eg, Q, K, K, out_val, out_id, stream);
 }
@@ -1470,23 +1448,6 @@ extern "C" int mr_score_topk_exclude(const float* Uhi, const float* Ulo, int64_t
 }
 
 // ---- label rank against the whole catalog ------------------------------------------------------------------------
-static int rank_check(const char* who, const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo,
-                      int64_t N, int E, int32_t id_base, int mode) {
-    using namespace mr;
-    MR_REQUIRE(Q >= 0 && N >= 0 && E >= 1, "%s: need Q, N >= 0 and E >= 1", who);
-    MR_REQUIRE(mode == MR_SCORE_TF32X3 || mode == MR_SCORE_TF32X1 || mode == MR_SCORE_BF16, "%s: unknown mode %d", who, mode);
-    const bool bf16 = mode == MR_SCORE_BF16;
-    MR_REQUIRE(E % (bf16 ? 8 : 4) == 0, "%s: E=%d must be a multiple of %d (16-byte rows for TMA)", who, E, bf16 ? 8 : 4);
-    MR_REQUIRE(Q < (1ll << 31) - 512 && N < (1ll << 31) - 512 && (int64_t)id_base + N < (1ll << 31),
-               "%s: Q, N and id_base + N must fit 31 bits", who);
-    if (Q == 0) return MR_OK;
-    MR_REQUIRE(Uhi && Ihi, "%s: null pointer", who);
-    MR_REQUIRE(mode != MR_SCORE_TF32X3 || (Ulo && Ilo), "%s: the 3xTF32 mode needs the lo operands", who);
-    MR_REQUIRE(host_aligned16(Uhi) && host_aligned16(Ihi) && host_aligned16(Ulo) && host_aligned16(Ilo),
-               "%s: operands must be 16-byte aligned", who);
-    return MR_OK;
-}
-
 extern "C" int64_t mr_score_rank_workspace_bytes(int64_t Q, int64_t N, int E) {
     using namespace mr;
     if (Q < 0 || N < 0 || E < 1) {
@@ -1496,16 +1457,16 @@ extern "C" int64_t mr_score_rank_workspace_bytes(int64_t Q, int64_t N, int E) {
     if (Q == 0) return 0;
     // one scratch for both passes and every mode: the gathered fp32 (hi, lo) label rows, or the counting pass's counts
     // (the plan mr_score_rank builds: N = 0 plans as N = 1)
-    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, false, true, true);
-    const int64_t a = st::diag_bytes(Q, E, false), b = pl.part_bytes + pl.sync_bytes;
-    return (a > b ? a : b) + 256;
+    const int64_t a = st::ws_need(st::make_plan(st::Pass::Diag, Q, N, E, 1, false));
+    const int64_t b = st::ws_need(st::make_plan(st::Pass::Count, Q, N > 0 ? N : 1, E, 1, false));
+    return a > b ? a : b;
 }
 
 extern "C" int mr_label_score(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
                               int E, int32_t id_base, int mode, const int64_t* labels, uint32_t* label_key, void* ws,
                               int64_t ws_bytes, mr_stream_t stream) {
     using namespace mr;
-    int rc = rank_check("mr_label_score", Uhi, Ulo, Q, Ihi, Ilo, N, E, id_base, mode);
+    int rc = score_check("mr_label_score", Uhi, Ulo, Q, Ihi, Ilo, N, E, 1, id_base, mode, true);
     if (rc != MR_OK || Q == 0) return rc;
     MR_REQUIRE(labels && label_key, "mr_label_score: null pointer");
     cudaStream_t s = (cudaStream_t)stream;
@@ -1515,15 +1476,16 @@ extern "C" int mr_label_score(const float* Uhi, const float* Ulo, int64_t Q, con
         return MR_OK;
     }
     const bool bf16 = mode == MR_SCORE_BF16;
-    const int64_t need = st::diag_bytes(Q, E, bf16) + 256;
-    if (!ws || ws_bytes < need) {
-        set_error("mr_label_score: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
-        return MR_ERR_WORKSPACE;
-    }
-    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
     const int row_bytes = E * (bf16 ? 2 : 4);
-    void* ghi = w;
-    void* glo = w + st::align256(Q * row_bytes);
+    // the item operand: the gathered (hi, lo) label rows, which are the pass's workspace
+    unsigned char* ghi = st::ws_base(ws);
+    unsigned char* glo = ghi + st::align256(Q * row_bytes);
+    const st::Plan pl = st::make_plan(st::Pass::Diag, Q, N, E, 1, bf16);
+    st::RankParams p;
+    CUtensorMap maps[4];
+    unsigned char* w;
+    rc = st::setup_pass("mr_label_score", pl, p, maps, w, Uhi, Ulo, Q, ghi, glo, N, E, 1, id_base, mode, ws, ws_bytes, s);
+    if (rc != MR_OK) return rc;
     int64_t blocks = (Q * (row_bytes / 16) + 255) / 256;
     const int64_t cap = (int64_t)sm_count() * 16;
     if (blocks > cap) blocks = cap;
@@ -1534,20 +1496,9 @@ extern "C" int mr_label_score(const float* Uhi, const float* Ulo, int64_t Q, con
                                                                       reinterpret_cast<uint4*>(glo), Q, N, row_bytes / 16,
                                                                       id_base, labels);
     MR_CUDA_LAUNCH_CHECK("mr_label_score");
-    // one unit per query block, one tile each: the block's own gathered label rows
-    st::Plan pl{};
-    pl.cg = st::env_int("MR_SCORE_CTA_GROUP", 2) == 1 ? 1 : 2;
-    pl.bk = 32; pl.eg = 1;
-    pl.QB = (int)((Q + (int64_t)st::kBlockM * pl.cg - 1) / ((int64_t)st::kBlockM * pl.cg));
-    pl.T = 1; pl.S = 1; pl.QG = 0;
-    const int clusters = sm_count() / pl.cg;
-    pl.grid = (pl.QB < clusters ? pl.QB : clusters) * pl.cg;
-    st::RankParams p;
-    CUtensorMap maps[4];
-    rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, ghi, glo, Q, N, E, id_base, mode, labels);
-    if (rc != MR_OK) return rc;
+    p.labels = labels;
     p.out_key = label_key;
-    return st::launch_rank<st::kEpiDiag, false>(pl, maps, p, bf16, s);
+    return st::launch_pass<st::kEpiDiag>(pl, maps, p, s);
 }
 
 extern "C" int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
@@ -1557,34 +1508,24 @@ extern "C" int mr_score_rank(const float* Uhi, const float* Ulo, int64_t Q, cons
     using namespace mr;
     MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr),
                "mr_score_rank: excl_off and excl_ids must both be NULL or both be set");
-    int rc = rank_check("mr_score_rank", Uhi, Ulo, Q, Ihi, Ilo, N, E, id_base, mode);
+    int rc = score_check("mr_score_rank", Uhi, Ulo, Q, Ihi, Ilo, N, E, 1, id_base, mode, true);
     if (rc != MR_OK || Q == 0) return rc;
     MR_REQUIRE(labels && label_key && count, "mr_score_rank: null pointer");
     cudaStream_t s = (cudaStream_t)stream;
-    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, mode == MR_SCORE_BF16, true, true);
-    const int64_t need = pl.part_bytes + pl.sync_bytes + 256;
-    if (!ws || ws_bytes < need) {
-        set_error("mr_score_rank: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
-        return MR_ERR_WORKSPACE;
-    }
-    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    const st::Plan pl = st::make_plan(st::Pass::Count, Q, N > 0 ? N : 1, E, 1, mode == MR_SCORE_BF16);
+    st::RankParams p;
+    CUtensorMap maps[4];
+    unsigned char* w;
+    rc = st::setup_pass("mr_score_rank", pl, p, maps, w, Uhi, Ulo, Q, Ihi, Ilo, N, E, 1, id_base, mode, ws, ws_bytes, s);
+    if (rc != MR_OK) return rc;
     int32_t* part = reinterpret_cast<int32_t*>(w);
     if (N > 0) {
-        st::RankParams p;
-        CUtensorMap maps[4];
-        rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, Ihi, Ilo, N, N, E, id_base, mode, labels);
-        if (rc != MR_OK) return rc;
+        p.labels = labels;
         p.label_key = label_key;
         p.part = part;
         p.excl_off = excl_off;
         p.excl_ids = excl_ids;
-        if (pl.sync_bytes) {
-            p.sync = reinterpret_cast<int32_t*>(w + pl.part_bytes);
-            cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
-            if (e != cudaSuccess) { set_error("mr_score_rank: memset: %s", cudaGetErrorString(e)); return (int)e; }
-        }
-        rc = excl_off ? st::launch_rank<st::kEpiCount, true>(pl, maps, p, mode == MR_SCORE_BF16, s)
-                      : st::launch_rank<st::kEpiCount, false>(pl, maps, p, mode == MR_SCORE_BF16, s);
+        rc = st::launch_pass<st::kEpiCount>(pl, maps, p, s);
         if (rc != MR_OK) return rc;
     }
     st::rank_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(part, N > 0 ? pl.S : 0, Q, label_key, count);
@@ -1648,8 +1589,7 @@ extern "C" int64_t mr_score_lse_workspace_bytes(int64_t Q, int64_t N, int E) {
     }
     if (Q == 0) return 0;
     // the plan mr_score_lse builds (N = 0 plans as N = 1); the sync counters do not depend on the mode
-    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, false, true, true);
-    return st::lse_part_bytes(pl, Q) + pl.sync_bytes + 256;
+    return st::ws_need(st::make_plan(st::Pass::Lse, Q, N > 0 ? N : 1, E, 1, false));
 }
 
 extern "C" int mr_score_lse(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N,
@@ -1661,38 +1601,26 @@ extern "C" int mr_score_lse(const float* Uhi, const float* Ulo, int64_t Q, const
                "mr_score_lse: excl_off and excl_ids must both be NULL or both be set");
     MR_REQUIRE(temperature > 0.0f && temperature < INFINITY, "mr_score_lse: temperature must be finite and > 0");
     // N = 0: no item operand is read (an empty table may hand in NULL), only the empty partials are written
-    int rc = rank_check("mr_score_lse", Uhi, Ulo, Q, N > 0 ? Ihi : Uhi, N > 0 ? Ilo : Ulo, N, E, id_base, mode);
+    int rc = score_check("mr_score_lse", Uhi, Ulo, Q, N > 0 ? Ihi : Uhi, N > 0 ? Ilo : Ulo, N, E, 1, id_base, mode, true);
     if (rc != MR_OK || Q == 0) return rc;
     MR_REQUIRE(shift && sum, "mr_score_lse: null pointer");
     cudaStream_t s = (cudaStream_t)stream;
-    const st::Plan pl = st::make_plan(Q, N > 0 ? N : 1, 1, mode == MR_SCORE_BF16, true, true);
-    const int64_t part_bytes = st::lse_part_bytes(pl, Q);
-    const int64_t need = part_bytes + pl.sync_bytes + 256;
-    if (!ws || ws_bytes < need) {
-        set_error("mr_score_lse: workspace of %lld bytes needed, %lld given", (long long)need, (long long)ws_bytes);
-        return MR_ERR_WORKSPACE;
-    }
-    unsigned char* w = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    const st::Plan pl = st::make_plan(st::Pass::Lse, Q, N > 0 ? N : 1, E, 1, mode == MR_SCORE_BF16);
+    st::LseParams p;
+    CUtensorMap maps[4];
+    unsigned char* w;
+    rc = st::setup_pass("mr_score_lse", pl, p, maps, w, Uhi, Ulo, Q, Ihi, Ilo, N, E, 1, id_base, mode, ws, ws_bytes, s);
+    if (rc != MR_OK) return rc;
     double* psum = reinterpret_cast<double*>(w);
     int32_t* pshift = reinterpret_cast<int32_t*>(w + st::align256(pl.S * Q * 8));
     const float lc = st::lse_scale(temperature);
     if (N > 0) {
-        st::LseParams p;
-        CUtensorMap maps[4];
-        rc = st::rank_params(p, maps, pl, Uhi, Ulo, Q, Ihi, Ilo, N, N, E, id_base, mode, nullptr);
-        if (rc != MR_OK) return rc;
         p.lse_c = lc;
         p.lse_shift = pshift;
         p.lse_sum = psum;
         p.excl_off = excl_off;
         p.excl_ids = excl_ids;
-        if (pl.sync_bytes) {
-            p.sync = reinterpret_cast<int32_t*>(w + part_bytes);
-            cudaError_t e = cudaMemsetAsync(p.sync, 0, (size_t)pl.sync_bytes, s);
-            if (e != cudaSuccess) { set_error("mr_score_lse: memset: %s", cudaGetErrorString(e)); return (int)e; }
-        }
-        rc = excl_off ? st::launch_rank<st::kEpiLse, true>(pl, maps, p, mode == MR_SCORE_BF16, s)
-                      : st::launch_rank<st::kEpiLse, false>(pl, maps, p, mode == MR_SCORE_BF16, s);
+        rc = st::launch_pass<st::kEpiLse>(pl, maps, p, s);
         if (rc != MR_OK) return rc;
     }
     // the S splits merged in split order (none for N = 0: the empty pair)

@@ -56,6 +56,17 @@ def _device_csr(exclude: Optional[torch.Tensor], Q: int, dev) -> Optional[Tuple[
     return tuple(t.to(dev, non_blocking=True) for t in exclusion_csr(exclude, Q))
 
 
+def _row_chunks(scores: torch.Tensor, dev):
+    """(q0, q1, rows q0..q1 of `scores` as fp32 with unit column stride on `dev`): the whole matrix when it is on the
+    GPU, otherwise row chunks of at most 1 GiB."""
+    Q, N = scores.shape
+    rows_per_chunk = Q if scores.is_cuda else max(1, min(Q, (1 << 30) // max(4 * N, 1)))
+    for q0 in range(0, Q, max(rows_per_chunk, 1)):
+        q1 = min(Q, q0 + rows_per_chunk)
+        chunk = scores[q0:q1].to(device=dev, dtype=torch.float32, non_blocking=True)
+        yield q0, q1, chunk if chunk.stride(1) == 1 else chunk.contiguous()
+
+
 def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0,
               exclude: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """(values (Q, k) fp32, ids (Q, k) int32) of a (Q, N) score matrix: `mr_topk_rows`, the drop-in for
@@ -72,29 +83,27 @@ def topk_rows(scores: torch.Tensor, k: int, id_base: int = 0,
     csr = _device_csr(exclude, Q, dev)
     out_v = torch.empty((Q, k), dtype=torch.float32, device=dev)
     out_i = torch.empty((Q, k), dtype=torch.int32, device=dev)
-    rows_per_chunk = Q if scores.is_cuda else max(1, min(Q, (1 << 30) // max(4 * N, 1)))
-    for q0 in range(0, Q, max(rows_per_chunk, 1)):
-        q1 = min(Q, q0 + rows_per_chunk)
-        chunk = scores[q0:q1].to(device=dev, dtype=torch.float32, non_blocking=True)
-        if chunk.stride(1) != 1:
-            chunk = chunk.contiguous()
+    for q0, q1, chunk in _row_chunks(scores, dev):
+        args = (_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base, _lib.dptr(out_v[q0:q1]),
+                _lib.dptr(out_i[q0:q1]))
         if csr is None:
-            _lib.check(lib.mr_topk_rows(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base,
-                                        _lib.dptr(out_v[q0:q1]), _lib.dptr(out_i[q0:q1]), _lib.stream_handle()),
-                       "mr_topk_rows")
+            _lib.check(lib.mr_topk_rows(*args, _lib.stream_handle()), "mr_topk_rows")
         else:   # the offsets index the whole ids array: the chunk's rows are offsets[q0 : q1 + 1]
-            _lib.check(lib.mr_topk_rows_exclude(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), k, id_base,
-                                                _lib.dptr(out_v[q0:q1]), _lib.dptr(out_i[q0:q1]), _lib.dptr(csr[0][q0:]),
-                                                _lib.dptr(csr[1]), _lib.stream_handle()), "mr_topk_rows_exclude")
+            _lib.check(lib.mr_topk_rows_exclude(*args, _lib.dptr(csr[0][q0:]), _lib.dptr(csr[1]), _lib.stream_handle()),
+                       "mr_topk_rows_exclude")
     return out_v, out_i
+
+
+def _own_exclusion(labels: torch.Tensor, exclude: torch.Tensor) -> torch.Tensor:
+    """(Q,) bool on the labels' device: label q is in its own `exclude` row."""
+    return (exclude.to(device=labels.device, dtype=torch.int64) == labels[:, None]).any(dim=1)
 
 
 def _exclusion_miss(rank: torch.Tensor, labels: torch.Tensor, exclude: Optional[torch.Tensor]) -> torch.Tensor:
     """The miss rule of every evaluator path: a label inside its own `exclude` row has rank -1."""
     if exclude is None:
         return rank
-    own = (exclude.to(device=rank.device, dtype=torch.int64) == labels[:, None]).any(dim=1)
-    return torch.where(own, torch.full_like(rank, -1), rank)
+    return torch.where(_own_exclusion(labels, exclude), torch.full_like(rank, -1), rank)
 
 
 def _device_labels(labels: torch.Tensor, Q: int, dev) -> torch.Tensor:
@@ -118,17 +127,20 @@ def rank_rows(scores: torch.Tensor, labels: torch.Tensor, id_base: int = 0,
     labels = _device_labels(labels, Q, dev)
     csr = _device_csr(exclude, Q, dev)
     rank = torch.empty(Q, dtype=torch.int32, device=dev)
-    rows_per_chunk = Q if scores.is_cuda else max(1, min(Q, (1 << 30) // max(4 * N, 1)))
-    for q0 in range(0, Q, max(rows_per_chunk, 1)):
-        q1 = min(Q, q0 + rows_per_chunk)
-        chunk = scores[q0:q1].to(device=dev, dtype=torch.float32, non_blocking=True)
-        if chunk.stride(1) != 1:
-            chunk = chunk.contiguous()
+    for q0, q1, chunk in _row_chunks(scores, dev):
         off, ids = (None, None) if csr is None else (csr[0][q0:], csr[1])   # the offsets index the whole ids array
         _lib.check(lib.mr_rank_rows(_lib.dptr(chunk), q1 - q0, N, chunk.stride(0), id_base, _lib.dptr(labels[q0:q1]),
                                     _lib.dptr(off), _lib.dptr(ids), _lib.dptr(rank[q0:q1]), _lib.stream_handle()),
                    "mr_rank_rows")
     return _exclusion_miss(rank, labels, exclude)
+
+
+def _workspace(table: ShardedItemTable, query: str, *args) -> Tuple[torch.Tensor, int]:
+    """(the table's scratch, its size in bytes) for a call that needs what `lib.<query>(*args)` returns."""
+    ws_bytes = int(getattr(_lib.load(), query)(*args))
+    if ws_bytes < 0:
+        _lib.check(ws_bytes, query)
+    return table.workspace(ws_bytes), ws_bytes
 
 
 def score_topk(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: ShardedItemTable, k: int,
@@ -156,19 +168,13 @@ def _score_topk(user_hi, user_lo, table: ShardedItemTable, k: int, mode: int,
         out_i = torch.empty((Q, k), dtype=torch.int32, device=dev)
     else:
         out_v, out_i = out
-    ws_bytes = int(lib.mr_score_topk_workspace_bytes(Q, table.n_local, E, k))
-    if ws_bytes < 0:
-        _lib.check(ws_bytes, "mr_score_topk_workspace_bytes")
-    ws = table.workspace(ws_bytes)
+    ws, ws_bytes = _workspace(table, "mr_score_topk_workspace_bytes", Q, table.n_local, E, k)
+    args = (_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo), table.n_local, E, k,
+            table.id_base, mode, _lib.dptr(out_v), _lib.dptr(out_i), _lib.dptr(ws), ws_bytes)
     if csr is None:
-        _lib.check(lib.mr_score_topk(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
-                                     table.n_local, E, k, table.id_base, mode, _lib.dptr(out_v), _lib.dptr(out_i),
-                                     _lib.dptr(ws), ws_bytes, _lib.stream_handle()), "mr_score_topk")
+        _lib.check(lib.mr_score_topk(*args, _lib.stream_handle()), "mr_score_topk")
     else:
-        _lib.check(lib.mr_score_topk_exclude(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi),
-                                             _lib.dptr(table.lo), table.n_local, E, k, table.id_base, mode,
-                                             _lib.dptr(out_v), _lib.dptr(out_i), _lib.dptr(ws), ws_bytes,
-                                             _lib.dptr(csr[0]), _lib.dptr(csr[1]), _lib.stream_handle()),
+        _lib.check(lib.mr_score_topk_exclude(*args, _lib.dptr(csr[0]), _lib.dptr(csr[1]), _lib.stream_handle()),
                    "mr_score_topk_exclude")
     return out_v, out_i
 
@@ -181,10 +187,7 @@ def label_score(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: S
     lib = _lib.load()
     Q, E = user_hi.shape
     key = torch.empty(Q, dtype=torch.int32, device=user_hi.device)
-    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, table.n_local, E))
-    if ws_bytes < 0:
-        _lib.check(ws_bytes, "mr_score_rank_workspace_bytes")
-    ws = table.workspace(ws_bytes)
+    ws, ws_bytes = _workspace(table, "mr_score_rank_workspace_bytes", Q, table.n_local, E)
     _lib.check(lib.mr_label_score(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
                                   table.n_local, E, table.id_base, mode, _lib.dptr(labels), _lib.dptr(key), _lib.dptr(ws),
                                   ws_bytes, _lib.stream_handle()), "mr_label_score")
@@ -207,10 +210,7 @@ def score_rank(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: Sh
         raise ValueError(f"rows [{a}, {b}) outside the shard's {table.n_local} rows")
     hi, lo = table.hi[a:b], None if table.lo is None else table.lo[a:b]
     count = torch.empty(Q, dtype=torch.int32, device=user_hi.device)
-    ws_bytes = int(lib.mr_score_rank_workspace_bytes(Q, b - a, E))
-    if ws_bytes < 0:
-        _lib.check(ws_bytes, "mr_score_rank_workspace_bytes")
-    ws = table.workspace(ws_bytes)
+    ws, ws_bytes = _workspace(table, "mr_score_rank_workspace_bytes", Q, b - a, E)
     off, ids = (None, None) if csr is None else csr
     _lib.check(lib.mr_score_rank(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(hi), _lib.dptr(lo),
                                  b - a, E, table.id_base + a, mode, _lib.dptr(labels), _lib.dptr(label_key),
@@ -244,12 +244,11 @@ def bounded_count(queries: "PreparedQueries", table: ShardedItemTable, labels: t
     Q, E = queries.shape
     dev = queries.hi.device
     n_local = table.n_local
-    sharded = table.group is not None and table.world > 1
-    if sharded:
+    if table.sharded:
         import torch.distributed as dist
     n1 = _probe_rows(n_local)
     count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr, rows=(0, n1))
-    if sharded:
+    if table.sharded:
         dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
     elif n1 == n_local:
         return count                    # the probe was the whole table: the counts are exact
@@ -282,7 +281,7 @@ def bounded_count(queries: "PreparedQueries", table: ShardedItemTable, labels: t
                                       _lib.dptr(None if csr is None else csr_c[1]), _lib.stream_handle()),
                    "mr_rank_gather")
         rest = score_rank(hi, lo, table, labels_c[:n], key_c[:n], mode, csr_c, rows=rows)
-    if sharded:
+    if table.sharded:
         dist.all_reduce(rest, op=dist.ReduceOp.SUM, group=table.group)
     if in_place:
         idx, n = None, Q
@@ -302,10 +301,7 @@ def score_lse(user_hi: torch.Tensor, user_lo: Optional[torch.Tensor], table: Sha
     if out is None:
         out = (torch.empty(Q, dtype=torch.int32, device=user_hi.device),
                torch.empty(Q, dtype=torch.float64, device=user_hi.device))
-    ws_bytes = int(lib.mr_score_lse_workspace_bytes(Q, table.n_local, E))
-    if ws_bytes < 0:
-        _lib.check(ws_bytes, "mr_score_lse_workspace_bytes")
-    ws = table.workspace(ws_bytes)
+    ws, ws_bytes = _workspace(table, "mr_score_lse_workspace_bytes", Q, table.n_local, E)
     off, ids = (None, None) if csr is None else csr
     _lib.check(lib.mr_score_lse(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
                                 table.n_local, E, table.id_base, mode, float(temperature), _lib.dptr(off), _lib.dptr(ids),
@@ -394,7 +390,7 @@ class Evaluator:
             raise ValueError(f"fused top-k supports k <= {MAX_FUSED_TOPK}")
         queries, table = self._operands(user_emb, item_emb, normalize, mode, k)
         csr = _device_csr(exclude, queries.shape[0], queries.hi.device)
-        if table.group is None or table.world == 1:
+        if not table.sharded:
             return _score_topk(queries.hi, queries.lo, table, k, mode, None, csr)
         # sharded: the kernel writes this rank's list into the buffer that the single all-gather sends
         local, loc_v, loc_i = new_packed_list(queries.shape[0], k, queries.hi.device)
@@ -435,17 +431,16 @@ class Evaluator:
         labels = _device_labels(labels, Q, dev)
         csr = _device_csr(exclude, Q, dev)
         key = self._label_key(queries, table, labels, mode)
-        sharded = table.group is not None and table.world > 1
         if cap is not None:
             if not 1 <= int(cap) < 1 << 31:
                 raise ValueError(f"cap must be in [1, 2^31), not {cap}")
             count = bounded_count(queries, table, labels, key, mode, csr, int(cap))
         else:
             count = score_rank(queries.hi, queries.lo, table, labels, key, mode, csr)
-            if sharded:
+            if table.sharded:
                 import torch.distributed as dist
                 dist.all_reduce(count, op=dist.ReduceOp.SUM, group=table.group)
-        if sharded:
+        if table.sharded:
             count = torch.where(key == 0, torch.full_like(count, -1), count)
         return _exclusion_miss(count, labels, exclude)
 
@@ -453,7 +448,7 @@ class Evaluator:
     def _label_key(queries: PreparedQueries, table: ShardedItemTable, labels: torch.Tensor, mode: int) -> torch.Tensor:
         """`label_score`; on a sharded table the all-reduce MAX over the ranks, so every rank holds the label's key."""
         key = label_score(queries.hi, queries.lo, table, labels, mode)
-        if table.group is not None and table.world > 1:   # unsigned maximum as a signed one: flip the sign bit
+        if table.sharded:   # unsigned maximum as a signed one: flip the sign bit
             import torch.distributed as dist
             key ^= -(1 << 31)
             dist.all_reduce(key, op=dist.ReduceOp.MAX, group=table.group)
@@ -478,7 +473,7 @@ class Evaluator:
         labels = _device_labels(labels, Q, dev)
         csr = _device_csr(exclude, Q, dev)
         key = Evaluator._label_key(queries, table, labels, mode)
-        if table.group is None or table.world == 1:
+        if not table.sharded:
             shift, sums = score_lse(queries.hi, queries.lo, table, temperature, mode, csr)
             logp = lse_finish(shift[None], sums[None], key, temperature)
         else:
@@ -492,7 +487,7 @@ class Evaluator:
             logp = lse_finish(gathered[:, 2 * Q:].contiguous(), gathered[:, :2 * Q].contiguous().view(torch.float64),
                               key, temperature)
         if exclude is not None:   # the miss rule of `_exclusion_miss`, for labels of the catalog
-            own = (exclude.to(device=dev, dtype=torch.int64) == labels[:, None]).any(dim=1) & (key != 0)
+            own = _own_exclusion(labels, exclude) & (key != 0)
             logp = torch.where(own, torch.full_like(logp, -float("inf")), logp)
         return logp
 

@@ -153,6 +153,11 @@ class ShardedItemTable:
         import torch.distributed as dist
         return dist.get_world_size(self.group)
 
+    @property
+    def sharded(self) -> bool:
+        """The catalog is split over more than one rank: results need a collective over `group`."""
+        return self.group is not None and self.world > 1
+
 
 def topk_merge_packed(packed: torch.Tensor, k_out: int) -> Tuple[torch.Tensor, torch.Tensor]:
     """Merge the exchange buffer (L, 2, Q, K_in) int32 -- plane 0 the fp32 score bits, plane 1 the global ids of
