@@ -426,21 +426,26 @@ ties_pick_kernel(TiesState* st, const uint32_t* __restrict__ hist, const u64* __
     if (t == 0) {
         int bhi = s_bhi, blo = s_blo;
         int err = 0;
+        // a rank outside the bracket is clamped to its end bins (sample passes).  The top end is the bin holding hi, not
+        // bin kTiesBins - 1: a bracket narrower than 1024 << shift leaves the upper bins empty, and a bracket made of one
+        // of them would start above hi -- an inverted bracket whose magnitude window wraps and takes in almost every key
+        // of the vector in the full pass
+        const int top = (int)((s.hi - s.lo) >> s.shift);
         if (bhi < 0) {  // rank_hi above the bracket (<= above) or below it
-            if ((u64)rank_hi <= above) { if (strict) err = TIES_ERR_BRACKET_LOW; bhi = kTiesBins - 1; }
+            if ((u64)rank_hi <= above) { if (strict) err = TIES_ERR_BRACKET_LOW; bhi = top; }
             else { if (strict) err = TIES_ERR_BRACKET_HIGH; bhi = 0; }
         }
         if (blo < 0) {
-            if ((u64)rank_lo <= above) { if (strict) err = TIES_ERR_BRACKET_LOW; blo = kTiesBins - 1; }
+            if ((u64)rank_lo <= above) { if (strict) err = TIES_ERR_BRACKET_LOW; blo = top; }
             else { if (strict) err = TIES_ERR_BRACKET_HIGH; blo = 0; }
         }
-        if (rank_hi < 1) bhi = kTiesBins - 1;
+        if (rank_hi < 1) bhi = top;
         if (err) {
             s.status = err;
         } else {
             const u64 new_lo = s.lo + ((u64)blo << s.shift);
             u64 new_hi = s.lo + (((u64)bhi + 1) << s.shift) - 1;
-            if (new_hi > s.hi || bhi == kTiesBins - 1) new_hi = s.hi;
+            if (new_hi > s.hi || bhi == top) new_hi = s.hi;
             s.above = above + s_suffix[bhi + 1];
             s.in_bracket = s_suffix[blo] - s_suffix[bhi + 1];
             s.lo = new_lo;
@@ -1029,7 +1034,10 @@ ties_spec_kernel(const float* __restrict__ base, PtrPack<K> models, int64_t d, c
                     xs[k][0] = v.x; xs[k][1] = v.y; xs[k][2] = v.z; xs[k][3] = v.w;
                 }
             }
-            __syncthreads();   // every thread holds its quad in registers: the stage can be refilled
+            // every thread holds its quad in registers: the stage can be refilled.  The refill is a write of the async
+            // proxy, the reads above were generic ones: each thread orders its reads before it, then the CTA barrier
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            __syncthreads();
             if (threadIdx.x == 0) {
                 const int64_t next = tile_of(it + kSpecStages);
                 if (next < n_tiles) issue_tile(next, stage);

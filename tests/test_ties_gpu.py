@@ -221,11 +221,29 @@ def test_select_build_equals_select_then_build(K, d, quantize):
     """`mr_ties_select_build` (speculative build + exact cut + fix-up) == `mr_ties_select` + `mr_ties_build`, bit for bit:
     cut keys and every element of the (K, d) TIES vectors, including the interleaved-order tail columns (K >= 5), a partial
     last quad, and inputs with many equal magnitudes around the cut."""
-    _, _, _, cut, want, got, cut2, status = _spec_case(K, d, seed=300 + K, quantize=quantize)
-    if status.cpu().tolist() != [1] * K:
-        pytest.skip(f"sampled bracket missed on this input (status {status.cpu().tolist()}): the public path falls back")
-    assert torch.equal(cut2, cut)
-    assert torch.equal(got.view(torch.int32), want.view(torch.int32))
+    tb, tm, k_cnt, cut, want, got, cut2, status = _spec_case(K, d, seed=300 + K, quantize=quantize)
+    _check_deferred_status(tb, tm, k_cnt, cut, want, got, cut2, status)
+    # thousands of equal magnitudes at the cut (quantised inputs) may defeat the two 1024-way refinements; nothing else may
+    assert status.cpu().tolist() == [1] * K or quantize > 0, status.cpu().tolist()
+
+
+def _check_deferred_status(tb, tm, k_cnt, cut, want, got, cut2, status):
+    """A deferred select + build: every model reporting 1 carries the exact cut, a failure is one of the TIES_ERR_*
+    codes, all 1 means the output is exact, and the public (non-deferred) call is exact whatever the status."""
+    from mergerec_b200 import _lib
+    from mergerec_b200.merger.algorithms.ties import select_build
+    from mergerec_b200.merger.layout import alloc_rows
+    st = status.cpu()
+    assert set(st.tolist()) <= {1, -1, -2, -3, -4, -5}, st.tolist()
+    assert torch.equal(cut2.cpu()[st == 1], cut.cpu()[st == 1]), "status 1 with a wrong cut"
+    if bool((st == 1).all()):
+        assert torch.equal(cut2, cut)
+        assert torch.equal(got.view(torch.int32), want.view(torch.int32))
+    K, d = len(tm), tb.numel()
+    pub = alloc_rows(K, d, "cuda")
+    pub.fill_(float("nan"))
+    assert torch.equal(select_build(tb, tm, k_cnt, _lib.MR_TIES_VECTORS, pub, ldo=max(pub.stride(0), d)), cut)
+    assert torch.equal(pub.view(torch.int32), want.view(torch.int32))
 
 
 @pytest.mark.parametrize("shift", [1, 2, 3])
@@ -237,9 +255,8 @@ def test_select_build_unaligned_pointers(shift):
 
 @pytest.mark.parametrize("density", [0.0, 1e-7, 0.01, 0.5, 0.999, 1.0])
 def test_select_build_edge_densities(density):
-    _, _, _, cut, want, got, cut2, status = _spec_case(5, 70_001, seed=5, density=density)
-    if status.cpu().tolist() == [1] * 5:
-        assert torch.equal(cut2, cut) and torch.equal(got.view(torch.int32), want.view(torch.int32))
+    tb, tm, k_cnt, cut, want, got, cut2, status = _spec_case(5, 70_001, seed=5, density=density)
+    _check_deferred_status(tb, tm, k_cnt, cut, want, got, cut2, status)
 
 
 def test_select_build_falls_back_on_massive_ties():
