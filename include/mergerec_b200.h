@@ -303,6 +303,22 @@ int mr_score_lse(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi
 int mr_lse_finish(const int32_t* shift, const double* sum, int64_t P, int64_t Q, const uint32_t* label_key,
                   float temperature, float* logp, mr_stream_t stream);
 
+/* Gradient of the label log-softmax with respect to the queries, 3xTF32 only: with logp_q = f_{q,l} / T - lse_q over
+ * row q's eligible items and upstream gradient g_q = gscale[q] (dev fp32, Q),
+ *     dU[q] += -(g_q / T) * sum_n (p_qn - [n == labels[q]]) * I_n,    p_qn = exp(f_qn / T - lse_q),
+ * summed over this table's eligible items (not in the row's exclusion list; excl_off / excl_ids as for mr_score_lse).
+ * dU: dev fp32 (Q, E), 16-byte aligned; this table's contribution is added to what it holds.  The scores are recomputed
+ * by the instruction sequence of mr_score_lse, and lse_q comes from the (P, Q) partials (shift, sum) of the catalog's
+ * shards merged in index order, as mr_lse_finish merges them (P >= 1).  The table is walked in chunks of a fixed
+ * number of items, in ascending order: the same inputs give the same bits.  A row with gscale[q] = 0 adds exactly 0;
+ * rows whose label is not in the catalog or is excluded want a zero gscale (their log-softmax is NaN / -inf).
+ * ws: dev scratch of at least mr_score_lse_grad_workspace_bytes(Q, N, E) bytes (0 for Q = 0 or N = 0). */
+int64_t mr_score_lse_grad_workspace_bytes(int64_t Q, int64_t N, int E);
+int mr_score_lse_grad(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo, int64_t N, int E,
+                      int32_t id_base, float temperature, const int64_t* excl_off, const int32_t* excl_ids,
+                      const int64_t* labels, const int32_t* shift, const double* sum, int64_t P, const float* gscale,
+                      float* dU, void* ws, int64_t ws_bytes, mr_stream_t stream);
+
 /* Host-only view of the kernel's static schedule for a problem shape (no CUDA call; tests/test_schedule.py).  A unit =
  * (block of 256 queries, contiguous range of 256-item tiles); the grid's CTA pairs run the units in waves of `wave`,
  * unit u on pair u % wave.  plan_out (8 int32): query blocks, item tiles, item splits S, wave, CTAs per pair, item

@@ -59,6 +59,9 @@ SIGNATURES = {
     "mr_score_lse": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
                      C.c_int),
     "mr_lse_finish": ([_vp, _vp, _i64, _i64, _vp, C.c_float, _vp, _vp], C.c_int),
+    "mr_score_lse_grad_workspace_bytes": ([_i64, _i64, _i32], _i64),
+    "mr_score_lse_grad": ([_vp, _vp, _i64, _vp, _vp, _i64, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp,
+                           _vp, _i64, _vp], C.c_int),
     "mr_score_topk_schedule": ([_i64, _i64, _i32, _i32, _vp, _vp, _i64], _i64),
     "mr_to_bf16": ([_vp, _i64, _vp, _vp], C.c_int),
     "mr_split_tf32": ([_vp, _i64, _vp, _vp, _vp], C.c_int),

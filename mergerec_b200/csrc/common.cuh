@@ -32,6 +32,13 @@ int sm_count();
         }                                                                       \
     } while (0)
 
+// x rounded to TF32 (nearest, ties away): the hi part of the 3xTF32 split, and of x - hi its lo part
+__device__ __forceinline__ float rna_tf32(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r);
+}
+
 // ---- streaming 128-bit global accesses (read-once data: keep it out of L1) --------------------
 __device__ __forceinline__ float4 ldg_stream4(const float* p) {
     float4 r;

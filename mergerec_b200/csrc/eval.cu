@@ -282,12 +282,7 @@ rank_rows_kernel(const float* __restrict__ scores, int64_t Q, int64_t N, int64_t
 }
 
 // ---- hi/lo split for the 3xTF32 contraction -----------------------------------------------------------------------
-// hi = rna_tf32(x), lo = rna_tf32(x - hi): x = hi + lo up to 2^-22 |x|, both exactly representable in TF32.
-__device__ __forceinline__ float rna_tf32(float x) {
-    uint32_t r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return __uint_as_float(r);
-}
+// hi = rna_tf32(x), lo = rna_tf32(x - hi) (common.cuh): x = hi + lo up to 2^-22 |x|, both exactly representable in TF32.
 __global__ void split_tf32_kernel(const float* __restrict__ x, int64_t n, float* __restrict__ hi, float* __restrict__ lo) {
     const int64_t gsz = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gsz) {

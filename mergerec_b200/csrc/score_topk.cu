@@ -23,6 +23,7 @@
 // Two accumulator stages (2 x 256 TMEM columns) let the epilogue of tile i overlap the MMAs of tile i + 1.
 #include <cuda.h>
 
+#include <algorithm>
 #include <type_traits>
 
 #include "common.cuh"
@@ -112,11 +113,29 @@ struct LseParams : RankParams {
 // Shift range of a (shift, sum) pair: an empty sum is (kLseMinShift, 0).  Logits stay exact in the fp32 fma of the
 // epilogue while |shift| <= 2^24, which bounds the supported |score / temperature| to about 1.1e7.
 constexpr int kLseMinShift = -(1 << 24), kLseMaxShift = 1 << 24;
+// The two passes of mr_score_lse_grad, run once per catalog chunk.  kEpiProb: the chunk's scores, as kEpiLse computes
+// them, turned into W[q, n] = a_q (p_qn - [n == label_q]) with a_q = -gscale[q] / temperature and p the softmax under
+// the row's merged normaliser; 0 for padding and excluded ids.  Written as its TF32 (hi, lo) split into (Q, ldw).
+// kEpiAccum: the same mainloop with W as the query operand and the transposed chunk (E rows of ldw items) as the item
+// operand, so the contraction runs over the chunk's items and the 256-column tiles span E: dU[q, e] += acc.
+constexpr int kEpiProb = 4, kEpiAccum = 5;
+struct GradParams : LseParams {
+    float temperature;
+    const int32_t* row_shift;    // kEpiProb: (Q) the row's normaliser over the whole catalog as total * 2^shift
+    const double* row_sum;       // (Q) total
+    const float* gscale;         // (Q) upstream gradient of each row
+    float* w_hi;                 // kEpiProb: (Q, ldw) W, TF32 split as mr_split_tf32
+    float* w_lo;
+    int64_t ldw;
+    float* grad;                 // kEpiAccum: (Q, N) fp32, N = the embedding width of the gradient
+};
 template <bool EXCL, int EPI = kEpiTopK>
 using KernelParams = typename std::conditional<
-    EPI == kEpiLse, LseParams,
-    typename std::conditional<EPI != kEpiTopK, RankParams,
-                              typename std::conditional<EXCL, ExclParams, Params>::type>::type>::type;
+    EPI == kEpiProb || EPI == kEpiAccum, GradParams,
+    typename std::conditional<
+        EPI == kEpiLse, LseParams,
+        typename std::conditional<EPI != kEpiTopK, RankParams,
+                                  typename std::conditional<EXCL, ExclParams, Params>::type>::type>::type>::type;
 
 // ---- PTX helpers ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -527,6 +546,18 @@ __device__ __forceinline__ void label_epilogue(const P& p, uint32_t tmem_base, u
                 if (ex_cur < ex_end) ex_next = p.excl_ids[ex_cur];
             }
         }
+        // kEpiProb: p = 2^(f c - shift) / total, the term of kEpiLse over the merged total; one FMA correction of the
+        // prepared reciprocal makes p exactly 1 for a row whose total is its one term
+        float g_nk = 0.0f, g_tot = 1.0f, g_rinv = 1.0f, g_a = 0.0f;
+        if constexpr (EPI == kEpiProb) {
+            if (active) {
+                lab = p.labels[q];
+                g_nk = -(float)p.row_shift[q];
+                g_tot = (float)p.row_sum[q];
+                g_rinv = 1.0f / g_tot;
+                g_a = -p.gscale[q] / p.temperature;
+            }
+        }
         const uint32_t gt_keep = L == 0xFFFFFFFFu ? 0u : 0xFFFFu;   // NaN label: the NaN columns count only below its id
         int cnt = 0;
         int k = kLseMinShift;
@@ -553,6 +584,35 @@ __device__ __forceinline__ void label_epilogue(const P& p, uint32_t tmem_base, u
                     const int64_t l = p.labels[q];
                     const bool mine = l >= (int64_t)p.id_base && l < (int64_t)p.id_base + p.N;
                     p.out_key[q] = mine ? score_key(ranked_score<BF16>(bits)) : 0u;
+                }
+            } else if constexpr (EPI == kEpiAccum) {
+                // tile t = gradient columns [256 t, 256 t + 256) of the row; this unit is their only writer in the launch
+                const int64_t e0 = (int64_t)t * kBlockN;
+                const int ncols = (int)((p.N - e0) < kBlockN ? (p.N - e0) : kBlockN);
+                float* out = p.grad + (size_t)q * p.N + e0;
+#pragma unroll 1
+                for (int c = 0; c < ncols; c += kChunk) {
+                    uint32_t v[kChunk];
+                    tmem_ld16(taddr + c, v);
+                    tmem_ld_wait();
+                    if (active) {
+                        if (c + kChunk <= ncols) {
+                            float4* o4 = reinterpret_cast<float4*>(out + c);
+#pragma unroll
+                            for (int h = 0; h < kChunk / 4; ++h) {
+                                float4 d = o4[h];
+                                d.x += __uint_as_float(v[4 * h]);
+                                d.y += __uint_as_float(v[4 * h + 1]);
+                                d.z += __uint_as_float(v[4 * h + 2]);
+                                d.w += __uint_as_float(v[4 * h + 3]);
+                                o4[h] = d;
+                            }
+                        } else {
+#pragma unroll
+                            for (int j = 0; j < kChunk; ++j)
+                                if (c + j < ncols) out[c + j] += __uint_as_float(v[j]);
+                        }
+                    }
                 }
             } else {
                 const int64_t n0 = (int64_t)t * kBlockN;
@@ -587,6 +647,35 @@ __device__ __forceinline__ void label_epilogue(const P& p, uint32_t tmem_base, u
                     }
                     if constexpr (EPI == kEpiCount) {
                         cnt += __popc(m);
+                    } else if constexpr (EPI == kEpiProb) {
+                        const float lc = p.lse_c;
+                        float wh[kChunk], wl[kChunk];
+#pragma unroll
+                        for (int j = 0; j < kChunk; ++j) {
+                            const float term = ex2_approx(fmaf(ranked_score<BF16>(v[j]), lc, g_nk));
+                            const float p0 = term * g_rinv;
+                            const float pj = fmaf(fmaf(-p0, g_tot, term), g_rinv, p0);
+                            const float w = ((m >> j) & 1u) && g_a != 0.0f ? g_a * (id0 + j == lab ? pj - 1.0f : pj) : 0.0f;
+                            wh[j] = rna_tf32(w);
+                            wl[j] = rna_tf32(__fsub_rn(w, wh[j]));
+                        }
+                        // the row's columns [n0 + c, n0 + c + 16) of W; columns at or past ldw belong to the next row
+                        const int64_t col = n0 + c;
+                        if (active) {
+                            float* oh = p.w_hi + (size_t)q * p.ldw + col;
+                            float* ol = p.w_lo + (size_t)q * p.ldw + col;
+                            if (col + kChunk <= p.ldw) {
+#pragma unroll
+                                for (int h = 0; h < kChunk / 4; ++h) {
+                                    reinterpret_cast<float4*>(oh)[h] = make_float4(wh[4 * h], wh[4 * h + 1], wh[4 * h + 2], wh[4 * h + 3]);
+                                    reinterpret_cast<float4*>(ol)[h] = make_float4(wl[4 * h], wl[4 * h + 1], wl[4 * h + 2], wl[4 * h + 3]);
+                                }
+                            } else {
+#pragma unroll
+                                for (int j = 0; j < kChunk; ++j)
+                                    if (col + j < p.ldw) { oh[j] = wh[j]; ol[j] = wl[j]; }
+                            }
+                        }
                     } else {
                         const float lc = p.lse_c;
                         float f[kChunk];
@@ -1027,9 +1116,10 @@ static bool make_map(CUtensorMap* map, const void* ptr, int64_t rows, int E, int
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// The passes of the kernel: the top-K lists (without and with exclusion lists) and the label passes of mr_label_score
-// (kEpiDiag), mr_score_rank (kEpiCount) and mr_score_lse (kEpiLse).
-enum class Pass { TopK, TopKExcl, Diag, Count, Lse };
+// The passes of the kernel: the top-K lists (without and with exclusion lists), the label passes of mr_label_score
+// (kEpiDiag), mr_score_rank (kEpiCount) and mr_score_lse (kEpiLse), and the two gradient passes of mr_score_lse_grad
+// (kEpiProb, kEpiAccum).
+enum class Pass { TopK, TopKExcl, Diag, Count, Lse, Prob, Accum };
 struct Plan {
     Pass pass;
     bool bf16;
@@ -1114,6 +1204,8 @@ static Plan make_plan(Pass pass, int64_t Q, int64_t N, int E, int K, bool bf16) 
     case Pass::Diag: pl.part_bytes = (bf16 ? 1 : 2) * align256(Q * E * (bf16 ? 2 : 4)); break;   // gathered (hi, lo) rows
     case Pass::Count: pl.part_bytes = align256(pl.S * Q * 4); break;   // (S, Q) int32 counts
     case Pass::Lse: pl.part_bytes = align256(pl.S * Q * 8) + align256(pl.S * Q * 4); break;   // (S, Q) fp64 sums, int32 shifts
+    case Pass::Prob:
+    case Pass::Accum: pl.part_bytes = 0; break;   // they write W and dU, which mr_score_lse_grad places itself
     }
     return pl;
 }
@@ -1193,15 +1285,22 @@ static int launch_cg(const Plan& pl, const CUtensorMap (&m)[4], const P& p, cuda
 // the label-score pass has no exclusion.
 template <int EPI, class P>
 static int launch_pass(const Plan& pl, const CUtensorMap (&m)[4], const P& p, cudaStream_t s) {
-    if constexpr (EPI == kEpiTopK) {
-        if (pl.eg == 2) return launch_cg<32, true, 2, false, EPI>(pl, m, p, s);
-        if (pl.bk == 16) return launch_cg<16, false, 1, false, EPI>(pl, m, p, s);
+    // the gradient passes exist in 3xTF32 only, and the accumulation has no exclusion
+    if constexpr (EPI == kEpiProb) {
+        return p.excl_off ? launch_cg<32, false, 1, true, EPI>(pl, m, p, s) : launch_cg<32, false, 1, false, EPI>(pl, m, p, s);
+    } else if constexpr (EPI == kEpiAccum) {
+        return launch_cg<32, false, 1, false, EPI>(pl, m, p, s);
+    } else {
+        if constexpr (EPI == kEpiTopK) {
+            if (pl.eg == 2) return launch_cg<32, true, 2, false, EPI>(pl, m, p, s);
+            if (pl.bk == 16) return launch_cg<16, false, 1, false, EPI>(pl, m, p, s);
+        }
+        if constexpr (EPI != kEpiDiag) {
+            if (p.excl_off)
+                return pl.bf16 ? launch_cg<32, true, 1, true, EPI>(pl, m, p, s) : launch_cg<32, false, 1, true, EPI>(pl, m, p, s);
+        }
+        return pl.bf16 ? launch_cg<32, true, 1, false, EPI>(pl, m, p, s) : launch_cg<32, false, 1, false, EPI>(pl, m, p, s);
     }
-    if constexpr (EPI != kEpiDiag) {
-        if (p.excl_off)
-            return pl.bf16 ? launch_cg<32, true, 1, true, EPI>(pl, m, p, s) : launch_cg<32, false, 1, true, EPI>(pl, m, p, s);
-    }
-    return pl.bf16 ? launch_cg<32, true, 1, false, EPI>(pl, m, p, s) : launch_cg<32, false, 1, false, EPI>(pl, m, p, s);
 }
 
 // kEpiDiag operand: dst row q = the item row of labels[q] (src row labels[q] - id_base), zeros when the label is not in
@@ -1326,6 +1425,68 @@ __global__ void lse_finish_kernel(const int32_t* __restrict__ shift, const doubl
 }
 // log2(e) / temperature, rounded once to fp32: the same scale in the epilogue and in the finish
 static float lse_scale(float temperature) { return (float)(1.4426950408889634 / (double)temperature); }
+
+// ---- gradient of the label log-softmax with respect to the queries -------------------------------------------------
+// Items per chunk of mr_score_lse_grad (a multiple of 256): the scratch is (Q + E) x chunk x 8 bytes (W and the
+// transposed chunk, hi and lo), each chunk costs three launches, and TMEM accumulates W . I in fp32 over a whole chunk.
+// Measured at N = 10^6, E = 768 (DESIGN.md section 3.4): 2,048 keeps the gradient's error below that of an fp32 autograd,
+// 19 % slower than 8,192 at Q = 4,096 with 3.6x its error.  MR_LSE_GRAD_CHUNK overrides it for measurements.
+constexpr int64_t kGradChunk = 2048;
+static int64_t grad_chunk(int64_t N) {
+    int64_t c = env_int("MR_LSE_GRAD_CHUNK", (int)kGradChunk);
+    c = c < kBlockN ? kBlockN : (c + kBlockN - 1) / kBlockN * kBlockN;
+    const int64_t n = (N + kBlockN - 1) / kBlockN * kBlockN;   // no chunk wider than the table
+    return n > 0 && n < c ? n : c;
+}
+// Scratch of mr_score_lse_grad, each part 256-byte aligned: the two passes' own scratch (pacing counters, shared: the
+// passes run one after the other), the merged normaliser (shift int32, total fp64), W (hi, lo) and the transposed chunk.
+struct GradLayout {
+    int64_t chunk, pass, shift, sum, w_hi, w_lo, t_hi, t_lo, total;
+};
+static GradLayout grad_layout(int64_t Q, int64_t N, int E) {
+    GradLayout g{};
+    g.chunk = grad_chunk(N);
+    const int64_t last = N > 0 ? N - (N - 1) / g.chunk * g.chunk : g.chunk;   // items of the last chunk
+    for (int64_t n : {g.chunk, last}) {
+        const int64_t ld = (n + 3) & ~(int64_t)3;
+        const int64_t a = ws_need(make_plan(Pass::Prob, Q, n, E, 1, false));
+        const int64_t b = ws_need(make_plan(Pass::Accum, Q, E, (int)ld, 1, false));
+        g.pass = align256(std::max({g.pass, a, b}));
+    }
+    g.shift = g.pass;
+    g.sum = g.shift + align256(Q * 4);
+    g.w_hi = g.sum + align256(Q * 8);
+    g.w_lo = g.w_hi + align256(Q * g.chunk * 4);
+    g.t_hi = g.w_lo + align256(Q * g.chunk * 4);
+    g.t_lo = g.t_hi + align256((int64_t)E * g.chunk * 4);
+    g.total = g.t_lo + align256((int64_t)E * g.chunk * 4) + 256;
+    return g;
+}
+// rows [0, n) of the (n, E) operand pair (hi, lo) -> (E, ld) transposes, zero in columns [n, ld): the item operand of
+// kEpiAccum.  32 x 32 tiles through shared memory; the bits are copied, so the transposes hold the table's split.
+__global__ void __launch_bounds__(256) transpose_chunk_kernel(const float* __restrict__ hi, const float* __restrict__ lo,
+                                                              int64_t n, int E, int64_t ld, float* __restrict__ thi,
+                                                              float* __restrict__ tlo) {
+    __shared__ float sh[32][33], sl[32][33];
+    const int64_t n0 = (int64_t)blockIdx.x * 32;
+    const int e0 = blockIdx.y * 32;
+    for (int i = threadIdx.y; i < 32; i += 8) {
+        const int64_t r = n0 + i;
+        const int e = e0 + threadIdx.x;
+        const bool ok = r < n && e < E;
+        sh[i][threadIdx.x] = ok ? hi[r * E + e] : 0.0f;
+        sl[i][threadIdx.x] = ok ? lo[r * E + e] : 0.0f;
+    }
+    __syncthreads();
+    for (int i = threadIdx.y; i < 32; i += 8) {
+        const int e = e0 + i;
+        const int64_t col = n0 + threadIdx.x;
+        if (e < E && col < ld) {
+            thi[(int64_t)e * ld + col] = sh[threadIdx.x][i];
+            tlo[(int64_t)e * ld + col] = sl[threadIdx.x][i];
+        }
+    }
+}
 
 }  // namespace st
 }  // namespace mr
@@ -1640,5 +1801,94 @@ extern "C" int mr_lse_finish(const int32_t* shift, const double* sum, int64_t P,
     st::lse_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         shift, sum, (int)P, Q, label_key, st::lse_scale(temperature), nullptr, nullptr, logp);
     MR_CUDA_LAUNCH_CHECK("mr_lse_finish");
+    return MR_OK;
+}
+
+// ---- gradient of the label log-softmax with respect to the queries ------------------------------------------------
+extern "C" int64_t mr_score_lse_grad_workspace_bytes(int64_t Q, int64_t N, int E) {
+    using namespace mr;
+    if (Q < 0 || N < 0 || E < 1) {
+        set_error("mr_score_lse_grad_workspace_bytes: need Q, N >= 0 and E >= 1");
+        return MR_ERR_INVALID_ARG;
+    }
+    if (Q == 0 || N == 0) return 0;
+    return st::grad_layout(Q, N, E).total;
+}
+
+extern "C" int mr_score_lse_grad(const float* Uhi, const float* Ulo, int64_t Q, const float* Ihi, const float* Ilo,
+                                 int64_t N, int E, int32_t id_base, float temperature, const int64_t* excl_off,
+                                 const int32_t* excl_ids, const int64_t* labels, const int32_t* shift, const double* sum,
+                                 int64_t P, const float* gscale, float* dU, void* ws, int64_t ws_bytes,
+                                 mr_stream_t stream) {
+    using namespace mr;
+    MR_REQUIRE((excl_off == nullptr) == (excl_ids == nullptr),
+               "mr_score_lse_grad: excl_off and excl_ids must both be NULL or both be set");
+    MR_REQUIRE(temperature > 0.0f && temperature < INFINITY, "mr_score_lse_grad: temperature must be finite and > 0");
+    MR_REQUIRE(P >= 1 && P < (1 << 20), "mr_score_lse_grad: need 1 <= P < 2^20 partials");
+    int rc = score_check("mr_score_lse_grad", Uhi, Ulo, Q, N > 0 ? Ihi : Uhi, N > 0 ? Ilo : Ulo, N, E, 1, id_base,
+                         MR_SCORE_TF32X3, labels && shift && sum && gscale && dU);
+    if (rc != MR_OK || Q == 0 || N == 0) return rc;   // no item of this table: nothing to add
+    MR_REQUIRE(host_aligned16(dU), "mr_score_lse_grad: dU must be 16-byte aligned");
+    const st::GradLayout g = st::grad_layout(Q, N, E);
+    if (!ws || ws_bytes < g.total) {
+        set_error("mr_score_lse_grad: workspace of %lld bytes needed, %lld given", (long long)g.total, (long long)ws_bytes);
+        return MR_ERR_WORKSPACE;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned char* w = st::ws_base(ws);
+    int32_t* row_shift = reinterpret_cast<int32_t*>(w + g.shift);
+    double* row_sum = reinterpret_cast<double*>(w + g.sum);
+    float* w_hi = reinterpret_cast<float*>(w + g.w_hi);
+    float* w_lo = reinterpret_cast<float*>(w + g.w_lo);
+    float* t_hi = reinterpret_cast<float*>(w + g.t_hi);
+    float* t_lo = reinterpret_cast<float*>(w + g.t_lo);
+    const float lc = st::lse_scale(temperature);
+    // the row normalisers: the partials merged in index order, as mr_lse_finish merges them
+    st::lse_finish_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, s>>>(shift, sum, (int)P, Q, nullptr, lc, row_shift,
+                                                                       row_sum, nullptr);
+    MR_CUDA_LAUNCH_CHECK("mr_score_lse_grad");
+    // chunks in ascending order, each adding its contribution to dU: the same sums in the same order on every call
+    for (int64_t c0 = 0; c0 < N; c0 += g.chunk) {
+        const int64_t n = N - c0 < g.chunk ? N - c0 : g.chunk;
+        const int64_t ld = (n + 3) & ~(int64_t)3;
+        st::transpose_chunk_kernel<<<dim3((unsigned)((ld + 31) / 32), (unsigned)((E + 31) / 32)), dim3(32, 8), 0, s>>>(
+            Ihi + c0 * E, Ilo + c0 * E, n, E, ld, t_hi, t_lo);
+        MR_CUDA_LAUNCH_CHECK("mr_score_lse_grad");
+        {
+            const st::Plan pl = st::make_plan(st::Pass::Prob, Q, n, E, 1, false);
+            st::GradParams p;
+            CUtensorMap maps[4];
+            unsigned char* pw;
+            rc = st::setup_pass("mr_score_lse_grad", pl, p, maps, pw, Uhi, Ulo, Q, Ihi + c0 * E, Ilo + c0 * E, n, E, 1,
+                                (int32_t)(id_base + c0), MR_SCORE_TF32X3, w, g.pass, s);
+            if (rc != MR_OK) return rc;
+            p.lse_c = lc;
+            p.excl_off = excl_off;
+            p.excl_ids = excl_ids;
+            p.labels = labels;
+            p.temperature = temperature;
+            p.row_shift = row_shift;
+            p.row_sum = row_sum;
+            p.gscale = gscale;
+            p.w_hi = w_hi;
+            p.w_lo = w_lo;
+            p.ldw = ld;
+            rc = st::launch_pass<st::kEpiProb>(pl, maps, p, s);
+            if (rc != MR_OK) return rc;
+        }
+        {
+            // W (Q x ld) against the transposed chunk (E x ld): the contraction over the chunk's items
+            const st::Plan pl = st::make_plan(st::Pass::Accum, Q, E, (int)ld, 1, false);
+            st::GradParams p;
+            CUtensorMap maps[4];
+            unsigned char* pw;
+            rc = st::setup_pass("mr_score_lse_grad", pl, p, maps, pw, w_hi, w_lo, Q, t_hi, t_lo, E, (int)ld, 1, 0,
+                                MR_SCORE_TF32X3, w, g.pass, s);
+            if (rc != MR_OK) return rc;
+            p.grad = dU;
+            rc = st::launch_pass<st::kEpiAccum>(pl, maps, p, s);
+            if (rc != MR_OK) return rc;
+        }
+    }
     return MR_OK;
 }

@@ -12,6 +12,7 @@ Top-K order is (score desc, item id asc): ``torch.topk``'s order among equal sco
 from __future__ import annotations
 
 import os
+import warnings
 from typing import Dict, List, Optional, Tuple, Union
 
 import numpy as np
@@ -24,6 +25,15 @@ from .sharded import (MAX_FUSED_TOPK, MR_SCORE_BF16, MR_SCORE_TF32X3, ShardedIte
                       new_packed_list, split_tf32, to_bf16)
 
 MAX_TOPK = 1024
+_warned_item_grad = False
+
+
+def _warn_item_grad() -> None:
+    global _warned_item_grad
+    if not _warned_item_grad:
+        _warned_item_grad = True
+        warnings.warn("label_log_softmax: the item embeddings are a constant of the loss; they receive no gradient",
+                      stacklevel=3)
 _INT_DTYPES = (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8)
 
 
@@ -327,6 +337,74 @@ def lse_finish(shift: torch.Tensor, sum_: torch.Tensor, label_key: torch.Tensor,
     return logp
 
 
+def score_lse_grad(user_hi: torch.Tensor, user_lo: torch.Tensor, table: ShardedItemTable, temperature: float,
+                   labels: torch.Tensor, shift: torch.Tensor, sum_: torch.Tensor, gscale: torch.Tensor,
+                   csr: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """This shard's part of the gradient of the label log-softmax with respect to the 3xTF32 queries, (Q, E) fp32:
+    -(gscale[q] / temperature) * sum over row q's eligible items n of (p_qn - [n == labels[q]]) * item_n, with p the
+    softmax whose normaliser the (P, Q) `score_lse` partials `shift` / `sum_` give (merged as `lse_finish` merges
+    them) (`mr_score_lse_grad`).  `out`: optional (Q, E) fp32 tensor the contribution is added to (zeros by default)."""
+    lib = _lib.load()
+    Q, E = user_hi.shape
+    if table.bf16 or user_lo is None:
+        raise ValueError("the log-softmax gradient exists for the 3xTF32 operands only")
+    if shift.dim() != 2 or sum_.shape != shift.shape or shift.shape[1] != Q or shift.dtype != torch.int32 \
+            or sum_.dtype != torch.float64 or not (shift.is_contiguous() and sum_.is_contiguous()):
+        raise ValueError(f"expected contiguous (P, {Q}) int32 shifts and (P, {Q}) float64 sums")
+    gscale = gscale.to(device=user_hi.device, dtype=torch.float32).contiguous()
+    if out is None:
+        out = torch.zeros((Q, E), dtype=torch.float32, device=user_hi.device)
+    ws, ws_bytes = _workspace(table, "mr_score_lse_grad_workspace_bytes", Q, table.n_local, E)
+    off, ids = (None, None) if csr is None else csr
+    _lib.check(lib.mr_score_lse_grad(_lib.dptr(user_hi), _lib.dptr(user_lo), Q, _lib.dptr(table.hi), _lib.dptr(table.lo),
+                                     table.n_local, E, table.id_base, float(temperature), _lib.dptr(off), _lib.dptr(ids),
+                                     _lib.dptr(labels), _lib.dptr(shift), _lib.dptr(sum_), shift.shape[0],
+                                     _lib.dptr(gscale), _lib.dptr(out), _lib.dptr(ws), ws_bytes, _lib.stream_handle()),
+               "mr_score_lse_grad")
+    return out
+
+
+def _ordered_sum(parts: torch.Tensor) -> torch.Tensor:
+    """parts[0] + parts[1] + ... added in index order: the same bits wherever the same (G, ...) stack is summed."""
+    total = parts[0].clone()
+    for part in parts[1:]:
+        total += part
+    return total
+
+
+class _LabelLogSoftmax(torch.autograd.Function):
+    """`Evaluator.label_log_softmax` with a backward to the (normalised) query embeddings.  The forward runs the
+    kernels of the graph-free call; the backward recomputes the scores chunk by chunk (`score_lse_grad`)."""
+
+    @staticmethod
+    def forward(ctx, users, queries, table, labels, temperature, mode, exclude):
+        logp, parts = Evaluator._label_log_softmax(queries, table, labels, temperature, mode, exclude)
+        ctx.queries, ctx.table, ctx.temperature, ctx.mode = queries, table, temperature, mode
+        ctx.labels, ctx.csr, ctx.parts = parts
+        ctx.save_for_backward(logp)
+        return logp
+
+    @staticmethod
+    def backward(ctx, grad_logp):
+        if ctx.mode != MR_SCORE_TF32X3:
+            raise RuntimeError("label_log_softmax: the gradient exists in MR_SCORE_TF32X3 only; run the forward in "
+                               "that mode to train through it")
+        (logp,) = ctx.saved_tensors
+        queries, table = ctx.queries, ctx.table
+        # rows whose label is outside the catalog (NaN) or excluded (-inf) have no gradient
+        g = torch.where(logp.isfinite(), grad_logp.to(torch.float32), torch.zeros_like(logp))
+        shift, sums = ctx.parts
+        dU = score_lse_grad(queries.hi, queries.lo, table, ctx.temperature, ctx.labels, shift, sums, g, ctx.csr)
+        if table.sharded:
+            # every rank gets the partials of all ranks and adds them in rank order: the same bits on every rank
+            import torch.distributed as dist
+            gathered = torch.empty((table.world,) + tuple(dU.shape), dtype=dU.dtype, device=dU.device)
+            dist.all_gather_into_tensor(gathered.view(-1), dU.view(-1), group=table.group)
+            dU = _ordered_sum(gathered)
+        return dU, None, None, None, None, None, None
+
+
 class PreparedQueries:
     """Query embeddings in the operand format of the scoring kernel ((hi, lo) TF32 split, or bf16), prepared once and
     reusable against any number of item tables / evaluations (`Evaluator.prepare_queries`)."""
@@ -466,8 +544,35 @@ class Evaluator:
         those the lists rank (bf16-rounded in `MR_SCORE_BF16`).  Computed inside the fused scoring kernel: one pass
         scores each label (`label_score`), one sums exp(score / temperature) per row (`score_lse`).  On a sharded table
         every rank passes the same arguments and receives the same bits, after one all-reduce MAX of the label keys and
-        one all-gather of the (shift, sum) partials, merged in rank order (`lse_finish`)."""
+        one all-gather of the (shift, sum) partials, merged in rank order (`lse_finish`).
+
+        Differentiable with respect to `user_emb` when it is a tensor that requires grad (through the normalisation
+        when `normalize` is set): the backward recomputes the scores in the fused kernel, one catalog chunk at a time,
+        and contracts W[q, n] = -(g_q / T) (p_qn - [n == label_q]) with the items without building the (Q, N) matrix
+        (`score_lse_grad`).  Rows whose log-probability is NaN or -inf get a zero gradient.  The item embeddings are a
+        constant: an item tensor that requires grad gets none (a warning says so once).  `PreparedQueries` are
+        constants too.  The backward exists in `MR_SCORE_TF32X3` only; in the other modes it raises.  On a sharded
+        table every rank must call backward: each computes its shard's part, one all-gather of the (G, Q, E) parts
+        follows, and every rank adds them in rank order, so that all ranks hold the same bits."""
+        if isinstance(item_emb, torch.Tensor) and item_emb.requires_grad and torch.is_grad_enabled():
+            _warn_item_grad()
+            item_emb = item_emb.detach()
+        if isinstance(user_emb, torch.Tensor) and user_emb.requires_grad and torch.is_grad_enabled():
+            # the torch ops PreparedQueries applies, kept in the graph so that the gradient reaches user_emb
+            users = user_emb.to(device=_lib.require_cuda(), dtype=torch.float32)
+            if normalize:
+                users = torch.nn.functional.normalize(users, p=2, dim=-1)
+            queries = PreparedQueries(users.detach(), False, mode == MR_SCORE_BF16)
+            queries, table = Evaluator._operands(queries, item_emb, normalize, mode, 1)
+            return _LabelLogSoftmax.apply(users, queries, table, labels, temperature, mode, exclude)
         queries, table = Evaluator._operands(user_emb, item_emb, normalize, mode, 1)
+        return Evaluator._label_log_softmax(queries, table, labels, temperature, mode, exclude)[0]
+
+    @staticmethod
+    def _label_log_softmax(queries: PreparedQueries, table: ShardedItemTable, labels: torch.Tensor, temperature: float,
+                           mode: int, exclude: Optional[torch.Tensor]):
+        """(logp, (labels, exclusion CSR, (shift, sum) partials of every shard)): the forward of `label_log_softmax`
+        and what its backward needs."""
         Q = queries.shape[0]
         dev = queries.hi.device
         labels = _device_labels(labels, Q, dev)
@@ -475,7 +580,7 @@ class Evaluator:
         key = Evaluator._label_key(queries, table, labels, mode)
         if not table.sharded:
             shift, sums = score_lse(queries.hi, queries.lo, table, temperature, mode, csr)
-            logp = lse_finish(shift[None], sums[None], key, temperature)
+            shift, sums = shift[None], sums[None]
         else:
             # one buffer per rank, (sums fp64 | shifts int32) as 3Q words, written by the kernel and sent by ONE all-gather
             import torch.distributed as dist
@@ -484,12 +589,12 @@ class Evaluator:
                       out=(local[2 * Q:], local[:2 * Q].view(torch.float64)))
             gathered = torch.empty((table.world, 3 * Q), dtype=torch.int32, device=dev)
             dist.all_gather_into_tensor(gathered.view(-1), local, group=table.group)
-            logp = lse_finish(gathered[:, 2 * Q:].contiguous(), gathered[:, :2 * Q].contiguous().view(torch.float64),
-                              key, temperature)
+            shift, sums = gathered[:, 2 * Q:].contiguous(), gathered[:, :2 * Q].contiguous().view(torch.float64)
+        logp = lse_finish(shift, sums, key, temperature)
         if exclude is not None:   # the miss rule of `_exclusion_miss`, for labels of the catalog
             own = _own_exclusion(labels, exclude) & (key != 0)
             logp = torch.where(own, torch.full_like(logp, -float("inf")), logp)
-        return logp
+        return logp, (labels, csr, (shift, sums))
 
     def topk_embeddings_streamed(self, user_emb: Union[torch.Tensor, "PreparedQueries"], host_items: torch.Tensor,
                                  k: Optional[int] = None, id_base: int = 0, n_total: Optional[int] = None, group=None,
